@@ -20,6 +20,9 @@ the path, the drop-in binary on files, the loaders, the KZG10 consumer calls.
 `--impl reference` times the CPU restatement of the reference's algorithms (oracle/cpu_ref.c,
 kind "port": the Rust reference cannot be built here) on a bounded sample of the same
 workload (Algorithm-9 Fq2 sqrt, multiplication by r) with all host threads.
+
+`--dump-outputs DIR` writes what the last timed headline step returned (see dump_outputs) as
+DIR/<name>.npy, so that two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import csv
@@ -60,6 +63,30 @@ TAU = 0x1234567890ABCDEF1234567890ABCDEF
 # the ncu capture the `traffic` / pipe-busy figures of the roofline object are read from (tools/ncu_summary.py output)
 NCU_SUMMARY = os.path.join("profiles", "r02_ncu_full_all_kernels.csv")
 KERNEL_G1C, KERNEL_G2C = "convert_kernel<1, 2, 3, 1>", "convert_kernel<2, 2, 3, 1>"
+# --dump-outputs: points per group it writes, 2^15 x (96 + 192) bytes as float32 = 38 MB, and the seed of their indices
+DUMP_POINTS = 1 << 15
+DUMP_SEED = 0xB200
+
+
+def dump_outputs(out_dir, n, d_out1, d_out2, status):
+    """Write the headline step's results as the caller receives them: the ark uncompressed G1 and G2 records
+    (96 / 192 bytes each, one row per point, bytes as float32) of a fixed seeded sample of DUMP_POINTS point indices
+    (every index when n is smaller), the sorted indices themselves, and the status word (-1: every point passed)."""
+    import numpy as np
+    import torch
+
+    if n <= DUMP_POINTS:
+        idx = np.arange(n)
+    else:
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n, DUMP_POINTS, replace=False))
+    sel = torch.from_numpy(idx).to(d_out1.device)
+    arrays = {"index": idx.astype(np.float64),
+              "g1_ark_uncompressed": d_out1.view(n, 96).index_select(0, sel).cpu().numpy().astype(np.float32),
+              "g2_ark_uncompressed": d_out2.view(n, 192).index_select(0, sel).cpu().numpy().astype(np.float32),
+              "status": np.array([status.item()], dtype=np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def workload_config(log2_points, world):
@@ -323,7 +350,13 @@ def main():
                          "the 2^K-power setup, printed as its own line")
     ap.add_argument("--log2-powers", type=int, default=26, help="powers of the config5 setup (0: skip it)")
     ap.add_argument("--no-e2e", action="store_true", help="config5: skip the host -> host leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed headline step to DIR/<name>.npy (one process only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "config3" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs writes the headline (config3) outputs of --impl b200 in a single process")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         return run_reference(args)
@@ -406,6 +439,8 @@ def main():
     barrier()
     stop.set()
     th.join()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, n_loc, d_out1, d_out2, status)
     assert int(status.item()) == -1, "synthetic input failed validation"
     ms = sharding.reduce_max_ms(ms_step)
     ms_g1_max, ms_g2_max = sharding.reduce_max_ms(ms_g1), sharding.reduce_max_ms(ms_g2)

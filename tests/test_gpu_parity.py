@@ -578,6 +578,44 @@ def test_config3_compressed_full_size(ctx):
         assert 0.4 < float((flags != 0).mean()) < 0.6
 
 
+def test_bench_dump_outputs_vs_c_oracle(cref, tmp_path):
+    """`bench.py --dump-outputs` at 2^16 points per group: --steps sets the timed steps, the files hold a sorted sample
+    of 2^15 distinct indices with their G1 / G2 ark records as float32 bytes, and the records of the sampled indices
+    below 2^14 equal the C oracle's conversion of the same [tau^i]G."""
+    import subprocess
+    import sys
+
+    import bench
+    from conftest import ROOT
+
+    n, n_check, th = 1 << 16, 1 << 14, os.cpu_count() or 1
+    out = tmp_path / "dump"
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--log2-points", "16", "--steps", "2",
+                        "--warmup", "3", "--no-extra", "--dump-outputs", str(out)],
+                       capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("{")][0])["steps"] == 2
+    arrays = {p.stem: np.load(p) for p in out.glob("*.npy")}
+    assert sorted(arrays) == ["g1_ark_uncompressed", "g2_ark_uncompressed", "index", "status"]
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20
+    assert all(a.dtype in (np.float32, np.float64) for a in arrays.values())
+    assert arrays["status"].tolist() == [-1.0]
+    idx = arrays["index"]
+    assert idx.shape == (1 << 15,) and np.all(np.diff(idx) > 0) and idx[0] >= 0 and idx[-1] < n
+    assert np.array_equal(idx, idx.astype(np.int64))
+    mask = idx < n_check
+    for g, name, ro in ((1, "g1_ark_uncompressed", 96), (2, "g2_ark_uncompressed", 192)):
+        rec = arrays[name]
+        assert rec.shape == (1 << 15, ro) and np.array_equal(rec, rec.astype(np.uint8))
+        zc = cref.generate(g, ZC, 1, bench.TAU, 0, n_check, th)
+        zu, st = cref.convert(g, ZC, zc, ZU, 0, th)
+        assert not any(st)
+        want, st = cref.convert(g, ZU, zu, AU, 4, th)
+        assert not any(st)
+        want = np.frombuffer(want, dtype=np.uint8).reshape(n_check, ro)[idx[mask].astype(np.int64)]
+        assert np.array_equal(rec[mask].astype(np.uint8), want)
+
+
 def test_config4_validated_load(ctx, tmp_path):
     """BASELINE configs[3]: load of a 2^21-power setup (powers_of_g up to degree 2^22-2; 2^17
     powers under PTAU_TEST_FAST), both variants, through the file loaders: validated and
