@@ -82,6 +82,7 @@ extern "C" {
 #define PTAU_BAD_INFINITY 3
 #define PTAU_BAD_NOT_ON_CURVE 4
 #define PTAU_BAD_NOT_IN_SUBGROUP 5
+#define PTAU_BAD_NOT_POWERS 6 /* ptau_verify_powers: the points are valid but not powers of one tau */
 /* runtime errors (< 0) */
 #define PTAU_ERR_CUDA (-1)
 #define PTAU_ERR_ARG (-2)
@@ -254,6 +255,55 @@ int ptau_pairing_product2(ptau_ctx* ctx, const void* g1, const void* g2, size_t 
  * |z|); infinity_out[i] = 1 for a point at infinity (ark keeps no coefficients then; the slot is zero-filled). */
 #define PTAU_G2_PREPARED_COEFFS 68
 int ptau_g2_prepare(ptau_ctx* ctx, const void* g2, size_t n, void* coeffs_out, uint8_t* infinity_out);
+/* sum_i [scalars_i] points_i over G2: points = n ARK_MONT_LIMBS G2 records (200 B), scalars 32 B little-endian < r,
+ * out: one 200-byte record.  Same conventions, sharding and < r check (PTAU_ERR_ARG) as ptau_kzg_commit. */
+int ptau_msm_g2(ptau_ctx* ctx, const void* points, const void* scalars, size_t n, void* out);
+
+/* ---- are the powers powers of one tau? ---------------------------------------------------- */
+/* what ptau_verify_powers reads */
+#define PTAU_POWERS_RESPONSE 1 /* `powersoftau` response bytes (compressed, ptau_response_size(n) bytes, hash prefix and pubkey included) */
+#define PTAU_POWERS_KGZ 2      /* `kzg_setup` of preprocess-kgz     (ptau_setup_size(PTAU_VARIANT_KGZ, n))     */
+#define PTAU_POWERS_FASTKGZ 3  /* `kzg_setup` of preprocess-fastkgz (ptau_setup_size(PTAU_VARIANT_FASTKGZ, n)) */
+/* relations, reported through *bad_relation (the lowest failing one) */
+#define PTAU_REL_GENERATORS 0 /* tau_g1[0] / powers_of_g[0] is the G1 generator, tau_g2[0] / h the G2 generator */
+#define PTAU_REL_TAU_G1 1     /* consecutive G1 tau powers have ratio tau (against the first two G2 powers)   */
+#define PTAU_REL_TAU_G2 2     /* consecutive G2 tau powers have ratio tau (against the first two G1 powers)   */
+#define PTAU_REL_ALPHA_G1 3   /* alpha_tau powers / powers_of_gamma_g have ratio tau                          */
+#define PTAU_REL_BETA_G1 4    /* beta_tau powers have ratio tau (response only)                               */
+#define PTAU_REL_BETA_G2 5    /* e(beta_g1[0], H) == e(G, beta_g2) (response only)                            */
+#define PTAU_REL_KEY 6        /* kgz: g == powers_of_g[0], gamma_g == powers_of_gamma_g[0];                  */
+                              /* fastkgz: h == powers_of_h[0], beta_h == powers_of_h[1]                        */
+/* Checks that the points of a response or kzg_setup are powers of one tau: tau_g1[i] = [tau^i]G with the G1
+ * generator G, alpha powers and beta powers with the same tau, and the G2 powers matching the G1 powers.
+ *   Relations checked -- response: GENERATORS, TAU_G1, TAU_G2, ALPHA_G1, BETA_G1, BETA_G2; kgz: GENERATORS, TAU_G1,
+ *   ALPHA_G1, KEY (h, beta_h play tau_g2[0], tau_g2[1]); fastkgz: GENERATORS, TAU_G1, TAU_G2, ALPHA_G1, KEY
+ *   (powers_of_h[0], powers_of_h[1] play tau_g2[0], tau_g2[1]).
+ * Point checks come first: every point is checked with PTAU_CHECKS_STRICT, and a bad point is reported exactly as
+ * ptau_preprocess (response: *bad_section, *bad_index within it, *bad_kind) or ptau_load_setup (setups: *bad_index
+ * in file order over all points, *bad_section = 0) report the same bytes.  Only when every point is valid are the
+ * relations checked; a failure returns PTAU_BAD_NOT_POWERS with the lowest failing relation in *bad_relation.
+ * n_powers < 2: PTAU_ERR_ARG; len not the size of the kind for n_powers: PTAU_ERR_SIZE.
+ *
+ * A ratio relation over a section S of length L with reference pair (Q0, Q1) in G2 holds iff
+ *     e(B, Q0) e(-A, Q1) = 1,   A = sum_{i<L-1} rho_{k,i} S_i,   B = sum_{i<L-1} rho_{k,i} S_{i+1}
+ * (a G2 section with reference pair (P0, P1) in G1: e(P0, B) e(-P1, A) = 1), where k is the relation number and
+ *     rho_{k,i} = BLAKE2b(key = seed, digest 16 bytes)(k as one byte || i as 8 bytes little-endian),
+ * read little-endian and cut to its low 127 bits.  Soundness: all points are in the order-r subgroup, so for a seed
+ * chosen after the file exists, a file that is not a powers sequence passes a relation with probability at most
+ * 2^-127.  A seed known to whoever made the file voids this check.  The check says nothing about whether tau is
+ * secret; that is what the ceremony transcript is for.  seed NULL: 32 bytes from getrandom(2).
+ *
+ * combos_out (may be NULL): 8 slots of 200 bytes; slots 2k-2 and 2k-1 hold A and B of ratio relation k = 1..4 as
+ * ARK_MONT_LIMBS records (a G1 record fills the first 104 bytes of its slot); a slot is zero-filled when the relation
+ * does not apply to the kind.  Filled only when every point is valid.
+ *
+ * The file is streamed: device memory per GPU is bounded by the context's chunk_points c (rounded up to a multiple
+ * of 16), independent of n_powers -- about 16 c x 540 bytes (at the default c = 2^18: about 2.3 GB) -- so a 2^26
+ * response verifies on one GPU. */
+int ptau_verify_powers(ptau_ctx* ctx, int kind, const void* data, uint64_t len, uint64_t n_powers,
+                       const uint8_t seed[32], uint64_t* bad_index, int* bad_kind, int* bad_section, int* bad_relation,
+                       void* combos_out);
+
 /* ---- self-test hook --------------------------------------------------------------- */
 /* Raw Fq operations on n pairs of 48-byte Montgomery-limb values (host pointers), computed by
  * the kernels' own field code on the GPU: op 0 mul, 1 add, 2 sub, 3 neg, 4 sqr, 5 a^((p-3)/4),

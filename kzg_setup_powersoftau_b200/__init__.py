@@ -27,6 +27,8 @@ from ._ffi import (  # noqa: F401  (re-exported constants)
     CHECK_ON_CURVE, CHECK_REJECT_INFINITY, CHECK_SUBGROUP, CHECKS_DECOMPRESS, CHECKS_LOAD, CHECKS_READ,
     CHECKS_STRICT, FMT_ARK_MONT_LIMBS, FMT_ARK_UNCOMPRESSED, FMT_ZCASH_COMPRESSED, FMT_ZCASH_UNCOMPRESSED,
     G1, G2, STATUS_NONE, VARIANT_FASTKGZ, VARIANT_KGZ,
+    BAD_NOT_POWERS, POWERS_FASTKGZ, POWERS_KGZ, POWERS_RESPONSE, REL_ALPHA_G1, REL_BETA_G1, REL_BETA_G2,
+    REL_GENERATORS, REL_KEY, REL_NAMES, REL_TAU_G1, REL_TAU_G2,
 )
 
 # ---- reference constants (src/lib.rs:20-28, src/bin/preprocess-kgz.rs:18-23) --
@@ -56,16 +58,20 @@ class PtauError(Exception):
     """Data or runtime error from the C ABI.  The reference panics at this point
     (`unwrap()` at src/bin/preprocess-kgz.rs:142, src/lib.rs:180, ...)."""
 
-    def __init__(self, code: int, index: Optional[int] = None, section: Optional[int] = None, detail: str = ""):
+    def __init__(self, code: int, index: Optional[int] = None, section: Optional[int] = None, detail: str = "",
+                 relation: Optional[int] = None):
         self.code = code
         self.kind = BAD_NAMES.get(code)
         self.index = index
         self.section = section
+        self.relation = relation  # verify_powers: the lowest failing relation (REL_*)
         msg = _ffi.strerror(code)
         if index is not None:
             msg += " at point %d" % index
         if section is not None and 0 <= section < len(SECTION_NAMES):
             msg += " of section %s" % SECTION_NAMES[section]
+        if relation is not None and 0 <= relation < len(REL_NAMES):
+            msg += " (relation %s)" % REL_NAMES[relation]
         if detail:
             msg += " (%s)" % detail
         super().__init__(msg)
@@ -271,6 +277,40 @@ class Context:
         if rc != 0:
             self._raise(rc, bad_i.value if rc > 0 else None)
         return g1.reshape(-1, 104), g2.reshape(-1, 200)
+
+    def verify_powers(self, kind: int, data, n_powers: int, seed: Optional[bytes] = None, combos: bool = False):
+        """ptau_verify_powers: are the points of a response (POWERS_RESPONSE) or kzg_setup (POWERS_KGZ /
+        POWERS_FASTKGZ) powers of one tau?  Raises PtauError: a bad point as ptau_preprocess / ptau_load_setup
+        report it, or BAD_NOT_POWERS with `.relation`.  seed: 32 bytes (None: random).  combos=True returns the
+        8 x 200-byte combinations (A_k, B_k of ratio relation k in slots 2k-2, 2k-1), else None."""
+        src = _as_u8(data)
+        if seed is not None and len(seed) != 32:
+            raise PtauError(_ffi.ERR_ARG, detail="seed must be 32 bytes")
+        out = np.zeros((8, 200), dtype=np.uint8) if combos else None
+        bad_i, bad_k, bad_s, bad_r = C.c_uint64(0), C.c_int(0), C.c_int(-1), C.c_int(-1)
+        rc = _ffi.lib().ptau_verify_powers(self._h, kind, _ptr(src), src.size, n_powers,
+                                           bytes(seed) if seed is not None else None, C.byref(bad_i), C.byref(bad_k),
+                                           C.byref(bad_s), C.byref(bad_r), _ptr(out) if combos else None)
+        if rc == BAD_NOT_POWERS:
+            raise PtauError(rc, relation=bad_r.value)
+        if rc != 0:
+            section = bad_s.value if (rc > 0 and kind == POWERS_RESPONSE) else None
+            self._raise(rc, bad_i.value if rc > 0 else None, section)
+        return out
+
+    def msm_g2(self, points, scalars) -> np.ndarray:
+        """sum_i scalars[i] * points[i] over G2 (ptau_msm_g2): points [n, 200] Montgomery-limb records, scalars ints
+        (taken mod r) or a [n, 32] u8 array of little-endian scalars < r.  Returns one 200-byte record."""
+        pts = np.ascontiguousarray(np.asarray(points, dtype=np.uint8).reshape(-1, 200))
+        sc = KZG10._scalars(scalars)
+        n = sc.size // 32
+        if pts.shape[0] < n:
+            raise PtauError(_ffi.ERR_ARG, detail="more scalars than points")
+        out = np.zeros(200, dtype=np.uint8)
+        rc = _ffi.lib().ptau_msm_g2(self._h, _ptr(pts) if n else None, _ptr(sc) if n else None, n, _ptr(out))
+        if rc != 0:
+            self._raise(rc)
+        return out
 
     def microbench(self, kind: int, iters: int, gpu: int = 0) -> Tuple[float, float]:
         ms, ops = C.c_double(0), C.c_double(0)
@@ -720,6 +760,38 @@ def load_fastkzg_setup(path: str = KZG_SETUP_FILE, log2_powers: Optional[int] = 
         prepared_beta_h_src=g2[1],
     )
     return params, powers_of_h
+
+
+# ---- are the powers powers of one tau? (ptau_verify_powers) --------------------------------------
+def _verify_file(kind: int, path: str, n: int, ctx: Optional[Context], seed: Optional[bytes]) -> None:
+    if not os.path.exists(path):
+        raise FileNotFoundError(path)
+    data = np.memmap(path, dtype=np.uint8, mode="r")
+    try:
+        (ctx or default_context()).verify_powers(kind, data, n, seed=seed)
+    finally:
+        del data
+
+
+def verify_kzg_setup(path: str = KZG_SETUP_FILE, log2_powers: Optional[int] = None, ctx: Optional[Context] = None,
+                     seed: Optional[bytes] = None) -> None:
+    """Checks that a preprocess-kgz `kzg_setup` holds powers of one tau (strict point checks, then the ratio
+    relations by pairing).  n from log2_powers, or inferred from the file size.  Raises PtauError on failure."""
+    n = (1 << log2_powers) if log2_powers is not None else _n_from_setup_size(VARIANT_KGZ, os.path.getsize(path))
+    _verify_file(POWERS_KGZ, path, n, ctx, seed)
+
+
+def verify_fastkzg_setup(path: str = KZG_SETUP_FILE, log2_powers: Optional[int] = None, ctx: Optional[Context] = None,
+                         seed: Optional[bytes] = None) -> None:
+    """verify_kzg_setup for a preprocess-fastkgz `kzg_setup` (its powers_of_h are checked too)."""
+    n = (1 << log2_powers) if log2_powers is not None else _n_from_setup_size(VARIANT_FASTKGZ, os.path.getsize(path))
+    _verify_file(POWERS_FASTKGZ, path, n, ctx, seed)
+
+
+def verify_powersoftau(path: str = POWERSOFTAU_FILE, log2_powers: int = DEFAULT_LOG2_POWERS, ctx: Optional[Context] = None,
+                       seed: Optional[bytes] = None) -> None:
+    """Checks that a `powersoftau` response holds powers of one tau: tau, alpha and beta powers, both groups."""
+    _verify_file(POWERS_RESPONSE, path, 1 << log2_powers, ctx, seed)
 
 
 # ---- the two binaries (src/bin/preprocess-kgz.rs, preprocess-fastkgz.rs) -------------

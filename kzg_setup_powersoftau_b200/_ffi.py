@@ -23,10 +23,13 @@ CHECKS_DECOMPRESS = 0
 CHECKS_STRICT = CHECK_ON_CURVE | CHECK_SUBGROUP | CHECK_REJECT_INFINITY
 OK = 0
 BAD_NON_CANONICAL, BAD_FLAGS, BAD_INFINITY, BAD_NOT_ON_CURVE, BAD_NOT_IN_SUBGROUP = 1, 2, 3, 4, 5
+BAD_NOT_POWERS = 6
 ERR_CUDA, ERR_ARG, ERR_SIZE, ERR_NOMEM, ERR_IO, ERR_DIGEST, ERR_EXISTS = -1, -2, -3, -4, -5, -6, -7
 FILE_SKIP_DIGEST, FILE_NO_UNCOMPRESSED, FILE_FSYNC = 1, 2, 4
 VARIANT_KGZ, VARIANT_FASTKGZ = 1, 2
 STATUS_NONE = 0xFFFFFFFFFFFFFFFF
+POWERS_RESPONSE, POWERS_KGZ, POWERS_FASTKGZ = 1, 2, 3
+REL_GENERATORS, REL_TAU_G1, REL_TAU_G2, REL_ALPHA_G1, REL_BETA_G1, REL_BETA_G2, REL_KEY = 0, 1, 2, 3, 4, 5, 6
 
 BAD_NAMES = {
     BAD_NON_CANONICAL: "NON_CANONICAL",
@@ -34,7 +37,9 @@ BAD_NAMES = {
     BAD_INFINITY: "INFINITY",
     BAD_NOT_ON_CURVE: "NOT_ON_CURVE",
     BAD_NOT_IN_SUBGROUP: "NOT_IN_SUBGROUP",
+    BAD_NOT_POWERS: "NOT_POWERS",
 }
+REL_NAMES = ("GENERATORS", "TAU_G1", "TAU_G2", "ALPHA_G1", "BETA_G1", "BETA_G2", "KEY")
 
 
 class Timing(C.Structure):
@@ -123,6 +128,12 @@ _SIGNATURES = {
     "ptau_kzg_check": (C.c_int, [C.c_void_p] * 8 + [C.c_size_t, C.c_void_p]),
     "ptau_pairing_product2": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]),
     "ptau_g2_prepare": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]),
+    "ptau_msm_g2": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "ptau_verify_powers": (
+        C.c_int,
+        [C.c_void_p, C.c_int, C.c_void_p, C.c_uint64, C.c_uint64, C.c_char_p, C.POINTER(C.c_uint64), C.POINTER(C.c_int),
+         C.POINTER(C.c_int), C.POINTER(C.c_int), C.c_void_p],
+    ),
     "ptau_selftest_fq_op": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t]),
     "ptau_microbench": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double)]),
 }

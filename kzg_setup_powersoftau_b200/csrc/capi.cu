@@ -19,45 +19,16 @@
 #include "../../include/ptau_b200.h"
 #include <future>
 
+#include "context.h"
 #include "kernels.h"
 
+using ptau::GpuSlot;
+using ptau::kBufs;
+using ptau::kMaxGpus;
+
 namespace {
 
-constexpr int kMaxGpus = 8;
 constexpr size_t kEdgePoints = 148 * 2 * 128;  // one wave of convert-kernel blocks on a B200
-constexpr int kBufs = 2;  // double buffering per GPU
-
-struct GpuSlot {
-  int device = -1;
-  cudaStream_t stream[kBufs] = {nullptr, nullptr};
-  void* d_in[kBufs] = {nullptr, nullptr};
-  void* d_out[kBufs] = {nullptr, nullptr};
-  size_t cap_in = 0, cap_out = 0;
-  unsigned long long* d_status = nullptr;
-  cudaEvent_t ev_first = nullptr, ev_last = nullptr;
-  cudaEvent_t ev_k0[kBufs] = {nullptr, nullptr}, ev_k1[kBufs] = {nullptr, nullptr};
-  uint32_t* d_tbl[2] = {nullptr, nullptr};  // fixed-base tables of the generator (G1, G2), built lazily
-  // KZG10::check: fixed-base tables of the verifier key's g, gamma_g, h, rebuilt when the key changes
-  void* d_kzg_tbl = nullptr;
-  std::string kzg_tbl_key;
-  // multi-scalar multiplication: device points / scalars / scratch / result and the pinned staging buffer of the
-  // scalars, kept between calls and grown on demand (no cudaMalloc / cudaFree inside a commitment)
-  void *d_msm_pts = nullptr, *d_msm_sc = nullptr, *d_msm_scratch = nullptr, *d_msm_out = nullptr, *h_msm_sc = nullptr;
-  size_t cap_msm_pts = 0, cap_msm_sc = 0, cap_msm_scratch = 0, cap_h_msm_sc = 0;
-  uint32_t* h_msm_out = nullptr;  // pinned: 26 words of the result record + 1 word "a scalar was >= r"
-};
-
-}  // namespace
-
-struct ptau_ctx {
-  int n_gpus = 0;
-  size_t chunk_points = 0;
-  GpuSlot gpu[kMaxGpus];
-  ptau_timing timing;
-  std::string last_error;
-};
-
-namespace {
 
 #define CUDA_TRY(ctx, expr)                                                          \
   do {                                                                               \
@@ -210,6 +181,7 @@ const char* ptau_strerror(int code) {
     case PTAU_BAD_INFINITY: return "point at infinity";
     case PTAU_BAD_NOT_ON_CURVE: return "point not on the curve";
     case PTAU_BAD_NOT_IN_SUBGROUP: return "point not in the prime-order subgroup";
+    case PTAU_BAD_NOT_POWERS: return "points are valid but not powers of one tau";
     case PTAU_ERR_CUDA: return "CUDA runtime error (no CPU fallback exists)";
     case PTAU_ERR_ARG: return "invalid argument";
     case PTAU_ERR_SIZE: return "buffer or file size does not match the layout";
@@ -751,29 +723,37 @@ void copy_parts(void* dst, const void* src, size_t len) {
   for (int i = 1; i < parts; i++) f[i].get();
 }
 // One multi-scalar multiplication on one GPU, issued asynchronously on the slot's first stream; result and the
-// "scalar >= r" flag land in s.h_msm_out.  pts: host records, or (resident = true) device records on this GPU.
-cudaError_t msm_issue(GpuSlot& s, const void* pts, const void* sc, size_t n, int* launches, bool resident = false) {
+// "scalar >= r" flag land in s.h_msm_out.  pts: host records, or (resident = true) device records on this GPU;
+// G1 (104-byte records) or, with g2, G2 (200-byte records).
+cudaError_t msm_issue(GpuSlot& s, const void* pts, const void* sc, size_t n, int* launches, bool resident = false,
+                      bool g2 = false) {
   cudaError_t e = cudaSetDevice(s.device);
+  const size_t rb = g2 ? 200 : 104;
   ptau::MsmPlan plan;
-  ptau::msm_g1_plan(n, &plan);
+  if (g2)
+    ptau::msm_g2_plan(n, &plan);
+  else
+    ptau::msm_g1_plan(n, &plan);
   const void* d_pts = pts;
   if (e == cudaSuccess && !resident) {
-    e = grow(&s.d_msm_pts, &s.cap_msm_pts, n * 104 + 16);
+    e = grow(&s.d_msm_pts, &s.cap_msm_pts, n * rb + 16);
     d_pts = s.d_msm_pts;
   }
   if (e == cudaSuccess) e = grow(&s.d_msm_sc, &s.cap_msm_sc, n * 32 + 16);
   if (e == cudaSuccess) e = grow(&s.d_msm_scratch, &s.cap_msm_scratch, plan.scratch_bytes);
   if (e == cudaSuccess) e = grow(&s.h_msm_sc, &s.cap_h_msm_sc, n * 32 + 16, true);
-  if (e == cudaSuccess && !s.d_msm_out) e = cudaMalloc(&s.d_msm_out, 128);
-  if (e == cudaSuccess && !s.h_msm_out) e = cudaHostAlloc((void**)&s.h_msm_out, 128, cudaHostAllocPortable);
+  if (e == cudaSuccess && !s.d_msm_out) e = cudaMalloc(&s.d_msm_out, 256);
+  if (e == cudaSuccess && !s.h_msm_out) e = cudaHostAlloc((void**)&s.h_msm_out, 256, cudaHostAllocPortable);
   if (e != cudaSuccess) return e;
   copy_parts(s.h_msm_sc, sc, n * 32);
-  if (!resident) e = cudaMemcpyAsync(s.d_msm_pts, pts, n * 104, cudaMemcpyHostToDevice, s.stream[0]);
+  if (!resident) e = cudaMemcpyAsync(s.d_msm_pts, pts, n * rb, cudaMemcpyHostToDevice, s.stream[0]);
   if (e == cudaSuccess) e = cudaMemcpyAsync(s.d_msm_sc, s.h_msm_sc, n * 32, cudaMemcpyHostToDevice, s.stream[0]);
   if (e == cudaSuccess) e = cudaEventRecord(s.ev_k0[0], s.stream[0]);
-  if (e == cudaSuccess) e = ptau::launch_msm_g1(d_pts, s.d_msm_sc, n, s.d_msm_scratch, s.d_msm_out, launches, s.stream[0]);
+  if (e == cudaSuccess)
+    e = (g2 ? ptau::launch_msm_g2 : ptau::launch_msm_g1)(d_pts, s.d_msm_sc, n, s.d_msm_scratch, s.d_msm_out, launches,
+                                                         s.stream[0]);
   if (e == cudaSuccess) e = cudaEventRecord(s.ev_k1[0], s.stream[0]);
-  if (e == cudaSuccess) e = cudaMemcpyAsync(s.h_msm_out, s.d_msm_out, 108, cudaMemcpyDeviceToHost, s.stream[0]);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(s.h_msm_out, s.d_msm_out, rb + 4, cudaMemcpyDeviceToHost, s.stream[0]);
   return e;
 }
 cudaError_t msm_wait(GpuSlot& s, float* ms) {
@@ -793,11 +773,16 @@ struct ptau_kzg_powers {
 };
 
 static int kzg_commit_impl(ptau_ctx* ctx, const void* powers, const ptau_kzg_powers* res, const void* coeffs, size_t n,
-                           void* commitment);
+                           void* commitment, bool g2 = false);
 
 int ptau_kzg_commit(ptau_ctx* ctx, const void* powers, const void* coeffs, size_t n, void* commitment) {
   if (!ctx || (!powers && n) || (!coeffs && n) || !commitment) return PTAU_ERR_ARG;
   return kzg_commit_impl(ctx, powers, nullptr, coeffs, n, commitment);
+}
+
+int ptau_msm_g2(ptau_ctx* ctx, const void* points, const void* scalars, size_t n, void* out) {
+  if (!ctx || (!points && n) || (!scalars && n) || !out) return PTAU_ERR_ARG;
+  return kzg_commit_impl(ctx, points, nullptr, scalars, n, out, true);
 }
 
 // The powers of a setup are the same for every commitment: keep a copy on every GPU of the context and send only the
@@ -834,10 +819,15 @@ int ptau_kzg_commit_resident(ptau_ctx* ctx, const ptau_kzg_powers* powers, const
 }
 
 static int kzg_commit_impl(ptau_ctx* ctx, const void* powers, const ptau_kzg_powers* res, const void* coeffs, size_t n,
-                           void* commitment) {
+                           void* commitment, bool g2) {
   // scalars must be canonical (< r), like ark's Fr: checked on the device by the kernel that reads them anyway
+  const size_t rb = g2 ? 200 : 104;
+  const int rw = g2 ? 50 : 26;
   ptau::MsmPlan plan;
-  ptau::msm_g1_plan(n, &plan);
+  if (g2)
+    ptau::msm_g2_plan(n, &plan);
+  else
+    ptau::msm_g1_plan(n, &plan);
   // point indices travel in 31 bits and the bucket lists (n x W entries) are addressed with 32-bit offsets
   if (n >= (1ull << 31) || (uint64_t)n * (uint64_t)plan.W >= (1ull << 32)) return PTAU_ERR_ARG;
   const int G = (ctx->n_gpus > 1 && n >= (size_t)ctx->n_gpus * (1u << 12)) ? ctx->n_gpus : 1;
@@ -850,12 +840,13 @@ static int kzg_commit_impl(ptau_ctx* ctx, const void* powers, const ptau_kzg_pow
     if (res)
       e = msm_issue(ctx->gpu[g], (const uint8_t*)res->d_pts[g] + lo * 104, (const uint8_t*)coeffs + lo * 32, hi - lo, &launches[g], true);
     else
-      e = msm_issue(ctx->gpu[g], (const uint8_t*)powers + lo * 104, (const uint8_t*)coeffs + lo * 32, hi - lo, &launches[g]);
-    ctx->timing.h2d_bytes[g] = (hi - lo) * (res ? 32 : 136);
-    ctx->timing.d2h_bytes[g] = 104;
+      e = msm_issue(ctx->gpu[g], (const uint8_t*)powers + lo * rb, (const uint8_t*)coeffs + lo * 32, hi - lo, &launches[g],
+                    false, g2);
+    ctx->timing.h2d_bytes[g] = (hi - lo) * (res ? 32 : rb + 32);
+    ctx->timing.d2h_bytes[g] = rb;
   }
   bool bad_scalar = false;
-  uint8_t parts[kMaxGpus * 104];
+  uint8_t parts[kMaxGpus * 200];
   for (int g = 0; g < G && e == cudaSuccess; g++) {
     float ms = 0;
     e = msm_wait(ctx->gpu[g], &ms);
@@ -863,8 +854,8 @@ static int kzg_commit_impl(ptau_ctx* ctx, const void* powers, const ptau_kzg_pow
     ctx->timing.gpu_ms[g] = ms;
     ctx->timing.kernel_launches += launches[g];
     if (e == cudaSuccess) {
-      memcpy(parts + g * 104, ctx->gpu[g].h_msm_out, 104);
-      bad_scalar = bad_scalar || ctx->gpu[g].h_msm_out[26] != 0;
+      memcpy(parts + g * rb, ctx->gpu[g].h_msm_out, rb);
+      bad_scalar = bad_scalar || ctx->gpu[g].h_msm_out[rw] != 0;
     }
   }
   if (e == cudaSuccess && bad_scalar) return PTAU_ERR_ARG;
@@ -874,14 +865,14 @@ static int kzg_commit_impl(ptau_ctx* ctx, const void* powers, const ptau_kzg_pow
     for (int g = 0; g < G; g++) ones[g * 32] = 1;
     float ms = 0;
     int nl = 0;
-    e = msm_issue(ctx->gpu[0], parts, ones, (size_t)G, &nl);
+    e = msm_issue(ctx->gpu[0], parts, ones, (size_t)G, &nl, false, g2);
     if (e == cudaSuccess) e = msm_wait(ctx->gpu[0], &ms);
     ctx->timing.kernel_ms[0] += ms;
     ctx->timing.gpu_ms[0] += ms;
     ctx->timing.kernel_launches += nl;
-    if (e == cudaSuccess) memcpy(commitment, ctx->gpu[0].h_msm_out, 104);
+    if (e == cudaSuccess) memcpy(commitment, ctx->gpu[0].h_msm_out, rb);
   } else if (e == cudaSuccess) {
-    memcpy(commitment, parts, 104);
+    memcpy(commitment, parts, rb);
   }
   if (e != cudaSuccess) {
     ctx->last_error = std::string("kzg_commit: ") + cudaGetErrorString(e);

@@ -697,6 +697,40 @@ __global__ void __launch_bounds__(256) msm_digits(const uint32_t* __restrict__ p
   }
 }
 
+// the same over 50-word G2 records (only the position of the infinity flag differs; kept apart so that the
+// G1 kernel keeps its code)
+template <bool SCATTER>
+__global__ void __launch_bounds__(256) msm_g2_digits(const uint32_t* __restrict__ pts, const uint32_t* __restrict__ scalars,
+                                                  uint64_t n, MsmGeom g, uint32_t* __restrict__ cnt,
+                                                  uint32_t* __restrict__ entries, uint32_t* __restrict__ bad) {
+  const uint64_t i = (uint64_t)blockIdx.x * 256 + threadIdx.x;
+  if (i >= n) return;
+  const uint32_t* k = scalars + i * 8;
+  if (!SCATTER) {
+    uint32_t bf = 0;  // k - r borrows  <=>  k < r
+#pragma unroll
+    for (int j = 0; j < 8; j++) {
+      uint64_t t = (uint64_t)k[j] - K_R_ORDER_D[j] - bf;
+      bf = (uint32_t)(t >> 63);
+    }
+    if (!bf) *bad = 1u;
+  }
+  if (pts[i * 50 + 48] & 0xffu) return;  // a point flagged infinity contributes nothing
+  uint32_t carry = 0, base = 0;
+  int bit = 0;
+  for (int w = 0; w < g.W; w++) {
+    const int cw = w < g.a ? g.c : g.c - 1;
+    int d = msm_digit(k, bit, cw, carry);
+    if (d != 0) {
+      uint32_t b = base + (uint32_t)(d < 0 ? -d : d) - 1u;
+      uint32_t pos = atomicAdd(&cnt[b], 1u);
+      if (SCATTER) entries[pos] = (uint32_t)i | (d < 0 ? 0x80000000u : 0u);
+    }
+    bit += cw;
+    base += 1u << (cw - 1);
+  }
+}
+
 // exclusive scan of cnt[0..m) into off[0..m], off[m] = total; cur[] = copy of off[] (scatter cursors).
 // One block walks the array in coalesced tiles of 1024 x 4 counters (m <= 2^19 + 1: a few hundred tiles).
 __global__ void __launch_bounds__(1024) msm_scan(const uint32_t* __restrict__ cnt, uint32_t m, uint32_t* __restrict__ off,
@@ -855,7 +889,8 @@ __global__ void msm_finish(const uint32_t* __restrict__ wsum, int W, uint32_t* _
   msm_finish_item(wsum, W, out);
 }
 
-void msm_g1_plan(uint64_t n, MsmPlan* p) {
+// scratch layout for n terms; jac_bytes = 144 (G1) or 288 (G2) per Jacobian bucket / segment / window record
+static void msm_plan(uint64_t n, uint64_t jac_bytes, MsmPlan* p) {
   const MsmGeom g = msm_geometry(n);
   p->c = g.c;
   p->W = g.W;
@@ -871,16 +906,20 @@ void msm_g1_plan(uint64_t n, MsmPlan* p) {
   p->off_cursor = p->off_offsets + up((p->buckets + 1) * 4);
   p->off_entries = p->off_cursor + up((p->buckets + 1) * 4);
   p->off_buckets = p->off_entries + up((n ? n : 1) * (uint64_t)p->W * 4);
-  p->off_segments = p->off_buckets + up(p->buckets * 144);
-  p->off_wsum = p->off_segments + up(p->segments * 144);
-  p->off_order = p->off_wsum + up((uint64_t)p->W * 144);
+  p->off_segments = p->off_buckets + up(p->buckets * jac_bytes);
+  p->off_wsum = p->off_segments + up(p->segments * jac_bytes);
+  p->off_order = p->off_wsum + up((uint64_t)p->W * jac_bytes);
   p->scratch_bytes = p->off_order + up(p->buckets * 4);
 }
+void msm_g1_plan(uint64_t n, MsmPlan* p) { msm_plan(n, 144, p); }
+void msm_g2_plan(uint64_t n, MsmPlan* p) { msm_plan(n, 288, p); }
 
-cudaError_t launch_msm_g1(const void* d_pts, const void* d_scalars, uint64_t n, void* d_scratch, void* d_out,
-                          int* launches, cudaStream_t stream) {
+// steps 1-7 of either group; d_out: the result record (26 / 50 words) followed by the "scalar >= r" word
+template <bool G2>
+static cudaError_t launch_msm(const void* d_pts, const void* d_scalars, uint64_t n, void* d_scratch, void* d_out,
+                              int* launches, cudaStream_t stream) {
   MsmPlan p;
-  msm_g1_plan(n, &p);
+  msm_plan(n, G2 ? 288 : 144, &p);
   MsmGeom g;
   g.c = p.c;
   g.W = p.W;
@@ -902,18 +941,24 @@ cudaError_t launch_msm_g1(const void* d_pts, const void* d_scalars, uint64_t n, 
   const uint32_t* sc = (const uint32_t*)d_scalars;
   cudaError_t e = cudaMemsetAsync(counts, 0, (size_t)(m + 1 + PTAU_MSM_BINS) * 4, stream);
   if (e != cudaSuccess) return e;
-  uint32_t* bad = (uint32_t*)d_out + 26;  // d_out: 26 words of the result record + the "scalar >= r" flag
+  uint32_t* bad = (uint32_t*)d_out + (G2 ? 50 : 26);
   e = cudaMemsetAsync(bad, 0, 4, stream);
   if (e != cudaSuccess) return e;
   const unsigned gn = (unsigned)((n + 255) / 256);
   int nl = 0;
   if (gn) {
-    msm_digits<false><<<gn, 256, 0, stream>>>(pts, sc, n, g, counts, nullptr, bad);
+    if (G2)
+      msm_g2_digits<false><<<gn, 256, 0, stream>>>(pts, sc, n, g, counts, nullptr, bad);
+    else
+      msm_digits<false><<<gn, 256, 0, stream>>>(pts, sc, n, g, counts, nullptr, bad);
     nl++;
   }
   msm_scan<<<1, 1024, 0, stream>>>(counts, m, offsets, cursor);
   if (gn) {
-    msm_digits<true><<<gn, 256, 0, stream>>>(pts, sc, n, g, cursor, entries, nullptr);
+    if (G2)
+      msm_g2_digits<true><<<gn, 256, 0, stream>>>(pts, sc, n, g, cursor, entries, nullptr);
+    else
+      msm_digits<true><<<gn, 256, 0, stream>>>(pts, sc, n, g, cursor, entries, nullptr);
     nl++;
   }
   const unsigned gs = (m + PTAU_MSM_BINS - 1) / PTAU_MSM_BINS;
@@ -921,14 +966,27 @@ cudaError_t launch_msm_g1(const void* d_pts, const void* d_scalars, uint64_t n, 
   msm_size_scan<<<1, PTAU_MSM_BINS, 0, stream>>>(size_hist);
   msm_size_scatter<<<gs, PTAU_MSM_BINS, 0, stream>>>(counts, m, size_hist, order);
   nl += 3;
-  msm_bucket_sum<<<(m + PTAU_BLOCK - 1) / PTAU_BLOCK, PTAU_BLOCK, 0, stream>>>(pts, entries, offsets, order, m, buckets);
   const uint32_t nseg = (uint32_t)p.segments;
-  msm_window_segments<<<(nseg + PTAU_BLOCK - 1) / PTAU_BLOCK, PTAU_BLOCK, 0, stream>>>(buckets, g, nseg, segs);
-  msm_window_sum<<<p.W, PTAU_BLOCK, 0, stream>>>(segs, g, wsum);
-  msm_finish<<<1, 32, 0, stream>>>(wsum, p.W, (uint32_t*)d_out);
+  if (G2) {
+    e = launch_msm_g2_sums(pts, entries, offsets, order, m, buckets, g, nseg, segs, wsum, (uint32_t*)d_out, stream);
+    if (e != cudaSuccess) return e;
+  } else {
+    msm_bucket_sum<<<(m + PTAU_BLOCK - 1) / PTAU_BLOCK, PTAU_BLOCK, 0, stream>>>(pts, entries, offsets, order, m, buckets);
+    msm_window_segments<<<(nseg + PTAU_BLOCK - 1) / PTAU_BLOCK, PTAU_BLOCK, 0, stream>>>(buckets, g, nseg, segs);
+    msm_window_sum<<<p.W, PTAU_BLOCK, 0, stream>>>(segs, g, wsum);
+    msm_finish<<<1, 32, 0, stream>>>(wsum, p.W, (uint32_t*)d_out);
+  }
   nl += 5;
   if (launches) *launches = nl;
   return cudaGetLastError();
+}
+cudaError_t launch_msm_g1(const void* d_pts, const void* d_scalars, uint64_t n, void* d_scratch, void* d_out,
+                          int* launches, cudaStream_t stream) {
+  return launch_msm<false>(d_pts, d_scalars, n, d_scratch, d_out, launches, stream);
+}
+cudaError_t launch_msm_g2(const void* d_pts, const void* d_scalars, uint64_t n, void* d_scratch, void* d_out,
+                          int* launches, cudaStream_t stream) {
+  return launch_msm<true>(d_pts, d_scalars, n, d_scratch, d_out, launches, stream);
 }
 
 // =============================================================================

@@ -5,6 +5,8 @@
 
 namespace ptau {
 
+struct MsmGeom;  // msm_digits.cuh
+
 cudaError_t launch_convert(int group, int in_fmt, int out_fmt, const void* d_in, void* d_out, uint64_t n,
                            uint32_t checks, uint64_t base_index, unsigned long long* d_status,
                            cudaStream_t stream);
@@ -30,6 +32,14 @@ struct MsmPlan {
 void msm_g1_plan(uint64_t n, MsmPlan* plan);
 cudaError_t launch_msm_g1(const void* d_pts, const void* d_scalars, uint64_t n, void* d_scratch, void* d_out,
                           int* launches, cudaStream_t stream);
+// the same over ARK_MONT_LIMBS G2 records (200 B); d_out (51 words): one G2 record and the "scalar >= r" word
+void msm_g2_plan(uint64_t n, MsmPlan* plan);
+cudaError_t launch_msm_g2(const void* d_pts, const void* d_scalars, uint64_t n, void* d_scratch, void* d_out,
+                          int* launches, cudaStream_t stream);
+// msm_g2.cu: steps 4-7 of launch_msm_g2 (bucket sums, window segments, window sums, finish)
+cudaError_t launch_msm_g2_sums(const uint32_t* pts, const uint32_t* entries, const uint32_t* offsets, const uint32_t* order,
+                               uint32_t m, uint32_t* buckets, const MsmGeom& g, uint32_t nseg, uint32_t* segs, uint32_t* wsum,
+                               uint32_t* out, cudaStream_t stream);
 
 // kzg.cu: prod_{k<2} e(P_ik, Q_ik) for n items (d_gt: n x 576 bytes or null, d_is_one: n bytes or null), and
 // KZG10::check for n openings (d_random_v may be null: no hiding), one item per thread
