@@ -408,6 +408,11 @@ static int g2_one(int in_fmt, const uint8_t* in, int out_fmt, uint8_t* out, unsi
     if (inf) { memset(out, 0, 192); out[0] = 0x40; }
     else { limbs_to_be48(out, &xp.c1); limbs_to_be48(out + 48, &xp.c0); limbs_to_be48(out + 96, &yp.c1); limbs_to_be48(out + 144, &yp.c0); }
   } else {
+    /* zcash compressed infinity reaches here with the plain ark zero() = (0, 1): its limbs are Montgomery 0 and 1 */
+    if (st == OK && !have_m) {
+      fq_to_mont(&xm.c0, &xp.c0); fq_to_mont(&xm.c1, &xp.c1); fq_to_mont(&ym.c0, &yp.c0); fq_to_mont(&ym.c1, &yp.c1);
+      have_m = 1;
+    }
     if (!have_m) { memset(&xm, 0, sizeof xm); memset(&ym, 0, sizeof ym); }
     memcpy(out, xm.c0.l, 48); memcpy(out + 48, xm.c1.l, 48); memcpy(out + 96, ym.c0.l, 48); memcpy(out + 144, ym.c1.l, 48);
     memset(out + 192, 0, 8); out[192] = (uint8_t)inf;
