@@ -234,6 +234,20 @@ int ptau_kzg_commit_resident(ptau_ctx* ctx, const ptau_kzg_powers* powers, const
  * proof is ptau_kzg_commit(powers, quotient).  No context needed. */
 int ptau_kzg_quotient(const void* coeffs, size_t n, const void* point, void* quotient_out, void* value_out);
 
+/* KZG10::open of one polynomial at k points on the GPU (ark-poly-commit 0.2 kzg10 `open` /
+ * `compute_witness_polynomial`, reached from src/lib.rs:276).  For each z_j:
+ *   values_out[j] = p(z_j),  proofs_out[j] = sum_i q_{j,i} powers_of_g[i],  q_j = (p - p(z_j)) / (X - z_j);
+ * with n_b > 0 blinding coefficients also random_v_out[j] = b(z_j) and proofs_out[j] += the same for b over
+ * gamma_powers.  powers / gamma_powers: device-resident (ptau_kzg_powers_upload; gamma_powers may be NULL iff n_b = 0).
+ * coeffs n, blinding n_b, points k scalars: 32 B LE, < r.  proofs_out k x 104 (ARK_MONT_LIMBS), values_out and
+ * random_v_out k x 32 (random_v_out NULL iff n_b = 0).  n > powers' count or n_b > gamma_powers' count
+ * (ark: TooManyCoefficients), a non-canonical scalar, or handles of another context: PTAU_ERR_ARG.
+ * The quotient is computed on the device (a parallel scan) straight into the MSM's scalars; the points are split in
+ * contiguous ranges over the context's GPUs, each opening its points against its own copy of the powers. */
+int ptau_kzg_open(ptau_ctx* ctx, const ptau_kzg_powers* powers, const ptau_kzg_powers* gamma_powers,
+                  const void* coeffs, size_t n, const void* blinding, size_t n_b, const void* points, size_t k,
+                  void* proofs_out, void* values_out, void* random_v_out);
+
 /* KZG10::check for n openings in parallel -- ark-poly-commit 0.2 kzg10 `check`, the call the reference's
  * consumer code makes at /root/reference/src/lib.rs:276-286:
  *     e(C_i - [v_i] g - [rv_i] gamma_g, h) == e(w_i, beta_h - [z_i] h)

@@ -398,16 +398,47 @@ class KZG10:
     def open(powers: "Powers", coeffs, point: int, blinding=None, ctx: Optional["Context"] = None):
         """KZG10::open: witness commitment w = commit((p - p(z)) / (X - z)) (+ the blinding
         polynomial's witness on powers_of_gamma_g).  Returns (value p(z), proof record,
-        random_v = blinding(z) or None)."""
-        ctx = ctx or default_context()
-        value, q = KZG10._quotient([int(c) % R_ORDER for c in coeffs], int(point) % R_ORDER)
-        pairs = [(powers.powers_of_g, q)]
-        random_v = None
-        if blinding:
-            random_v, rq = KZG10._quotient([int(c) % R_ORDER for c in blinding], int(point) % R_ORDER)
-            pairs.append((powers.powers_of_gamma_g, rq))
-        return value, KZG10._msm(ctx, pairs), random_v
+        random_v = blinding(z) or None).  One point of open_many."""
+        values, proofs, random_vs = KZG10.open_many(powers, coeffs, [point], blinding=blinding, ctx=ctx)
+        return values[0], proofs[0], None if random_vs is None else random_vs[0]
 
+    @staticmethod
+    def open_many(powers: "Powers", coeffs, points, blinding=None, ctx: Optional["Context"] = None):
+        """KZG10::open of one polynomial at every point of `points` in one call (ptau_kzg_open): the witness
+        polynomials are computed on the GPU and committed to there, point after point, with no host round trip.
+        coeffs / points / blinding: ints (taken mod r) or [m, 32] u8 arrays of little-endian scalars < r.  powers:
+        Powers of arrays (the first len(coeffs) / len(blinding) powers are uploaded for the call) or
+        Powers.to_device().  Returns (values: list of p(z_j), proofs: u8 [k, 104], random_vs: list of b(z_j) or
+        None without blinding).  More coefficients than powers raises PtauError (ark: TooManyCoefficients)."""
+        ctx = ctx or default_context()
+        c, z = KZG10._scalars(coeffs), KZG10._scalars(points)
+        b = KZG10._scalars(blinding) if blinding is not None and len(blinding) else None
+        n, k, n_b = c.size // 32, z.size // 32, 0 if b is None else b.size // 32
+
+        def resident(pts, m):
+            if isinstance(pts, ResidentPoints):
+                return pts
+            if m > len(pts):
+                raise PtauError(_ffi.ERR_ARG, detail="polynomial degree exceeds the supported degree")  # TooManyCoefficients
+            return ResidentPoints(ctx, np.asarray(pts)[:m])
+
+        pg = resident(powers.powers_of_g, n)
+        gg = resident(powers.powers_of_gamma_g, n_b) if n_b else None
+        proofs = np.zeros((k, 104), dtype=np.uint8)
+        vals = np.zeros(k * 32, dtype=np.uint8)
+        rvs = np.zeros(k * 32, dtype=np.uint8) if n_b else None
+        rc = _ffi.lib().ptau_kzg_open(ctx._h, pg._h, gg._h if n_b else None, _ptr(c) if n else None, n,
+                                      _ptr(b) if n_b else None, n_b, _ptr(z) if k else None, k,
+                                      _ptr(proofs) if k else None, _ptr(vals) if k else None,
+                                      _ptr(rvs) if (n_b and k) else None)
+        if rc != 0:
+            ctx._raise(rc)
+
+        def ints(a):
+            raw = a.tobytes()
+            return [int.from_bytes(raw[32 * i:32 * i + 32], "little") for i in range(k)]
+
+        return ints(vals), proofs, None if rvs is None else ints(rvs)
 
     @staticmethod
     def _scalars(vals) -> np.ndarray:

@@ -125,6 +125,11 @@ _SIGNATURES = {
     "ptau_kzg_powers_free": (None, [C.c_void_p]),
     "ptau_kzg_commit_resident": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "ptau_kzg_quotient": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "ptau_kzg_open": (
+        C.c_int,
+        [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t,
+         C.c_void_p, C.c_void_p, C.c_void_p],
+    ),
     "ptau_kzg_check": (C.c_int, [C.c_void_p] * 8 + [C.c_size_t, C.c_void_p]),
     "ptau_pairing_product2": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]),
     "ptau_g2_prepare": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]),

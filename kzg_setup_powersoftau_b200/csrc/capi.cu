@@ -255,6 +255,7 @@ void ptau_destroy(ptau_ctx* ctx) {
     if (s.d_msm_out) cudaFree(s.d_msm_out);
     if (s.h_msm_sc) cudaFreeHost(s.h_msm_sc);
     if (s.h_msm_out) cudaFreeHost(s.h_msm_out);
+    if (s.d_open) cudaFree(s.d_open);
   }
   delete ctx;
 }
@@ -1069,6 +1070,153 @@ int ptau_kzg_quotient(const void* coeffs, size_t n, const void* point, void* quo
   Fr v = fr_add_mod(c0, fr_mont_mul(carry, zm));
   memcpy(value_out, v.l, 32);
   return PTAU_OK;
+}
+
+namespace {
+// the multipliers of the quotient scan for the point z: out[s] = z^(2^s) R mod r
+void kzg_zpow(const void* z, uint32_t (*out)[8]) {
+  Fr p = fr_to_mont(fr_from_le32((const uint8_t*)z));
+  for (int s = 0; s < ptau::kKzgZPowCount; s++) {
+    memcpy(out[s], p.l, 32);
+    p = fr_mont_mul(p, p);
+  }
+}
+// point indices travel in 31 bits and the bucket lists (n x W entries) are addressed with 32-bit offsets
+bool msm_fits(size_t n) {
+  ptau::MsmPlan plan;
+  ptau::msm_g1_plan(n, &plan);
+  return n < (1ull << 31) && (uint64_t)n * (uint64_t)plan.W < (1ull << 32);
+}
+size_t up256(size_t v) { return (v + 255) & ~(size_t)255; }
+}  // namespace
+
+// Per GPU, for its contiguous range of the points: the coefficients (and blinding coefficients) are uploaded once;
+// then, per point and on one stream with no host round trip, the quotient kernels write (p - p(z)) / (X - z) into the
+// MSM's scalar buffer and the bucket MSM runs over the resident powers.  With blinding the same follows for b over
+// gamma_powers, and a 2-term MSM with unit scalars adds the two results.  Values, proofs and the "coefficient >= r"
+// word come back once at the end.
+int ptau_kzg_open(ptau_ctx* ctx, const ptau_kzg_powers* powers, const ptau_kzg_powers* gamma_powers, const void* coeffs,
+                  size_t n, const void* blinding, size_t n_b, const void* points, size_t k, void* proofs_out,
+                  void* values_out, void* random_v_out) {
+  if (!ctx || !powers || powers->ctx != ctx || (gamma_powers && gamma_powers->ctx != ctx)) return PTAU_ERR_ARG;
+  if (n > powers->n || (n_b && (!gamma_powers || n_b > gamma_powers->n))) return PTAU_ERR_ARG;  // TooManyCoefficients
+  if ((n && !coeffs) || (n_b && !blinding)) return PTAU_ERR_ARG;
+  if (k && (!points || !proofs_out || !values_out || (n_b > 0) != (random_v_out != nullptr))) return PTAU_ERR_ARG;
+  if (!msm_fits(n) || !msm_fits(n_b)) return PTAU_ERR_ARG;
+  auto t0 = std::chrono::steady_clock::now();
+  memset(&ctx->timing, 0, sizeof(ctx->timing));
+  ctx->timing.n_gpus = ctx->n_gpus;
+  if (k == 0) return PTAU_OK;
+  if (!scalars_canonical(points, k)) return PTAU_ERR_ARG;
+  const int G = (size_t)ctx->n_gpus < k ? ctx->n_gpus : (int)k;
+  const size_t n_max = n > n_b ? n : n_b, nq = n > 1 ? n - 1 : 0, nbq = n_b > 1 ? n_b - 1 : 0;
+  size_t scratch = 0;
+  for (size_t m : {nq, nbq, (size_t)2}) {
+    ptau::MsmPlan plan;
+    ptau::msm_g1_plan(m, &plan);
+    scratch = plan.scratch_bytes > scratch ? plan.scratch_bytes : scratch;
+  }
+  // staging in GPU 0's pinned scalar buffer (portable: every GPU copies from it): coefficients | blinding | 1, 1
+  GpuSlot& s0 = ctx->gpu[0];
+  const size_t h_b = n * 32, h_one = h_b + n_b * 32, h_len = h_one + 64;
+  cudaError_t e = cudaSetDevice(s0.device);
+  if (e == cudaSuccess) e = grow(&s0.h_msm_sc, &s0.cap_h_msm_sc, h_len, true);
+  if (e != cudaSuccess) {
+    ctx->last_error = std::string("kzg_open: ") + cudaGetErrorString(e);
+    return PTAU_ERR_CUDA;
+  }
+  uint8_t* stage = (uint8_t*)s0.h_msm_sc;
+  if (n) copy_parts(stage, coeffs, n * 32);
+  if (n_b) copy_parts(stage + h_b, blinding, n_b * 32);
+  memset(stage + h_one, 0, 64);
+  stage[h_one] = stage[h_one + 32] = 1;
+  // device layout of d_open, per GPU: coefficients | blinding | 1, 1 | chunk sums | MSM results r0, r1 | the pair
+  // (r0, r1) as consecutive records | "coefficient >= r" word | values | random values | proofs
+  const size_t d_b = up256(n * 32), d_one = d_b + up256(n_b * 32), d_sums = d_one + 256,
+               d_r0 = d_sums + up256(ptau::kzg_quotient_sums_bytes(n_max)), d_r1 = d_r0 + 256, d_pair = d_r1 + 256,
+               d_bad = d_pair + 256, d_val = d_bad + 256;
+  int launches = 0;
+  for (int g = 0; g < G && e == cudaSuccess; g++) {
+    GpuSlot& s = ctx->gpu[g];
+    const size_t lo = k * g / G, cnt = k * (g + 1) / G - lo;
+    const size_t d_rv = d_val + up256(cnt * 32), d_pf = d_rv + up256(cnt * 32), d_len = d_pf + cnt * 104;
+    cudaStream_t st = s.stream[0];
+    e = cudaSetDevice(s.device);
+    if (e == cudaSuccess) e = grow(&s.d_open, &s.cap_open, d_len);
+    if (e == cudaSuccess) e = grow(&s.d_msm_sc, &s.cap_msm_sc, n_max * 32 + 16);
+    if (e == cudaSuccess) e = grow(&s.d_msm_scratch, &s.cap_msm_scratch, scratch);
+    if (e == cudaSuccess && !s.h_msm_out) e = cudaHostAlloc((void**)&s.h_msm_out, 256, cudaHostAllocPortable);
+    if (e != cudaSuccess) break;
+    uint8_t* d = (uint8_t*)s.d_open;
+    uint32_t* bad = (uint32_t*)(d + d_bad);
+    e = cudaEventRecord(s.ev_first, st);
+    if (e == cudaSuccess && n) e = cudaMemcpyAsync(d, stage, n * 32, cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess && n_b) e = cudaMemcpyAsync(d + d_b, stage + h_b, n_b * 32, cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d + d_one, stage + h_one, 64, cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(bad, 0, 4, st);
+    if (e == cudaSuccess) e = cudaEventRecord(s.ev_k0[0], st);
+    for (size_t j = 0; j < cnt && e == cudaSuccess; j++) {
+      uint32_t zp[ptau::kKzgZPowCount][8];
+      kzg_zpow((const uint8_t*)points + (lo + j) * 32, zp);
+      int nl = 0;
+      e = ptau::launch_kzg_quotient(d, n, zp, d + d_sums, s.d_msm_sc, d + d_val + j * 32, bad, &nl, st);
+      launches += nl;
+      if (e == cudaSuccess) e = ptau::launch_msm_g1(powers->d_pts[g], s.d_msm_sc, nq, s.d_msm_scratch, d + d_r0, &nl, st);
+      launches += nl;
+      if (n_b) {
+        if (e == cudaSuccess)
+          e = ptau::launch_kzg_quotient(d + d_b, n_b, zp, d + d_sums, s.d_msm_sc, d + d_rv + j * 32, bad, &nl, st);
+        launches += nl;
+        if (e == cudaSuccess)
+          e = ptau::launch_msm_g1(gamma_powers->d_pts[g], s.d_msm_sc, nbq, s.d_msm_scratch, d + d_r1, &nl, st);
+        launches += nl;
+        if (e == cudaSuccess) e = cudaMemcpyAsync(d + d_pair, d + d_r0, 104, cudaMemcpyDeviceToDevice, st);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(d + d_pair + 104, d + d_r1, 104, cudaMemcpyDeviceToDevice, st);
+        if (e == cudaSuccess) e = ptau::launch_msm_g1(d + d_pair, d + d_one, 2, s.d_msm_scratch, d + d_r0, &nl, st);
+        launches += nl;
+      }
+      if (e == cudaSuccess) e = cudaMemcpyAsync(d + d_pf + j * 104, d + d_r0, 104, cudaMemcpyDeviceToDevice, st);
+    }
+    if (e == cudaSuccess) e = cudaEventRecord(s.ev_k1[0], st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(s.h_msm_out, bad, 4, cudaMemcpyDeviceToHost, st);
+    ctx->timing.h2d_bytes[g] = (n + n_b) * 32 + 64;
+    ctx->timing.d2h_bytes[g] = cnt * (104 + 32 + (n_b ? 32 : 0)) + 4;
+  }
+  ctx->timing.kernel_launches = launches;
+  // results to the caller's (pageable) memory only once every GPU has its work queued
+  bool bad_coeff = false;
+  for (int g = 0; g < G && e == cudaSuccess; g++) {
+    GpuSlot& s = ctx->gpu[g];
+    const size_t lo = k * g / G, cnt = k * (g + 1) / G - lo;
+    const size_t d_rv = d_val + up256(cnt * 32), d_pf = d_rv + up256(cnt * 32);
+    const uint8_t* d = (const uint8_t*)s.d_open;
+    cudaStream_t st = s.stream[0];
+    e = cudaSetDevice(s.device);
+    if (e == cudaSuccess)
+      e = cudaMemcpyAsync((uint8_t*)proofs_out + lo * 104, d + d_pf, cnt * 104, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess)
+      e = cudaMemcpyAsync((uint8_t*)values_out + lo * 32, d + d_val, cnt * 32, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess && n_b)
+      e = cudaMemcpyAsync((uint8_t*)random_v_out + lo * 32, d + d_rv, cnt * 32, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaEventRecord(s.ev_last, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    float kms = 0, gms = 0;
+    if (e == cudaSuccess) e = cudaEventElapsedTime(&kms, s.ev_k0[0], s.ev_k1[0]);
+    if (e == cudaSuccess) e = cudaEventElapsedTime(&gms, s.ev_first, s.ev_last);
+    ctx->timing.kernel_ms[g] = kms;
+    ctx->timing.gpu_ms[g] = gms;
+    bad_coeff = bad_coeff || s.h_msm_out[0] != 0;
+  }
+  if (e != cudaSuccess) {
+    for (int g = 0; g < G; g++) {  // nothing may still be using the buffers when the call returns
+      cudaSetDevice(ctx->gpu[g].device);
+      cudaStreamSynchronize(ctx->gpu[g].stream[0]);
+    }
+    ctx->last_error = std::string("kzg_open: ") + cudaGetErrorString(e);
+    return PTAU_ERR_CUDA;
+  }
+  ctx->timing.wall_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+  return bad_coeff ? PTAU_ERR_ARG : PTAU_OK;
 }
 
 int ptau_selftest_fq_op(ptau_ctx* ctx, int gpu, int op, const void* a, const void* b, void* out, size_t n) {

@@ -31,6 +31,9 @@ struct GpuSlot {
   void *d_msm_pts = nullptr, *d_msm_sc = nullptr, *d_msm_scratch = nullptr, *d_msm_out = nullptr, *h_msm_sc = nullptr;
   size_t cap_msm_pts = 0, cap_msm_sc = 0, cap_msm_scratch = 0, cap_h_msm_sc = 0;
   uint32_t* h_msm_out = nullptr;  // pinned: the result record (26 or 50 words) + 1 word "a scalar was >= r"
+  // KZG10::open: coefficients, points, chunk sums, values and proofs of one call, kept and grown like the MSM buffers
+  void* d_open = nullptr;
+  size_t cap_open = 0;
 };
 
 }  // namespace ptau

@@ -408,53 +408,10 @@ struct FrParams {
   uint32_t pw[64][8];     // step^(2^j), Montgomery form
 };
 
-__constant__ uint32_t K_FR_MOD[8] = {0x00000001u, 0xffffffffu, 0xfffe5bfeu, 0x53bda402u,
-                                     0x09a1d805u, 0x3339d808u, 0x299d7d48u, 0x73eda753u};
-#define PTAU_FR_M0 0xffffffffu  // -r^-1 mod 2^32
-
-// Montgomery product in Fr (R = 2^256), plain 64-bit arithmetic: a few dozen calls per point
-static __device__ __noinline__ void fr_mul(uint32_t* r, const uint32_t* a, const uint32_t* b) {
-  uint32_t t[10];
-#pragma unroll
-  for (int i = 0; i < 10; i++) t[i] = 0;
-#pragma unroll 1
-  for (int i = 0; i < 8; i++) {
-    uint64_t c = 0;
-#pragma unroll
-    for (int j = 0; j < 8; j++) {
-      c += (uint64_t)a[j] * b[i] + t[j];
-      t[j] = (uint32_t)c;
-      c >>= 32;
-    }
-    c += t[8];
-    t[8] = (uint32_t)c;
-    t[9] = (uint32_t)(c >> 32);
-    uint32_t m = t[0] * PTAU_FR_M0;
-    c = (uint64_t)m * K_FR_MOD[0] + t[0];
-    c >>= 32;
-#pragma unroll
-    for (int j = 1; j < 8; j++) {
-      c += (uint64_t)m * K_FR_MOD[j] + t[j];
-      t[j - 1] = (uint32_t)c;
-      c >>= 32;
-    }
-    c += t[8];
-    t[7] = (uint32_t)c;
-    t[8] = t[9] + (uint32_t)(c >> 32);
-  }
-  // conditional subtraction
-  uint32_t d[8];
-  uint32_t bw = 0;
-#pragma unroll
-  for (int i = 0; i < 8; i++) {
-    uint64_t x = (uint64_t)t[i] - K_FR_MOD[i] - bw;
-    d[i] = (uint32_t)x;
-    bw = (uint32_t)(x >> 63);
-  }
-  bool ge = t[8] != 0 || bw == 0;
-#pragma unroll
-  for (int i = 0; i < 8; i++) r[i] = ge ? d[i] : t[i];
-}
+}  // namespace ptau
+// K_FR_MOD, fr_mul; included here so that the constant bank keeps its layout
+#include "fr.cuh"
+namespace ptau {
 
 template <class F>
 struct FieldInv;

@@ -52,6 +52,14 @@ cudaError_t launch_kzg_check(const void* d_vk_g1, const void* d_vk_g2, const voi
                              const void* d_values, const void* d_proofs, const void* d_random_v, const void* d_tbl,
                              uint64_t n, void* d_ok, cudaStream_t stream);
 
+// kzg_open.cu: the witness polynomial (p - p(z)) / (X - z) of n > 0 canonical 32-byte scalars d_coeffs into d_q (n - 1
+// scalars, the layout launch_msm_g1 reads) and p(z) into d_value; zpow[s] = z^(2^s) R mod r for s < kKzgZPowCount; d_sums:
+// kzg_quotient_sums_bytes(n) of scratch; *d_bad is set to 1 when a coefficient is >= r.  n == 0: p(z) = 0, no launch.
+constexpr int kKzgZPowCount = 32;
+size_t kzg_quotient_sums_bytes(uint64_t n);
+cudaError_t launch_kzg_quotient(const void* d_coeffs, uint64_t n, const uint32_t (*zpow)[8], void* d_sums, void* d_q,
+                                void* d_value, uint32_t* d_bad, int* launches, cudaStream_t stream);
+
 // G2Prepared (ark-ec 0.2): n x 68 x 288 bytes of line coefficients + n infinity bytes
 cudaError_t launch_g2_prepare(const void* d_g2, uint64_t n, void* d_coeffs, void* d_infinity, cudaStream_t stream);
 

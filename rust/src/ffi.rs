@@ -90,6 +90,11 @@ extern "C" {
     pub fn ptau_kzg_powers_free(powers: *mut ptau_kzg_powers);
     pub fn ptau_kzg_commit_resident(ctx: *mut ptau_ctx, powers: *const ptau_kzg_powers, coeffs: *const c_void, n: usize, commitment: *mut c_void) -> c_int;
     pub fn ptau_kzg_quotient(coeffs: *const c_void, n: usize, point: *const c_void, quotient_out: *mut c_void, value_out: *mut c_void) -> c_int;
+    pub fn ptau_kzg_open(
+        ctx: *mut ptau_ctx, powers: *const ptau_kzg_powers, gamma_powers: *const ptau_kzg_powers, coeffs: *const c_void,
+        n: usize, blinding: *const c_void, n_b: usize, points: *const c_void, k: usize, proofs_out: *mut c_void,
+        values_out: *mut c_void, random_v_out: *mut c_void,
+    ) -> c_int;
     pub fn ptau_kzg_check(
         ctx: *mut ptau_ctx, vk_g1: *const c_void, vk_g2: *const c_void, comms: *const c_void, points: *const c_void,
         values: *const c_void, proofs_w: *const c_void, random_v: *const c_void, n: usize, ok: *mut u8,
