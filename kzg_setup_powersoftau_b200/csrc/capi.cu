@@ -21,55 +21,86 @@
 
 #include "context.h"
 #include "kernels.h"
+#include "layout.h"
 
-using ptau::GpuSlot;
-using ptau::kBufs;
-using ptau::kMaxGpus;
+using namespace ptau;
 
 namespace {
 
 constexpr size_t kEdgePoints = 148 * 2 * 128;  // one wave of convert-kernel blocks on a B200
 
-#define CUDA_TRY(ctx, expr)                                                          \
-  do {                                                                               \
-    cudaError_t _e = (expr);                                                         \
-    if (_e != cudaSuccess) {                                                         \
-      if (ctx) (ctx)->last_error = std::string(#expr) + ": " + cudaGetErrorString(_e); \
-      return PTAU_ERR_CUDA;                                                          \
-    }                                                                                \
-  } while (0)
-
-int rec_size(int group, int fmt) {
-  if (group != PTAU_G1 && group != PTAU_G2) return 0;
-  bool g1 = group == PTAU_G1;
-  switch (fmt) {
-    case PTAU_FMT_ZCASH_UNCOMPRESSED:
-    case PTAU_FMT_ARK_UNCOMPRESSED:
-      return g1 ? 96 : 192;
-    case PTAU_FMT_ZCASH_COMPRESSED:
-      return g1 ? 48 : 96;
-    case PTAU_FMT_ARK_MONT_LIMBS:
-      return g1 ? 104 : 200;
+// the double buffers d_in or d_out of a slot, each at least `need` bytes; the capacity reads 0 until all of them are
+// allocated, so a failed call leaves no buffer a later call would trust
+cudaError_t ensure_buffers(void* (&d)[kBufs], size_t* cap, size_t need) {
+  if (need <= *cap) return cudaSuccess;
+  *cap = 0;
+  for (int b = 0; b < kBufs; b++) {
+    cudaError_t e = d[b] ? cudaFree(d[b]) : cudaSuccess;
+    d[b] = nullptr;
+    if (e == cudaSuccess) e = cudaMalloc(&d[b], need);
+    if (e != cudaSuccess) return e;
   }
-  return 0;
+  *cap = need;
+  return cudaSuccess;
 }
 
-int ensure_buffers(ptau_ctx* ctx, GpuSlot& s, size_t need_in, size_t need_out) {
-  if (need_in > s.cap_in) {
-    for (int b = 0; b < kBufs; b++) {
-      if (s.d_in[b]) CUDA_TRY(ctx, cudaFree(s.d_in[b]));
-      s.d_in[b] = nullptr;
-      CUDA_TRY(ctx, cudaMalloc(&s.d_in[b], need_in));
-    }
-    s.cap_in = need_in;
+// device copies of a list of host arrays, freed together
+struct DevArgs {
+  std::vector<void*> ptrs;
+  ~DevArgs() {
+    for (void* p : ptrs) cudaFree(p);
   }
-  if (need_out > s.cap_out) {
-    for (int b = 0; b < kBufs; b++) {
-      if (s.d_out[b]) CUDA_TRY(ctx, cudaFree(s.d_out[b]));
-      s.d_out[b] = nullptr;
-      CUDA_TRY(ctx, cudaMalloc(&s.d_out[b], need_out));
-    }
-    s.cap_out = need_out;
+  cudaError_t push(const void* host, size_t bytes, cudaStream_t st, void** out) {
+    void* d = nullptr;
+    cudaError_t e = cudaMalloc(&d, bytes ? bytes : 16);
+    if (e != cudaSuccess) return e;
+    ptrs.push_back(d);
+    if (host && bytes) e = cudaMemcpyAsync(d, host, bytes, cudaMemcpyHostToDevice, st);
+    *out = d;
+    return e;
+  }
+};
+
+// A device buffer of launch_once: uploaded from `in` before the launch and/or copied to `out` after it.  With neither,
+// nothing is allocated and *dev stays null.
+struct LaunchBuf {
+  const void* in;
+  void* out;
+  size_t bytes;
+  void** dev;
+};
+// One launch on the first stream of GPU `gpu` over freshly allocated buffers, their copies back and a synchronise.
+// With `timed` the launch is timed and ctx->timing describes the call.
+template <class Launch>
+int launch_once(ptau_ctx* ctx, int gpu, const char* where, bool timed, std::initializer_list<LaunchBuf> bufs,
+                Launch launch) {
+  GpuSlot& s = ctx->gpu[gpu];
+  const cudaStream_t st = s.stream[0];
+  DevArgs a;
+  size_t h2d = 0, d2h = 0;
+  cudaError_t e = cudaSetDevice(s.device);
+  for (const LaunchBuf& b : bufs) {
+    if (e == cudaSuccess && (b.in || b.out)) e = a.push(b.in, b.bytes, st, b.dev);
+    h2d += b.in ? b.bytes : 0;
+  }
+  if (e == cudaSuccess && timed) e = cudaEventRecord(s.ev_k0[0], st);
+  if (e == cudaSuccess) e = launch(st);
+  if (e == cudaSuccess && timed) e = cudaEventRecord(s.ev_k1[0], st);
+  for (const LaunchBuf& b : bufs) {
+    if (e == cudaSuccess && b.out) e = cudaMemcpyAsync(b.out, *b.dev, b.bytes, cudaMemcpyDeviceToHost, st);
+    d2h += b.out ? b.bytes : 0;
+  }
+  if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+  float ms = 0;
+  if (e == cudaSuccess && timed) e = cudaEventElapsedTime(&ms, s.ev_k0[0], s.ev_k1[0]);
+  if (e != cudaSuccess) return cuda_fail(ctx, where, e);
+  if (timed) {
+    timing_reset(ctx);
+    ctx->timing.kernel_ms[gpu] = ms;
+    ctx->timing.gpu_ms[gpu] = ms;
+    ctx->timing.kernel_launches = 1;
+    ctx->timing.h2d_bytes[gpu] = h2d;
+    ctx->timing.d2h_bytes[gpu] = d2h;
   }
   return PTAU_OK;
 }
@@ -158,10 +189,6 @@ Fr fr_add_mod(const Fr& a, const Fr& b) {
   }
   return r;
 }
-struct Section {
-  int group;
-  uint64_t count;
-};
 
 }  // namespace
 
@@ -284,13 +311,12 @@ int ptau_host_unregister(void* p) { return cudaHostUnregister(p) == cudaSuccess 
 size_t ptau_record_size(int group, int fmt) { return (size_t)rec_size(group, fmt); }
 
 uint64_t ptau_response_size(uint64_t n) {
-  return 64 + (2 * n - 1) * 48 + n * 96 + n * 48 + n * 48 + 96 + (3 * 192 + 6 * 96);
+  return ptau::kResponseHash + ptau::response_bytes(n, PTAU_FMT_ZCASH_COMPRESSED) + ptau::kResponsePubkey;
 }
-uint64_t ptau_uncompressed_size(uint64_t n) { return (2 * n - 1) * 96 + n * 192 + n * 96 + n * 96 + 192; }
+uint64_t ptau_uncompressed_size(uint64_t n) { return ptau::response_bytes(n, PTAU_FMT_ZCASH_UNCOMPRESSED); }
 uint64_t ptau_setup_size(int variant, uint64_t n) {
-  if (variant == PTAU_VARIANT_KGZ) return (2 * n - 1) * 96 + n * 96 + 96 + 96 + 192 + 192;
-  if (variant == PTAU_VARIANT_FASTKGZ) return (2 * n - 1) * 96 + n * 96 + 192 + 192 + n * 192;
-  return 0;
+  if (variant != PTAU_VARIANT_KGZ && variant != PTAU_VARIANT_FASTKGZ) return 0;
+  return ptau::setup_layout(variant, n).bytes();
 }
 
 int ptau_status_decode(uint64_t status, uint64_t* bad_index) {
@@ -319,8 +345,7 @@ int ptau_convert(ptau_ctx* ctx, int group, int in_fmt, const void* in, int out_f
   const int G = ctx->n_gpus;
   const size_t chunk = ctx->chunk_points;
   ptau_timing& tm = ctx->timing;
-  memset(&tm, 0, sizeof(tm));
-  tm.n_gpus = G;
+  timing_reset(ctx);
 
   struct Range {
     size_t lo, hi, next;
@@ -328,15 +353,13 @@ int ptau_convert(ptau_ctx* ctx, int group, int in_fmt, const void* in, int out_f
   } rg[kMaxGpus];
   const unsigned long long none = PTAU_STATUS_NONE;
   for (int g = 0; g < G; g++) {
-    rg[g].lo = (size_t)(((unsigned __int128)n_points * g) / G);
-    rg[g].hi = (size_t)(((unsigned __int128)n_points * (g + 1)) / G);
-    rg[g].next = rg[g].lo;
-    rg[g].issued = 0;
+    const ptau::Shard sh = shard(n_points, g, G);
+    rg[g] = {sh.lo, sh.hi, sh.lo, 0};
     GpuSlot& s = ctx->gpu[g];
     CUDA_TRY(ctx, cudaSetDevice(s.device));
     size_t maxpts = rg[g].hi - rg[g].lo < chunk ? rg[g].hi - rg[g].lo : chunk;
-    int rc = ensure_buffers(ctx, s, maxpts * ri + 16, maxpts * ro + 16);
-    if (rc) return rc;
+    CUDA_TRY(ctx, ensure_buffers(s.d_in, &s.cap_in, maxpts * ri + 16));
+    CUDA_TRY(ctx, ensure_buffers(s.d_out, &s.cap_out, maxpts * ro + 16));
     CUDA_TRY(ctx, cudaMemcpyAsync(s.d_status, &none, sizeof(none), cudaMemcpyHostToDevice, s.stream[0]));
     CUDA_TRY(ctx, cudaEventRecord(s.ev_first, s.stream[0]));
     // stream[1] must not start before the status word is initialised
@@ -440,33 +463,27 @@ static int ensure_gen_table(ptau_ctx* ctx, GpuSlot& s, int group, cudaStream_t s
       }
       k[w >> 2] = (uint32_t)d << ((w & 3) * 8);
     }
-  uint32_t* d_sc = nullptr;
-  uint8_t* d_zu = nullptr;
-  unsigned long long* d_st = nullptr;
-  CUDA_TRY(ctx, cudaMalloc((void**)&d_sc, cnt * 32));
-  CUDA_TRY(ctx, cudaMalloc((void**)&d_zu, cnt * r_zu));
-  CUDA_TRY(ctx, cudaMalloc((void**)&d_st, 8));
-  CUDA_TRY(ctx, cudaMalloc((void**)&s.d_tbl[gi], cnt * r_ml));
+  DevArgs a;
+  void *d_sc = nullptr, *d_zu = nullptr, *d_st = nullptr;
   const unsigned long long none = PTAU_STATUS_NONE;
-  cudaError_t e = cudaMemcpyAsync(d_sc, sc.data(), cnt * 32, cudaMemcpyHostToDevice, stream);
-  if (e == cudaSuccess) e = cudaMemcpyAsync(d_st, &none, 8, cudaMemcpyHostToDevice, stream);
-  if (e == cudaSuccess) e = ptau::launch_generate(group, PTAU_FMT_ZCASH_UNCOMPRESSED, d_sc, d_zu, cnt, stream);
-  if (e == cudaSuccess)
-    e = ptau::launch_convert(group, PTAU_FMT_ZCASH_UNCOMPRESSED, PTAU_FMT_ARK_MONT_LIMBS, d_zu, s.d_tbl[gi], cnt, 0, 0, d_st,
-                             stream);
   unsigned long long st = 0;
+  cudaError_t e = a.push(sc.data(), cnt * 32, stream, &d_sc);
+  if (e == cudaSuccess) e = a.push(nullptr, cnt * r_zu, stream, &d_zu);
+  if (e == cudaSuccess) e = a.push(&none, 8, stream, &d_st);
+  if (e == cudaSuccess) e = cudaMalloc((void**)&s.d_tbl[gi], cnt * r_ml);
+  if (e == cudaSuccess)
+    e = ptau::launch_generate(group, PTAU_FMT_ZCASH_UNCOMPRESSED, (const uint32_t*)d_sc, d_zu, cnt, stream);
+  if (e == cudaSuccess)
+    e = ptau::launch_convert(group, PTAU_FMT_ZCASH_UNCOMPRESSED, PTAU_FMT_ARK_MONT_LIMBS, d_zu, s.d_tbl[gi], cnt, 0, 0,
+                             (unsigned long long*)d_st, stream);
   if (e == cudaSuccess) e = cudaMemcpyAsync(&st, d_st, 8, cudaMemcpyDeviceToHost, stream);
   if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
-  cudaFree(d_sc);
-  cudaFree(d_zu);
-  cudaFree(d_st);
-  if (e != cudaSuccess || st != PTAU_STATUS_NONE) {
-    cudaFree(s.d_tbl[gi]);
-    s.d_tbl[gi] = nullptr;
-    ctx->last_error = std::string("generator table: ") + (e != cudaSuccess ? cudaGetErrorString(e) : "bad table point");
-    return PTAU_ERR_CUDA;
-  }
-  return PTAU_OK;
+  if (e == cudaSuccess && st == PTAU_STATUS_NONE) return PTAU_OK;
+  cudaFree(s.d_tbl[gi]);
+  s.d_tbl[gi] = nullptr;
+  if (e != cudaSuccess) return cuda_fail(ctx, "ptau_generate_device", e);
+  ctx->last_error = "ptau_generate_device: bad generator table point";
+  return PTAU_ERR_CUDA;
 }
 
 int ptau_generate_device(ptau_ctx* ctx, int gpu, int group, int fmt, const uint8_t scalar0[32], const uint8_t step[32],
@@ -505,11 +522,11 @@ int ptau_generate(ptau_ctx* ctx, int group, int fmt, const uint8_t scalar0[32], 
   GpuSlot& s = ctx->gpu[0];
   CUDA_TRY(ctx, cudaSetDevice(s.device));
   const size_t chunk = ctx->chunk_points;
-  int rc = ensure_buffers(ctx, s, 16, (n_points < chunk ? n_points : chunk) * ro + 16);
-  if (rc) return rc;
+  CUDA_TRY(ctx, ensure_buffers(s.d_in, &s.cap_in, 16));
+  CUDA_TRY(ctx, ensure_buffers(s.d_out, &s.cap_out, (n_points < chunk ? n_points : chunk) * ro + 16));
   for (size_t off = 0; off < n_points; off += chunk) {
     size_t n = n_points - off < chunk ? n_points - off : chunk;
-    rc = ptau_generate_device(ctx, 0, group, fmt, scalar0, step, first + off, n, s.d_out[0], s.stream[0]);
+    int rc = ptau_generate_device(ctx, 0, group, fmt, scalar0, step, first + off, n, s.d_out[0], s.stream[0]);
     if (rc) return rc;
     CUDA_TRY(ctx, cudaMemcpyAsync((uint8_t*)out + off * ro, s.d_out[0], n * ro, cudaMemcpyDeviceToHost, s.stream[0]));
     CUDA_TRY(ctx, cudaStreamSynchronize(s.stream[0]));
@@ -519,20 +536,19 @@ int ptau_generate(ptau_ctx* ctx, int group, int fmt, const uint8_t scalar0[32], 
 
 // ---- whole-file pipelines ----------------------------------------------------------
 // out[s] == NULL with process[s] set: the section is validated but nothing is copied back
-static int run_sections(ptau_ctx* ctx, const Section* secs, int nsec, int in_fmt, const uint8_t* in,
-                        const int* out_fmt, uint8_t* const* out, unsigned checks, uint64_t* bad_index, int* bad_kind,
-                        int* bad_section, const bool* process = nullptr) {
+static int run_sections(ptau_ctx* ctx, const Section* secs, int nsec, int in_fmt, const uint8_t* in, int out_fmt,
+                        uint8_t* const* out, unsigned checks, uint64_t* bad_index, int* bad_kind, int* bad_section,
+                        const bool* process = nullptr) {
   // Sections are processed in file order and the first failing section wins, so
   // the reported (section, index) is the first bad point in file order.
-  ptau_timing total;
-  memset(&total, 0, sizeof(total));
+  ptau_timing total{};
   total.n_gpus = ctx->n_gpus;
   size_t off = 0;
   for (int s = 0; s < nsec; s++) {
     const int ri = rec_size(secs[s].group, in_fmt);
     if (out[s] || (process && process[s])) {
-      int rc = ptau_convert(ctx, secs[s].group, in_fmt, in + off, out_fmt[s], out[s], secs[s].count, checks,
-                            bad_index, bad_kind);
+      int rc = ptau_convert(ctx, secs[s].group, in_fmt, in + off, out_fmt, out[s], secs[s].count, checks, bad_index,
+                            bad_kind);
       total.wall_ms += ctx->timing.wall_ms;
       total.kernel_launches += ctx->timing.kernel_launches;
       for (int g = 0; g < ctx->n_gpus; g++) {
@@ -553,46 +569,29 @@ static int run_sections(ptau_ctx* ctx, const Section* secs, int nsec, int in_fmt
   return PTAU_OK;
 }
 
-static int assemble_setup(int variant, uint64_t n, uint8_t* setup, const uint8_t* tau_g2_ark) {
-  // kgz tail: VerifierKey { g = tau_g1[0], gamma_g = alpha_g1[0], h = tau_g2[0], beta_h = tau_g2[1] }
-  //   (preprocess-kgz.rs:177-194)
-  // fastkgz: h, beta_h are the first two entries of powers_of_h, which follow
-  //   (preprocess-fastkgz.rs:163-208) -- already in place, copy h/beta_h in front.
-  const uint64_t g1_all = (2 * n - 1) * 96 + n * 96;
-  if (variant == PTAU_VARIANT_KGZ) {
-    uint8_t* tail = setup + g1_all;
-    memcpy(tail, setup, 96);                           // g
-    memcpy(tail + 96, setup + (2 * n - 1) * 96, 96);   // gamma_g
-    memcpy(tail + 192, tau_g2_ark, 192);               // h
-    memcpy(tail + 384, tau_g2_ark + 192, 192);         // beta_h
-  } else {
-    memcpy(setup + g1_all, tau_g2_ark, 384);           // h, beta_h
-  }
-  return PTAU_OK;
-}
-
 static int preprocess_common(ptau_ctx* ctx, int variant, int in_fmt, const uint8_t* body, uint64_t n, uint8_t* setup,
                              unsigned checks, uint64_t* bad_index, int* bad_kind, int* bad_section) {
   if (n < 2) return PTAU_ERR_ARG;
   const bool fast = variant == PTAU_VARIANT_FASTKGZ;
-  const Section secs[5] = {{PTAU_G1, 2 * n - 1}, {PTAU_G2, n}, {PTAU_G1, n}, {PTAU_G1, n}, {PTAU_G2, 1}};
+  const auto secs = ptau::response_sections(n);
+  const ptau::SetupLayout L = ptau::setup_layout(variant, n);
   // tau_g2: kgz needs only [0], [1] in the output but the reference checks all n
   // (preprocess-kgz.rs:146-148): all n are validated on the GPU without copying the
   // results back, and the first two are converted again for the VerifierKey; fastkgz
   // writes all n in place as powers_of_h.  beta_tau_powers_g1 is read, checked and
   // dropped by fastkgz (preprocess-fastkgz.rs:156-159) and never read by kgz; beta_g2
   // (section 4) is never read by either binary (preprocess-fastkgz.rs:161).
-  const uint64_t g1_all = (2 * n - 1) * 96 + n * 96;
   uint8_t first_g2[384];
-  int fmts[5] = {PTAU_FMT_ARK_UNCOMPRESSED, PTAU_FMT_ARK_UNCOMPRESSED, PTAU_FMT_ARK_UNCOMPRESSED,
-                 PTAU_FMT_ARK_UNCOMPRESSED, PTAU_FMT_ARK_UNCOMPRESSED};
-  uint8_t* outs[5] = {setup, fast ? setup + g1_all + 384 : nullptr, setup + (2 * n - 1) * 96, nullptr, nullptr};
+  uint8_t* outs[5] = {setup + L.g1(0), fast ? setup + L.g2(L.powers_of_h) : nullptr, setup + L.g1(L.gamma_g), nullptr,
+                      nullptr};
   const bool process[5] = {true, true, true, fast, false};
-  int rc = run_sections(ctx, secs, 5, in_fmt, body, fmts, outs, checks, bad_index, bad_kind, bad_section, process);
+  int rc = run_sections(ctx, secs.data(), 5, in_fmt, body, PTAU_FMT_ARK_UNCOMPRESSED, outs, checks, bad_index, bad_kind,
+                        bad_section, process);
   if (rc) return rc;
-  const uint8_t* tau_g2_ark = setup + g1_all + 384;
+  // fastkgz: h, beta_h are the first two entries of powers_of_h, which follow them (preprocess-fastkgz.rs:163-208)
+  const uint8_t* tau_g2_ark = setup + L.g2(L.powers_of_h);
   if (!fast) {
-    const size_t g2_off = (2 * n - 1) * (size_t)rec_size(PTAU_G1, in_fmt);
+    const size_t g2_off = secs[0].count * (size_t)rec_size(secs[0].group, in_fmt);
     ptau_timing keep = ctx->timing;
     rc = ptau_convert(ctx, PTAU_G2, in_fmt, body + g2_off, PTAU_FMT_ARK_UNCOMPRESSED, first_g2, 2, checks, bad_index,
                       bad_kind);
@@ -603,8 +602,13 @@ static int preprocess_common(ptau_ctx* ctx, int variant, int in_fmt, const uint8
       return rc;
     }
     tau_g2_ark = first_g2;
+    // kgz tail: VerifierKey { g = tau_g1[0], gamma_g = alpha_g1[0], h = tau_g2[0], beta_h = tau_g2[1] }
+    //   (preprocess-kgz.rs:177-194)
+    memcpy(setup + L.g1(L.vk_g), setup + L.g1(0), 96);              // g
+    memcpy(setup + L.g1(L.vk_g + 1), setup + L.g1(L.gamma_g), 96);  // gamma_g
   }
-  return assemble_setup(variant, n, setup, tau_g2_ark);
+  memcpy(setup + L.g2(0), tau_g2_ark, 384);  // h, beta_h
+  return PTAU_OK;
 }
 
 int ptau_preprocess(ptau_ctx* ctx, int variant, const void* response, uint64_t response_len, uint64_t n_powers,
@@ -617,22 +621,19 @@ int ptau_preprocess(ptau_ctx* ctx, int variant, const void* response, uint64_t r
   if (setup_len != ptau_setup_size(variant, n_powers)) return PTAU_ERR_SIZE;
   if (uncompressed_out && uncompressed_len != ptau_uncompressed_size(n_powers)) return PTAU_ERR_SIZE;
   // skip the 64-byte challenge hash (:96-101); the trailing public key is never read
-  const uint8_t* body = (const uint8_t*)response + 64;
+  const uint8_t* body = (const uint8_t*)response + ptau::kResponseHash;
   if (uncompressed_out) {
     // two stages, exactly as the reference: decompress everything into
     // `powersoftau_uncompressed` (:105-124), then read that back (:128-160)
-    const uint64_t n = n_powers;
-    const Section secs[5] = {{PTAU_G1, 2 * n - 1}, {PTAU_G2, n}, {PTAU_G1, n}, {PTAU_G1, n}, {PTAU_G2, 1}};
-    int fmts[5];
+    const auto secs = ptau::response_sections(n_powers);
     uint8_t* outs[5];
     size_t o = 0;
     for (int s = 0; s < 5; s++) {
-      fmts[s] = PTAU_FMT_ZCASH_UNCOMPRESSED;
       outs[s] = (uint8_t*)uncompressed_out + o;
       o += secs[s].count * (size_t)rec_size(secs[s].group, PTAU_FMT_ZCASH_UNCOMPRESSED);
     }
-    int rc = run_sections(ctx, secs, 5, PTAU_FMT_ZCASH_COMPRESSED, body, fmts, outs, PTAU_CHECKS_DECOMPRESS, bad_index,
-                          bad_kind, bad_section);
+    int rc = run_sections(ctx, secs.data(), 5, PTAU_FMT_ZCASH_COMPRESSED, body, PTAU_FMT_ZCASH_UNCOMPRESSED, outs,
+                          PTAU_CHECKS_DECOMPRESS, bad_index, bad_kind, bad_section);
     if (rc) return rc;
     return preprocess_common(ctx, variant, PTAU_FMT_ZCASH_UNCOMPRESSED, (const uint8_t*)uncompressed_out, n_powers,
                              (uint8_t*)setup_out, checks, bad_index, bad_kind, bad_section);
@@ -659,18 +660,15 @@ int ptau_load_setup(ptau_ctx* ctx, int variant, const void* setup, uint64_t setu
   if (!ctx || !setup || !g1_out || !g2_out) return PTAU_ERR_ARG;
   if (variant != PTAU_VARIANT_KGZ && variant != PTAU_VARIANT_FASTKGZ) return PTAU_ERR_ARG;
   if (setup_len != ptau_setup_size(variant, n)) return PTAU_ERR_SIZE;
-  const bool fast = variant == PTAU_VARIANT_FASTKGZ;
-  const uint64_t n_g1 = (3 * n - 1) + (fast ? 0 : 2);
-  const uint64_t n_g2 = fast ? n + 2 : 2;
-  if (g1_out_len != n_g1 * 104 || g2_out_len != n_g2 * 200) return PTAU_ERR_SIZE;
+  const ptau::SetupLayout L = ptau::setup_layout(variant, n);
+  if (g1_out_len != L.n_g1 * kMontG1 || g2_out_len != L.n_g2 * kMontG2) return PTAU_ERR_SIZE;
   // both layouts are "all G1 records, then all G2 records" (src/lib.rs:179-192, :202-215)
-  const Section secs[2] = {{PTAU_G1, n_g1}, {PTAU_G2, n_g2}};
-  int fmts[2] = {PTAU_FMT_ARK_MONT_LIMBS, PTAU_FMT_ARK_MONT_LIMBS};
+  const Section secs[2] = {{PTAU_G1, L.n_g1}, {PTAU_G2, L.n_g2}};
   uint8_t* outs[2] = {(uint8_t*)g1_out, (uint8_t*)g2_out};
   int sec = 0;
-  int rc = run_sections(ctx, secs, 2, PTAU_FMT_ARK_UNCOMPRESSED, (const uint8_t*)setup, fmts, outs, checks, bad_index,
-                        bad_kind, &sec);
-  if (rc > 0 && sec == 1 && bad_index) *bad_index += n_g1;  // index in file order over all points
+  int rc = run_sections(ctx, secs, 2, PTAU_FMT_ARK_UNCOMPRESSED, (const uint8_t*)setup, PTAU_FMT_ARK_MONT_LIMBS, outs,
+                        checks, bad_index, bad_kind, &sec);
+  if (rc > 0 && sec == 1 && bad_index) *bad_index += L.n_g1;  // index in file order over all points
   return rc;
 }
 
@@ -679,16 +677,13 @@ int ptau_load_phase1(ptau_ctx* ctx, const void* data, uint64_t len, uint64_t m, 
   if (!ctx || !data || !g1_out || !g2_out) return PTAU_ERR_ARG;
   // src/lib.rs:92-110: alpha, beta_g1 (G1), beta_g2 (G2), m G1, m G2, m G1, m G1
   if (len != 2 * 96 + 192 + m * 96 + m * 192 + m * 96 + m * 96) return PTAU_ERR_SIZE;
-  if (g1_out_len != (2 + 3 * m) * 104 || g2_out_len != (1 + m) * 200) return PTAU_ERR_SIZE;
+  if (g1_out_len != (2 + 3 * m) * kMontG1 || g2_out_len != (1 + m) * kMontG2) return PTAU_ERR_SIZE;
   const Section secs[5] = {{PTAU_G1, 2}, {PTAU_G2, 1}, {PTAU_G1, m}, {PTAU_G2, m}, {PTAU_G1, 2 * m}};
-  int fmts[5] = {PTAU_FMT_ARK_MONT_LIMBS, PTAU_FMT_ARK_MONT_LIMBS, PTAU_FMT_ARK_MONT_LIMBS, PTAU_FMT_ARK_MONT_LIMBS,
-                 PTAU_FMT_ARK_MONT_LIMBS};
   uint8_t* g1 = (uint8_t*)g1_out;
   uint8_t* g2 = (uint8_t*)g2_out;
-  uint8_t* outs[5] = {g1, g2, g1 + 2 * 104, g2 + 200, g1 + (2 + m) * 104};
-  int sec = 0;
-  return run_sections(ctx, secs, 5, PTAU_FMT_ZCASH_UNCOMPRESSED, (const uint8_t*)data, fmts, outs, checks, bad_index,
-                      bad_kind, &sec);
+  uint8_t* outs[5] = {g1, g2, g1 + 2 * kMontG1, g2 + kMontG2, g1 + (2 + m) * kMontG1};
+  return run_sections(ctx, secs, 5, PTAU_FMT_ZCASH_UNCOMPRESSED, (const uint8_t*)data, PTAU_FMT_ARK_MONT_LIMBS, outs,
+                      checks, bad_index, bad_kind, nullptr);
 }
 
 namespace {
@@ -729,12 +724,9 @@ void copy_parts(void* dst, const void* src, size_t len) {
 cudaError_t msm_issue(GpuSlot& s, const void* pts, const void* sc, size_t n, int* launches, bool resident = false,
                       bool g2 = false) {
   cudaError_t e = cudaSetDevice(s.device);
-  const size_t rb = g2 ? 200 : 104;
+  const size_t rb = g2 ? kMontG2 : kMontG1;
   ptau::MsmPlan plan;
-  if (g2)
-    ptau::msm_g2_plan(n, &plan);
-  else
-    ptau::msm_g1_plan(n, &plan);
+  (g2 ? ptau::msm_g2_plan : ptau::msm_g1_plan)(n, &plan);
   const void* d_pts = pts;
   if (e == cudaSuccess && !resident) {
     e = grow(&s.d_msm_pts, &s.cap_msm_pts, n * rb + 16);
@@ -762,6 +754,12 @@ cudaError_t msm_wait(GpuSlot& s, float* ms) {
   if (e == cudaSuccess) e = cudaStreamSynchronize(s.stream[0]);
   if (e == cudaSuccess) e = cudaEventElapsedTime(ms, s.ev_k0[0], s.ev_k1[0]);
   return e;
+}
+// point indices travel in 31 bits and the bucket lists (n x W entries) are addressed with 32-bit offsets
+bool msm_fits(size_t n, bool g2 = false) {
+  ptau::MsmPlan plan;
+  (g2 ? ptau::msm_g2_plan : ptau::msm_g1_plan)(n, &plan);
+  return n < (1ull << 31) && (uint64_t)n * (uint64_t)plan.W < (1ull << 32);
 }
 }  // namespace
 
@@ -795,12 +793,11 @@ int ptau_kzg_powers_upload(ptau_ctx* ctx, const void* powers, size_t n, ptau_kzg
   p->n = n;
   for (int g = 0; g < ctx->n_gpus; g++) {
     cudaError_t e = cudaSetDevice(ctx->gpu[g].device);
-    if (e == cudaSuccess) e = cudaMalloc(&p->d_pts[g], n * 104 + 16);
-    if (e == cudaSuccess && n) e = cudaMemcpy(p->d_pts[g], powers, n * 104, cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) e = cudaMalloc(&p->d_pts[g], n * kMontG1 + 16);
+    if (e == cudaSuccess && n) e = cudaMemcpy(p->d_pts[g], powers, n * kMontG1, cudaMemcpyHostToDevice);
     if (e != cudaSuccess) {
-      ctx->last_error = std::string("kzg_powers_upload: ") + cudaGetErrorString(e);
       ptau_kzg_powers_free(p);
-      return PTAU_ERR_CUDA;
+      return cuda_fail(ctx, __func__, e);
     }
   }
   *out = p;
@@ -822,24 +819,17 @@ int ptau_kzg_commit_resident(ptau_ctx* ctx, const ptau_kzg_powers* powers, const
 static int kzg_commit_impl(ptau_ctx* ctx, const void* powers, const ptau_kzg_powers* res, const void* coeffs, size_t n,
                            void* commitment, bool g2) {
   // scalars must be canonical (< r), like ark's Fr: checked on the device by the kernel that reads them anyway
-  const size_t rb = g2 ? 200 : 104;
-  const int rw = g2 ? 50 : 26;
-  ptau::MsmPlan plan;
-  if (g2)
-    ptau::msm_g2_plan(n, &plan);
-  else
-    ptau::msm_g1_plan(n, &plan);
-  // point indices travel in 31 bits and the bucket lists (n x W entries) are addressed with 32-bit offsets
-  if (n >= (1ull << 31) || (uint64_t)n * (uint64_t)plan.W >= (1ull << 32)) return PTAU_ERR_ARG;
+  const size_t rb = g2 ? kMontG2 : kMontG1;
+  if (!msm_fits(n, g2)) return PTAU_ERR_ARG;
   const int G = (ctx->n_gpus > 1 && n >= (size_t)ctx->n_gpus * (1u << 12)) ? ctx->n_gpus : 1;
-  memset(&ctx->timing, 0, sizeof(ctx->timing));
-  ctx->timing.n_gpus = ctx->n_gpus;
+  timing_reset(ctx);
   cudaError_t e = cudaSuccess;
   int launches[kMaxGpus] = {0};
   for (int g = 0; g < G && e == cudaSuccess; g++) {
-    const size_t lo = n * g / G, hi = n * (g + 1) / G;
+    const auto [lo, hi] = shard(n, g, G);
     if (res)
-      e = msm_issue(ctx->gpu[g], (const uint8_t*)res->d_pts[g] + lo * 104, (const uint8_t*)coeffs + lo * 32, hi - lo, &launches[g], true);
+      e = msm_issue(ctx->gpu[g], (const uint8_t*)res->d_pts[g] + lo * kMontG1, (const uint8_t*)coeffs + lo * 32,
+                    hi - lo, &launches[g], true);
     else
       e = msm_issue(ctx->gpu[g], (const uint8_t*)powers + lo * rb, (const uint8_t*)coeffs + lo * 32, hi - lo, &launches[g],
                     false, g2);
@@ -847,7 +837,7 @@ static int kzg_commit_impl(ptau_ctx* ctx, const void* powers, const ptau_kzg_pow
     ctx->timing.d2h_bytes[g] = rb;
   }
   bool bad_scalar = false;
-  uint8_t parts[kMaxGpus * 200];
+  uint8_t parts[kMaxGpus * kMontG2];
   for (int g = 0; g < G && e == cudaSuccess; g++) {
     float ms = 0;
     e = msm_wait(ctx->gpu[g], &ms);
@@ -856,7 +846,7 @@ static int kzg_commit_impl(ptau_ctx* ctx, const void* powers, const ptau_kzg_pow
     ctx->timing.kernel_launches += launches[g];
     if (e == cudaSuccess) {
       memcpy(parts + g * rb, ctx->gpu[g].h_msm_out, rb);
-      bad_scalar = bad_scalar || ctx->gpu[g].h_msm_out[rw] != 0;
+      bad_scalar = bad_scalar || ctx->gpu[g].h_msm_out[rb / 4] != 0;
     }
   }
   if (e == cudaSuccess && bad_scalar) return PTAU_ERR_ARG;
@@ -875,30 +865,10 @@ static int kzg_commit_impl(ptau_ctx* ctx, const void* powers, const ptau_kzg_pow
   } else if (e == cudaSuccess) {
     memcpy(commitment, parts, rb);
   }
-  if (e != cudaSuccess) {
-    ctx->last_error = std::string("kzg_commit: ") + cudaGetErrorString(e);
-    return PTAU_ERR_CUDA;
-  }
-  return PTAU_OK;
+  return e == cudaSuccess ? PTAU_OK : cuda_fail(ctx, g2 ? "ptau_msm_g2" : "ptau_kzg_commit", e);
 }
 
 namespace {
-// device copies of a list of host arrays, freed together
-struct DevArgs {
-  std::vector<void*> ptrs;
-  ~DevArgs() {
-    for (void* p : ptrs) cudaFree(p);
-  }
-  cudaError_t push(const void* host, size_t bytes, cudaStream_t st, void** out) {
-    void* d = nullptr;
-    cudaError_t e = cudaMalloc(&d, bytes ? bytes : 16);
-    if (e != cudaSuccess) return e;
-    ptrs.push_back(d);
-    if (host && bytes) e = cudaMemcpyAsync(d, host, bytes, cudaMemcpyHostToDevice, st);
-    *out = d;
-    return e;
-  }
-};
 bool scalars_canonical(const void* p, size_t n) {
   for (size_t i = 0; i < n; i++) {
     Fr c = fr_from_le32((const uint8_t*)p + i * 32);
@@ -906,72 +876,38 @@ bool scalars_canonical(const void* p, size_t n) {
   }
   return true;
 }
+// error path of a call with work queued on the first stream of GPUs 0..G-1: nothing may still be using its buffers
+// when the call returns
+int drain_fail(ptau_ctx* ctx, int G, const char* where, cudaError_t e) {
+  for (int g = 0; g < G; g++) {
+    cudaSetDevice(ctx->gpu[g].device);
+    cudaStreamSynchronize(ctx->gpu[g].stream[0]);
+  }
+  return cuda_fail(ctx, where, e);
+}
 }  // namespace
 
 int ptau_pairing_product2(ptau_ctx* ctx, const void* g1, const void* g2, size_t n, void* gt_out, uint8_t* is_one) {
   if (!ctx || (n && (!g1 || !g2)) || (!gt_out && !is_one)) return PTAU_ERR_ARG;
   if (n == 0) return PTAU_OK;
-  GpuSlot& s = ctx->gpu[0];
-  CUDA_TRY(ctx, cudaSetDevice(s.device));
-  DevArgs a;
   void *d1 = nullptr, *d2 = nullptr, *dgt = nullptr, *dis = nullptr;
-  cudaError_t e = a.push(g1, n * 2 * 104, s.stream[0], &d1);
-  if (e == cudaSuccess) e = a.push(g2, n * 2 * 200, s.stream[0], &d2);
-  if (e == cudaSuccess && gt_out) e = a.push(nullptr, n * 576, s.stream[0], &dgt);
-  if (e == cudaSuccess && is_one) e = a.push(nullptr, n, s.stream[0], &dis);
-  if (e == cudaSuccess) e = cudaEventRecord(s.ev_k0[0], s.stream[0]);
-  if (e == cudaSuccess) e = ptau::launch_pairing_product2(d1, d2, n, dgt, dis, s.stream[0]);
-  if (e == cudaSuccess) e = cudaEventRecord(s.ev_k1[0], s.stream[0]);
-  if (e == cudaSuccess && gt_out) e = cudaMemcpyAsync(gt_out, dgt, n * 576, cudaMemcpyDeviceToHost, s.stream[0]);
-  if (e == cudaSuccess && is_one) e = cudaMemcpyAsync(is_one, dis, n, cudaMemcpyDeviceToHost, s.stream[0]);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(s.stream[0]);
-  float ms = 0;
-  if (e == cudaSuccess) e = cudaEventElapsedTime(&ms, s.ev_k0[0], s.ev_k1[0]);
-  if (e != cudaSuccess) {
-    ctx->last_error = std::string("pairing_product2: ") + cudaGetErrorString(e);
-    return PTAU_ERR_CUDA;
-  }
-  memset(&ctx->timing, 0, sizeof(ctx->timing));
-  ctx->timing.n_gpus = ctx->n_gpus;
-  ctx->timing.kernel_ms[0] = ms;
-  ctx->timing.gpu_ms[0] = ms;
-  ctx->timing.kernel_launches = 1;
-  ctx->timing.h2d_bytes[0] = n * 608;
-  ctx->timing.d2h_bytes[0] = n * ((gt_out ? 576 : 0) + (is_one ? 1 : 0));
-  return PTAU_OK;
+  return launch_once(ctx, 0, __func__, true,
+                     {{g1, nullptr, n * 2 * kMontG1, &d1},
+                      {g2, nullptr, n * 2 * kMontG2, &d2},
+                      {nullptr, gt_out, n * 576, &dgt},
+                      {nullptr, is_one, n, &dis}},
+                     [&](cudaStream_t st) { return ptau::launch_pairing_product2(d1, d2, n, dgt, dis, st); });
 }
 
 int ptau_g2_prepare(ptau_ctx* ctx, const void* g2, size_t n, void* coeffs_out, uint8_t* infinity_out) {
   if (!ctx || (n && (!g2 || !coeffs_out || !infinity_out))) return PTAU_ERR_ARG;
   if (n == 0) return PTAU_OK;
-  GpuSlot& s = ctx->gpu[0];
-  CUDA_TRY(ctx, cudaSetDevice(s.device));
-  DevArgs a;
   void *d2 = nullptr, *dc = nullptr, *di = nullptr;
-  const size_t cb = (size_t)PTAU_G2_PREPARED_COEFFS * 288;
-  cudaError_t e = a.push(g2, n * 200, s.stream[0], &d2);
-  if (e == cudaSuccess) e = a.push(nullptr, n * cb, s.stream[0], &dc);
-  if (e == cudaSuccess) e = a.push(nullptr, n, s.stream[0], &di);
-  if (e == cudaSuccess) e = cudaEventRecord(s.ev_k0[0], s.stream[0]);
-  if (e == cudaSuccess) e = ptau::launch_g2_prepare(d2, n, dc, di, s.stream[0]);
-  if (e == cudaSuccess) e = cudaEventRecord(s.ev_k1[0], s.stream[0]);
-  if (e == cudaSuccess) e = cudaMemcpyAsync(coeffs_out, dc, n * cb, cudaMemcpyDeviceToHost, s.stream[0]);
-  if (e == cudaSuccess) e = cudaMemcpyAsync(infinity_out, di, n, cudaMemcpyDeviceToHost, s.stream[0]);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(s.stream[0]);
-  float ms = 0;
-  if (e == cudaSuccess) e = cudaEventElapsedTime(&ms, s.ev_k0[0], s.ev_k1[0]);
-  if (e != cudaSuccess) {
-    ctx->last_error = std::string("g2_prepare: ") + cudaGetErrorString(e);
-    return PTAU_ERR_CUDA;
-  }
-  memset(&ctx->timing, 0, sizeof(ctx->timing));
-  ctx->timing.n_gpus = ctx->n_gpus;
-  ctx->timing.kernel_ms[0] = ms;
-  ctx->timing.gpu_ms[0] = ms;
-  ctx->timing.kernel_launches = 1;
-  ctx->timing.h2d_bytes[0] = n * 200;
-  ctx->timing.d2h_bytes[0] = n * (cb + 1);
-  return PTAU_OK;
+  return launch_once(ctx, 0, __func__, true,
+                     {{g2, nullptr, n * kMontG2, &d2},
+                      {nullptr, coeffs_out, n * PTAU_G2_PREPARED_COEFFS * 288, &dc},
+                      {nullptr, infinity_out, n, &di}},
+                     [&](cudaStream_t st) { return ptau::launch_g2_prepare(d2, n, dc, di, st); });
 }
 
 int ptau_kzg_check(ptau_ctx* ctx, const void* vk_g1, const void* vk_g2, const void* comms, const void* points,
@@ -983,26 +919,26 @@ int ptau_kzg_check(ptau_ctx* ctx, const void* vk_g1, const void* vk_g2, const vo
     return PTAU_ERR_ARG;
   // openings are independent: contiguous index ranges over the context's GPUs, no exchange
   const int G = (ctx->n_gpus > 1 && n >= (size_t)ctx->n_gpus * 64) ? ctx->n_gpus : 1;
-  std::string key((const char*)vk_g1, 2 * 104);
-  key.append((const char*)vk_g2, 200);
-  memset(&ctx->timing, 0, sizeof(ctx->timing));
-  ctx->timing.n_gpus = ctx->n_gpus;
+  std::string key((const char*)vk_g1, 2 * kMontG1);
+  key.append((const char*)vk_g2, kMontG2);
+  timing_reset(ctx);
   DevArgs args[kMaxGpus];
   bool rebuilt[kMaxGpus] = {false};
   cudaError_t e = cudaSuccess;
   for (int g = 0; g < G && e == cudaSuccess; g++) {
     GpuSlot& s = ctx->gpu[g];
-    const size_t lo = n * g / G, cnt = n * (g + 1) / G - lo;
+    const ptau::Shard sh = shard(n, g, G);
+    const size_t lo = sh.lo, cnt = sh.hi - sh.lo;
     cudaStream_t st = s.stream[0];
     DevArgs& a = args[g];
     void *dv1 = nullptr, *dv2 = nullptr, *dc = nullptr, *dz = nullptr, *dv = nullptr, *dw = nullptr, *drv = nullptr, *dok = nullptr;
     e = cudaSetDevice(s.device);
-    if (e == cudaSuccess) e = a.push(vk_g1, 2 * 104, st, &dv1);
-    if (e == cudaSuccess) e = a.push(vk_g2, 2 * 200, st, &dv2);
-    if (e == cudaSuccess) e = a.push((const uint8_t*)comms + lo * 104, cnt * 104, st, &dc);
+    if (e == cudaSuccess) e = a.push(vk_g1, 2 * kMontG1, st, &dv1);
+    if (e == cudaSuccess) e = a.push(vk_g2, 2 * kMontG2, st, &dv2);
+    if (e == cudaSuccess) e = a.push((const uint8_t*)comms + lo * kMontG1, cnt * kMontG1, st, &dc);
     if (e == cudaSuccess) e = a.push((const uint8_t*)points + lo * 32, cnt * 32, st, &dz);
     if (e == cudaSuccess) e = a.push((const uint8_t*)values + lo * 32, cnt * 32, st, &dv);
-    if (e == cudaSuccess) e = a.push((const uint8_t*)proofs_w + lo * 104, cnt * 104, st, &dw);
+    if (e == cudaSuccess) e = a.push((const uint8_t*)proofs_w + lo * kMontG1, cnt * kMontG1, st, &dw);
     if (e == cudaSuccess && random_v) e = a.push((const uint8_t*)random_v + lo * 32, cnt * 32, st, &drv);
     if (e == cudaSuccess) e = a.push(nullptr, cnt, st, &dok);
     int launches = 1;
@@ -1021,7 +957,7 @@ int ptau_kzg_check(ptau_ctx* ctx, const void* vk_g1, const void* vk_g2, const vo
     if (e == cudaSuccess) e = cudaEventRecord(s.ev_k1[0], st);
     if (e == cudaSuccess) e = cudaMemcpyAsync(ok + lo, dok, cnt, cudaMemcpyDeviceToHost, st);
     ctx->timing.kernel_launches += launches;
-    ctx->timing.h2d_bytes[g] = 608 + cnt * (104 + 32 + 32 + 104 + (random_v ? 32 : 0));
+    ctx->timing.h2d_bytes[g] = 2 * (kMontG1 + kMontG2) + cnt * (kMontG1 + 32 + 32 + kMontG1 + (random_v ? 32 : 0));
     ctx->timing.d2h_bytes[g] = cnt;
   }
   for (int g = 0; g < G && e == cudaSuccess; g++) {
@@ -1034,15 +970,7 @@ int ptau_kzg_check(ptau_ctx* ctx, const void* vk_g1, const void* vk_g2, const vo
     ctx->timing.kernel_ms[g] = ms;
     ctx->timing.gpu_ms[g] = ms;
   }
-  if (e != cudaSuccess) {
-    for (int g = 0; g < G; g++) {  // nothing may still be reading the buffers DevArgs is about to free
-      cudaSetDevice(ctx->gpu[g].device);
-      cudaStreamSynchronize(ctx->gpu[g].stream[0]);
-    }
-    ctx->last_error = std::string("kzg_check: ") + cudaGetErrorString(e);
-    return PTAU_ERR_CUDA;
-  }
-  return PTAU_OK;
+  return e == cudaSuccess ? PTAU_OK : drain_fail(ctx, G, __func__, e);  // before DevArgs frees the buffers
 }
 
 // Witness polynomial of KZG10::open: (p(X) - p(z)) / (X - z) by synthetic division, and p(z).  A first-order
@@ -1081,12 +1009,6 @@ void kzg_zpow(const void* z, uint32_t (*out)[8]) {
     p = fr_mont_mul(p, p);
   }
 }
-// point indices travel in 31 bits and the bucket lists (n x W entries) are addressed with 32-bit offsets
-bool msm_fits(size_t n) {
-  ptau::MsmPlan plan;
-  ptau::msm_g1_plan(n, &plan);
-  return n < (1ull << 31) && (uint64_t)n * (uint64_t)plan.W < (1ull << 32);
-}
 size_t up256(size_t v) { return (v + 255) & ~(size_t)255; }
 }  // namespace
 
@@ -1104,8 +1026,7 @@ int ptau_kzg_open(ptau_ctx* ctx, const ptau_kzg_powers* powers, const ptau_kzg_p
   if (k && (!points || !proofs_out || !values_out || (n_b > 0) != (random_v_out != nullptr))) return PTAU_ERR_ARG;
   if (!msm_fits(n) || !msm_fits(n_b)) return PTAU_ERR_ARG;
   auto t0 = std::chrono::steady_clock::now();
-  memset(&ctx->timing, 0, sizeof(ctx->timing));
-  ctx->timing.n_gpus = ctx->n_gpus;
+  timing_reset(ctx);
   if (k == 0) return PTAU_OK;
   if (!scalars_canonical(points, k)) return PTAU_ERR_ARG;
   const int G = (size_t)ctx->n_gpus < k ? ctx->n_gpus : (int)k;
@@ -1121,10 +1042,7 @@ int ptau_kzg_open(ptau_ctx* ctx, const ptau_kzg_powers* powers, const ptau_kzg_p
   const size_t h_b = n * 32, h_one = h_b + n_b * 32, h_len = h_one + 64;
   cudaError_t e = cudaSetDevice(s0.device);
   if (e == cudaSuccess) e = grow(&s0.h_msm_sc, &s0.cap_h_msm_sc, h_len, true);
-  if (e != cudaSuccess) {
-    ctx->last_error = std::string("kzg_open: ") + cudaGetErrorString(e);
-    return PTAU_ERR_CUDA;
-  }
+  if (e != cudaSuccess) return cuda_fail(ctx, __func__, e);
   uint8_t* stage = (uint8_t*)s0.h_msm_sc;
   if (n) copy_parts(stage, coeffs, n * 32);
   if (n_b) copy_parts(stage + h_b, blinding, n_b * 32);
@@ -1138,8 +1056,9 @@ int ptau_kzg_open(ptau_ctx* ctx, const ptau_kzg_powers* powers, const ptau_kzg_p
   int launches = 0;
   for (int g = 0; g < G && e == cudaSuccess; g++) {
     GpuSlot& s = ctx->gpu[g];
-    const size_t lo = k * g / G, cnt = k * (g + 1) / G - lo;
-    const size_t d_rv = d_val + up256(cnt * 32), d_pf = d_rv + up256(cnt * 32), d_len = d_pf + cnt * 104;
+    const ptau::Shard sh = shard(k, g, G);
+    const size_t lo = sh.lo, cnt = sh.hi - sh.lo;
+    const size_t d_rv = d_val + up256(cnt * 32), d_pf = d_rv + up256(cnt * 32), d_len = d_pf + cnt * kMontG1;
     cudaStream_t st = s.stream[0];
     e = cudaSetDevice(s.device);
     if (e == cudaSuccess) e = grow(&s.d_open, &s.cap_open, d_len);
@@ -1170,30 +1089,33 @@ int ptau_kzg_open(ptau_ctx* ctx, const ptau_kzg_powers* powers, const ptau_kzg_p
         if (e == cudaSuccess)
           e = ptau::launch_msm_g1(gamma_powers->d_pts[g], s.d_msm_sc, nbq, s.d_msm_scratch, d + d_r1, &nl, st);
         launches += nl;
-        if (e == cudaSuccess) e = cudaMemcpyAsync(d + d_pair, d + d_r0, 104, cudaMemcpyDeviceToDevice, st);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(d + d_pair + 104, d + d_r1, 104, cudaMemcpyDeviceToDevice, st);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(d + d_pair, d + d_r0, kMontG1, cudaMemcpyDeviceToDevice, st);
+        if (e == cudaSuccess)
+          e = cudaMemcpyAsync(d + d_pair + kMontG1, d + d_r1, kMontG1, cudaMemcpyDeviceToDevice, st);
         if (e == cudaSuccess) e = ptau::launch_msm_g1(d + d_pair, d + d_one, 2, s.d_msm_scratch, d + d_r0, &nl, st);
         launches += nl;
       }
-      if (e == cudaSuccess) e = cudaMemcpyAsync(d + d_pf + j * 104, d + d_r0, 104, cudaMemcpyDeviceToDevice, st);
+      if (e == cudaSuccess)
+        e = cudaMemcpyAsync(d + d_pf + j * kMontG1, d + d_r0, kMontG1, cudaMemcpyDeviceToDevice, st);
     }
     if (e == cudaSuccess) e = cudaEventRecord(s.ev_k1[0], st);
     if (e == cudaSuccess) e = cudaMemcpyAsync(s.h_msm_out, bad, 4, cudaMemcpyDeviceToHost, st);
     ctx->timing.h2d_bytes[g] = (n + n_b) * 32 + 64;
-    ctx->timing.d2h_bytes[g] = cnt * (104 + 32 + (n_b ? 32 : 0)) + 4;
+    ctx->timing.d2h_bytes[g] = cnt * (kMontG1 + 32 + (n_b ? 32 : 0)) + 4;
   }
   ctx->timing.kernel_launches = launches;
   // results to the caller's (pageable) memory only once every GPU has its work queued
   bool bad_coeff = false;
   for (int g = 0; g < G && e == cudaSuccess; g++) {
     GpuSlot& s = ctx->gpu[g];
-    const size_t lo = k * g / G, cnt = k * (g + 1) / G - lo;
+    const ptau::Shard sh = shard(k, g, G);
+    const size_t lo = sh.lo, cnt = sh.hi - sh.lo;
     const size_t d_rv = d_val + up256(cnt * 32), d_pf = d_rv + up256(cnt * 32);
     const uint8_t* d = (const uint8_t*)s.d_open;
     cudaStream_t st = s.stream[0];
     e = cudaSetDevice(s.device);
     if (e == cudaSuccess)
-      e = cudaMemcpyAsync((uint8_t*)proofs_out + lo * 104, d + d_pf, cnt * 104, cudaMemcpyDeviceToHost, st);
+      e = cudaMemcpyAsync((uint8_t*)proofs_out + lo * kMontG1, d + d_pf, cnt * kMontG1, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess)
       e = cudaMemcpyAsync((uint8_t*)values_out + lo * 32, d + d_val, cnt * 32, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess && n_b)
@@ -1207,39 +1129,17 @@ int ptau_kzg_open(ptau_ctx* ctx, const ptau_kzg_powers* powers, const ptau_kzg_p
     ctx->timing.gpu_ms[g] = gms;
     bad_coeff = bad_coeff || s.h_msm_out[0] != 0;
   }
-  if (e != cudaSuccess) {
-    for (int g = 0; g < G; g++) {  // nothing may still be using the buffers when the call returns
-      cudaSetDevice(ctx->gpu[g].device);
-      cudaStreamSynchronize(ctx->gpu[g].stream[0]);
-    }
-    ctx->last_error = std::string("kzg_open: ") + cudaGetErrorString(e);
-    return PTAU_ERR_CUDA;
-  }
+  if (e != cudaSuccess) return drain_fail(ctx, G, __func__, e);
   ctx->timing.wall_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
   return bad_coeff ? PTAU_ERR_ARG : PTAU_OK;
 }
 
 int ptau_selftest_fq_op(ptau_ctx* ctx, int gpu, int op, const void* a, const void* b, void* out, size_t n) {
   if (!ctx || gpu < 0 || gpu >= ctx->n_gpus || !a || !b || !out) return PTAU_ERR_ARG;
-  GpuSlot& s = ctx->gpu[gpu];
-  CUDA_TRY(ctx, cudaSetDevice(s.device));
   void *da = nullptr, *db = nullptr, *dout = nullptr;
-  CUDA_TRY(ctx, cudaMalloc(&da, n * 48 + 16));
-  CUDA_TRY(ctx, cudaMalloc(&db, n * 48 + 16));
-  CUDA_TRY(ctx, cudaMalloc(&dout, n * 48 + 16));
-  cudaError_t e = cudaMemcpyAsync(da, a, n * 48, cudaMemcpyHostToDevice, s.stream[0]);
-  if (e == cudaSuccess) e = cudaMemcpyAsync(db, b, n * 48, cudaMemcpyHostToDevice, s.stream[0]);
-  if (e == cudaSuccess) e = ptau::launch_fq_op(op, da, db, dout, n, s.stream[0]);
-  if (e == cudaSuccess) e = cudaMemcpyAsync(out, dout, n * 48, cudaMemcpyDeviceToHost, s.stream[0]);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(s.stream[0]);
-  cudaFree(da);
-  cudaFree(db);
-  cudaFree(dout);
-  if (e != cudaSuccess) {
-    ctx->last_error = std::string("selftest: ") + cudaGetErrorString(e);
-    return PTAU_ERR_CUDA;
-  }
-  return PTAU_OK;
+  return launch_once(ctx, gpu, __func__, false,
+                     {{a, nullptr, n * 48, &da}, {b, nullptr, n * 48, &db}, {nullptr, out, n * 48, &dout}},
+                     [&](cudaStream_t st) { return ptau::launch_fq_op(op, da, db, dout, n, st); });
 }
 
 int ptau_microbench(ptau_ctx* ctx, int gpu, int kind, int iters, double* ms, double* ops) {
@@ -1261,10 +1161,7 @@ int ptau_microbench(ptau_ctx* ctx, int gpu, int kind, int iters, double* ms, dou
   float t = 0;
   if (e == cudaSuccess) e = cudaEventElapsedTime(&t, s.ev_k0[0], s.ev_k1[0]);
   cudaFree(d_out);
-  if (e != cudaSuccess) {
-    ctx->last_error = std::string("microbench: ") + cudaGetErrorString(e);
-    return PTAU_ERR_CUDA;
-  }
+  if (e != cudaSuccess) return cuda_fail(ctx, __func__, e);
   *ms = t;
   *ops = o;
   return PTAU_OK;

@@ -3,6 +3,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <string.h>
 
 #include <string>
 
@@ -45,3 +46,34 @@ struct ptau_ctx {
   ptau_timing timing;
   std::string last_error;
 };
+
+namespace ptau {
+
+// "<entry point>: <CUDA error>" as the context's last error; returns PTAU_ERR_CUDA
+inline int cuda_fail(ptau_ctx* ctx, const char* where, cudaError_t e) {
+  if (ctx) ctx->last_error = std::string(where) + ": " + cudaGetErrorString(e);
+  return PTAU_ERR_CUDA;
+}
+
+// every call starts with an empty record of what it did
+inline void timing_reset(ptau_ctx* ctx) {
+  memset(&ctx->timing, 0, sizeof(ctx->timing));
+  ctx->timing.n_gpus = ctx->n_gpus;
+}
+
+// [lo, hi): the g-th of G contiguous index ranges that split [0, n) over the context's GPUs
+struct Shard {
+  uint64_t lo, hi;
+};
+inline Shard shard(uint64_t n, int g, int G) {
+  return {(uint64_t)((unsigned __int128)n * g / G), (uint64_t)((unsigned __int128)n * (g + 1) / G)};
+}
+
+}  // namespace ptau
+
+// in an entry point: return from it when a CUDA call fails
+#define CUDA_TRY(ctx, expr)                                                   \
+  do {                                                                        \
+    const cudaError_t e_ = (expr);                                            \
+    if (e_ != cudaSuccess) return ptau::cuda_fail((ctx), __func__, e_);       \
+  } while (0)

@@ -22,6 +22,7 @@
 
 #include "../../include/ptau_b200.h"
 #include "blake2b.h"
+#include "layout.h"
 
 namespace {
 
@@ -188,19 +189,18 @@ int ptau_preprocess_files(ptau_ctx* ctx, int variant, const char* response_path,
   fd_out = open(setup_tmp.c_str(), O_WRONLY | O_CREAT | O_TRUNC, 0644);
   if (fd_out < 0) return fail(PTAU_ERR_IO);
 
-  struct Sec {
-    int group;
-    uint64_t count;
-    int64_t out_off;  // offset of the section's ark output in `kzg_setup`, -1 = checked but not written
-    bool process;
-  };
-  const uint64_t g1_all = (2 * n - 1) * 96 + n * 96;
-  const Sec secs[5] = {
-      {PTAU_G1, 2 * n - 1, 0, true},                                             // tau_g1 -> powers_of_g
-      {PTAU_G2, n, fast ? (int64_t)(g1_all + 384) : -1, true},                   // tau_g2 -> powers_of_h (fast)
-      {PTAU_G1, n, (int64_t)((2 * n - 1) * 96), true},                           // alpha_g1 -> powers_of_gamma_g
-      {PTAU_G1, n, -1, fast || emit_unc},  // beta_g1: fastkgz reads+checks+drops it (:156-159); kgz never reads it
-      {PTAU_G2, 1, -1, emit_unc},          // beta_g2: only ever decompressed into `powersoftau_uncompressed`
+  const auto secs = ptau::response_sections(n);
+  const ptau::SetupLayout L = ptau::setup_layout(variant, n);
+  // offset of each section's ark output in `kzg_setup`, -1 = checked but not written
+  const int64_t out_off[5] = {
+      (int64_t)L.g1(0),                          // tau_g1 -> powers_of_g
+      fast ? (int64_t)L.g2(L.powers_of_h) : -1,  // tau_g2 -> powers_of_h (fast)
+      (int64_t)L.g1(L.gamma_g),                  // alpha_g1 -> powers_of_gamma_g
+      -1, -1};
+  const bool process[5] = {
+      true, true, true,
+      fast || emit_unc,  // beta_g1: fastkgz reads+checks+drops it (:156-159); kgz never reads it
+      emit_unc,          // beta_g2: only ever decompressed into `powersoftau_uncompressed`
   };
   // points per slab: pinned memory is paid for by the page (allocation time), so no more than the pipeline needs
   unsigned slab_log2 = 18;
@@ -220,16 +220,16 @@ int ptau_preprocess_files(ptau_ctx* ctx, int variant, const char* response_path,
   // first stage-2 (read_g1 / read_g2) error, reported only if the decompression of everything after it is clean
   int s2_rc = PTAU_OK, s2_kind = 0, s2_sec = -1;
   uint64_t s2_index = 0;
-  uint64_t in_off = 64;  // skip the 64-byte challenge hash (:96-101)
+  uint64_t in_off = ptau::kResponseHash;  // skip the 64-byte challenge hash (:96-101)
   uint64_t unc_off = 0;
   std::future<bool> wr[2], wu[2];
   for (int s = 0; s < 5 && rc == PTAU_OK; s++) {
-    const Sec& sec = secs[s];
+    const ptau::Section& sec = secs[s];
     const size_t rc_in = ptau_record_size(sec.group, PTAU_FMT_ZCASH_COMPRESSED);
     const size_t r_unc = ptau_record_size(sec.group, PTAU_FMT_ZCASH_UNCOMPRESSED);
     const size_t r_out = ptau_record_size(sec.group, PTAU_FMT_ARK_UNCOMPRESSED);
     const bool only_decompress = (s == 3 && !fast) || s == 4;  // sections the binaries never validate
-    if (sec.process) {
+    if (process[s]) {
       const uint64_t nslab = (sec.count + slab - 1) / slab;
       std::future<bool> rd = std::async(std::launch::async, pread_all, fd_in, inb[0],
                                         (size_t)((sec.count < slab ? sec.count : slab) * rc_in), in_off);
@@ -251,7 +251,7 @@ int ptau_preprocess_files(ptau_ctx* ctx, int variant, const char* response_path,
         const bool stage2 = !only_decompress && s2_rc == PTAU_OK;
         // sections that are checked but not written (kgz: tau_g2 beyond its first slab;
         // fastkgz: beta_g1) are validated on the GPU without copying results back
-        uint8_t* dst = (sec.out_off >= 0 || k == 0) ? outb[b] : nullptr;
+        uint8_t* dst = (out_off[s] >= 0 || k == 0) ? outb[b] : nullptr;
         int rc2 = PTAU_OK;
         if (emit_unc) {
           // stage 1: decompress (CheckForCorrectness::No) -> `powersoftau_uncompressed`
@@ -315,9 +315,9 @@ int ptau_preprocess_files(ptau_ctx* ctx, int variant, const char* response_path,
             if (s == 2) memcpy(first_alpha, outb[b], 96);
             if (s == 1) memcpy(first_g2, outb[b], 384);  // n >= 2
           }
-          if (sec.out_off >= 0)
+          if (out_off[s] >= 0)
             wr[b] = std::async(std::launch::async, pwrite_parts, fd_out, (const void*)outb[b], cnt * r_out,
-                               (uint64_t)sec.out_off + lo * r_out);
+                               (uint64_t)out_off[s] + lo * r_out);
         }
       }
       if (rd.valid()) rd.wait();
@@ -350,9 +350,9 @@ int ptau_preprocess_files(ptau_ctx* ctx, int variant, const char* response_path,
     memcpy(tail, first_g1, 96);
     memcpy(tail + 96, first_alpha, 96);
     memcpy(tail + 192, first_g2, 384);
-    if (!pwrite_all(fd_out, tail, sizeof(tail), g1_all)) return fail(PTAU_ERR_IO);
+    if (!pwrite_all(fd_out, tail, sizeof(tail), L.g1(L.vk_g))) return fail(PTAU_ERR_IO);
   } else {  // h, beta_h in front of powers_of_h (preprocess-fastkgz.rs:199-208)
-    if (!pwrite_all(fd_out, first_g2, 384, g1_all)) return fail(PTAU_ERR_IO);
+    if (!pwrite_all(fd_out, first_g2, 384, L.g2(0))) return fail(PTAU_ERR_IO);
   }
   if (flags & PTAU_FILE_FSYNC) {
     if (fsync(fd_out) != 0 || (fd_unc >= 0 && fsync(fd_unc) != 0)) return fail(PTAU_ERR_IO);
@@ -416,12 +416,12 @@ int ptau_load_setup_file(ptau_ctx* ctx, int variant, const char* setup_path, uin
     close(fd);
     return PTAU_ERR_SIZE;
   }
-  const uint64_t n_g1 = 3 * n - 1 + (fast ? 0 : 2), n_g2 = fast ? n + 2 : 2;
+  const ptau::SetupLayout L = ptau::setup_layout(variant, n);
   if (!g1_out || !g2_out) {  // size query
     close(fd);
     return (g1_out_len == 0 && g2_out_len == 0) ? PTAU_OK : PTAU_ERR_ARG;
   }
-  if (g1_out_len != n_g1 * 104 || g2_out_len != n_g2 * 200) {
+  if (g1_out_len != L.n_g1 * ptau::kMontG1 || g2_out_len != L.n_g2 * ptau::kMontG2) {
     close(fd);
     return PTAU_ERR_SIZE;
   }
@@ -440,7 +440,7 @@ int ptau_load_setup_file(ptau_ctx* ctx, int variant, const char* setup_path, uin
     int group;
     uint64_t count;
     uint8_t* out;
-  } secs[2] = {{PTAU_G1, n_g1, (uint8_t*)g1_out}, {PTAU_G2, n_g2, (uint8_t*)g2_out}};
+  } secs[2] = {{PTAU_G1, L.n_g1, (uint8_t*)g1_out}, {PTAU_G2, L.n_g2, (uint8_t*)g2_out}};
   int rc = PTAU_OK;
   uint64_t off = 0, base = 0;
   for (int s = 0; s < 2 && rc == PTAU_OK; s++) {

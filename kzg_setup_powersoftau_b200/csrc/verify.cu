@@ -27,6 +27,7 @@
 #include "context.h"
 #include "curve.cuh"
 #include "kernels.h"
+#include "layout.h"
 
 namespace ptau {
 
@@ -194,21 +195,6 @@ struct Run {
   }
 };
 
-#define VTRY(expr)                                                                     \
-  do {                                                                                 \
-    cudaError_t e_ = (expr);                                                           \
-    if (e_ != cudaSuccess) {                                                           \
-      ctx->last_error = std::string("verify_powers: ") + #expr + ": " + cudaGetErrorString(e_); \
-      return PTAU_ERR_CUDA;                                                            \
-    }                                                                                  \
-  } while (0)
-
-int rec_bytes(int group, int fmt) {
-  if (fmt == PTAU_FMT_ZCASH_COMPRESSED) return group == PTAU_G1 ? 48 : 96;
-  if (fmt == PTAU_FMT_ARK_UNCOMPRESSED) return group == PTAU_G1 ? 96 : 192;
-  return group == PTAU_G1 ? 104 : 200;
-}
-
 }  // namespace
 }  // namespace ptau
 
@@ -220,9 +206,8 @@ extern "C" int ptau_verify_powers(ptau_ctx* ctx, int kind, const void* data, uin
   if (!ctx || !data) return PTAU_ERR_ARG;
   if (kind != PTAU_POWERS_RESPONSE && kind != PTAU_POWERS_KGZ && kind != PTAU_POWERS_FASTKGZ) return PTAU_ERR_ARG;
   if (n < 2 || n > (1ull << 40)) return PTAU_ERR_ARG;
-  const uint64_t want = kind == PTAU_POWERS_RESPONSE ? ptau_response_size(n)
-                                                     : ptau_setup_size(kind == PTAU_POWERS_KGZ ? PTAU_VARIANT_KGZ
-                                                                                               : PTAU_VARIANT_FASTKGZ, n);
+  const int variant = kind == PTAU_POWERS_KGZ ? PTAU_VARIANT_KGZ : PTAU_VARIANT_FASTKGZ;  // of a setup
+  const uint64_t want = kind == PTAU_POWERS_RESPONSE ? ptau_response_size(n) : ptau_setup_size(variant, n);
   if (len != want) return PTAU_ERR_SIZE;
   const auto t0 = std::chrono::steady_clock::now();
   const uint8_t* base = (const uint8_t*)data;
@@ -236,41 +221,39 @@ extern "C" int ptau_verify_powers(ptau_ctx* ctx, int kind, const void* data, uin
   uint64_t g2_index_offset = 0;  // setups report a G2 index in file order over all points
   if (kind == PTAU_POWERS_RESPONSE) {
     fmt = PTAU_FMT_ZCASH_COMPRESSED;
-    const uint8_t* p = base + 64;  // past the challenge hash; the trailing public key is not read
-    const int grp[5] = {PTAU_G1, PTAU_G2, PTAU_G1, PTAU_G1, PTAU_G2};
-    const uint64_t cnt[5] = {2 * n - 1, n, n, n, 1};
-    for (int s = 0; s < 5; s++) {
-      secs.push_back({grp[s], p, cnt[s]});
-      p += cnt[s] * rec_bytes(grp[s], fmt);
+    const uint8_t* p = base + kResponseHash;  // the trailing public key is not read
+    for (const Section& s : response_sections(n)) {
+      secs.push_back({s.group, p, s.count});
+      p += s.count * rec_size(s.group, fmt);
     }
-    pieces = {{0, 0, 2 * n - 1, PTAU_REL_TAU_G1}, {1, 0, n, PTAU_REL_TAU_G2}, {2, 0, n, PTAU_REL_ALPHA_G1},
+    pieces = {{0, 0, secs[0].count, PTAU_REL_TAU_G1}, {1, 0, n, PTAU_REL_TAU_G2}, {2, 0, n, PTAU_REL_ALPHA_G1},
               {3, 0, n, PTAU_REL_BETA_G1}, {4, 0, 1, 0}};
     keys = {{0, 0, K1_P0}, {0, 1, K1_P1}, {3, 0, K1_BETA0}, {1, 0, K2_Q0}, {1, 1, K2_Q1}, {4, 0, K2_BETA_G2}};
     rel_mask = (1u << PTAU_REL_TAU_G1) | (1u << PTAU_REL_TAU_G2) | (1u << PTAU_REL_ALPHA_G1) | (1u << PTAU_REL_BETA_G1) |
                (1u << PTAU_REL_BETA_G2);
   } else {
     fmt = PTAU_FMT_ARK_UNCOMPRESSED;
-    const bool fast = kind == PTAU_POWERS_FASTKGZ;
-    const uint64_t n_g1 = 3 * n - 1 + (fast ? 0 : 2), n_g2 = fast ? n + 2 : 2;
-    secs.push_back({PTAU_G1, base, n_g1});
-    secs.push_back({PTAU_G2, base + n_g1 * 96, n_g2});
-    g2_index_offset = n_g1;
-    pieces = {{0, 0, 2 * n - 1, PTAU_REL_TAU_G1}, {0, 2 * n - 1, n, PTAU_REL_ALPHA_G1}};
-    keys = {{0, 0, K1_P0}, {0, 1, K1_P1}, {0, 2 * n - 1, K1_GAMMA0}};
+    const SetupLayout L = setup_layout(variant, n);
+    secs.push_back({PTAU_G1, base, L.n_g1});
+    secs.push_back({PTAU_G2, base + L.g2(0), L.n_g2});
+    g2_index_offset = L.n_g1;
+    // powers_of_g are G1 records [0, gamma_g)
+    pieces = {{0, 0, L.gamma_g, PTAU_REL_TAU_G1}, {0, L.gamma_g, n, PTAU_REL_ALPHA_G1}};
+    keys = {{0, 0, K1_P0}, {0, 1, K1_P1}, {0, L.gamma_g, K1_GAMMA0}};
     rel_mask = (1u << PTAU_REL_TAU_G1) | (1u << PTAU_REL_ALPHA_G1);
-    if (fast) {
+    if (variant == PTAU_VARIANT_FASTKGZ) {
       pieces.push_back({1, 0, 2, 0});
-      pieces.push_back({1, 2, n, PTAU_REL_TAU_G2});
-      keys.push_back({1, 2, K2_Q0});
-      keys.push_back({1, 3, K2_Q1});
+      pieces.push_back({1, L.powers_of_h, n, PTAU_REL_TAU_G2});
+      keys.push_back({1, L.powers_of_h, K2_Q0});
+      keys.push_back({1, L.powers_of_h + 1, K2_Q1});
       keys.push_back({1, 0, K2_H});
       keys.push_back({1, 1, K2_BETA_H});
       rel_mask |= 1u << PTAU_REL_TAU_G2;
     } else {
-      pieces.push_back({0, 3 * n - 1, 2, 0});
+      pieces.push_back({0, L.vk_g, 2, 0});
       pieces.push_back({1, 0, 2, 0});
-      keys.push_back({0, 3 * n - 1, K1_G});
-      keys.push_back({0, 3 * n, K1_GAMMA_G});
+      keys.push_back({0, L.vk_g, K1_G});
+      keys.push_back({0, L.vk_g + 1, K1_GAMMA_G});
       keys.push_back({1, 0, K2_Q0});
       keys.push_back({1, 1, K2_Q1});
     }
@@ -310,7 +293,7 @@ extern "C" int ptau_verify_powers(ptau_ctx* ctx, int kind, const void* data, uin
     const uint64_t P = pc.count - 1;
     const int Gp = P >= (uint64_t)G * 4096 ? G : 1;
     for (int g = 0; g < Gp; g++) {
-      const uint64_t lo = P * g / Gp, hi = P * (g + 1) / Gp;
+      const auto [lo, hi] = shard(P, g, Gp);
       for (uint64_t a = lo; a < hi; a += slab) {
         const uint64_t b = a + slab < hi ? a + slab : hi;
         jobs.push_back({g, pi, a, b + 1, run.w[g].parts});
@@ -320,8 +303,8 @@ extern "C" int ptau_verify_powers(ptau_ctx* ctx, int kind, const void* data, uin
     }
   }
   // ---- device buffers (sizes bounded by the slab, i.e. by chunk_points)
-  const int rb_max = 200;
-  const int ri_max = rec_bytes(PTAU_G2, fmt);
+  const int rb_max = kMontG2;
+  const int ri_max = rec_size(PTAU_G2, fmt);
   ptau::MsmPlan p1, p2;
   msm_g1_plan(max_pts, &p1);
   msm_g2_plan(max_pts, &p2);
@@ -332,37 +315,38 @@ extern "C" int ptau_verify_powers(ptau_ctx* ctx, int kind, const void* data, uin
   for (int g = 0; g < G; g++) {
     GpuSlot& s = ctx->gpu[g];
     GpuWork& x = run.w[g];
-    VTRY(cudaSetDevice(s.device));
-    VTRY(cudaMalloc(&x.d_rec, max_pts * rb_max + 16));
-    VTRY(cudaMalloc(&x.d_in[0], conv * ri_max + 16));
-    VTRY(cudaMalloc(&x.d_in[1], conv * ri_max + 16));
-    VTRY(cudaMalloc((void**)&x.d_status, nsec * 8));
-    VTRY(cudaEventCreateWithFlags(&x.ev, cudaEventDisableTiming));
+    CUDA_TRY(ctx, cudaSetDevice(s.device));
+    CUDA_TRY(ctx, cudaMalloc(&x.d_rec, max_pts * rb_max + 16));
+    CUDA_TRY(ctx, cudaMalloc(&x.d_in[0], conv * ri_max + 16));
+    CUDA_TRY(ctx, cudaMalloc(&x.d_in[1], conv * ri_max + 16));
+    CUDA_TRY(ctx, cudaMalloc((void**)&x.d_status, nsec * 8));
+    CUDA_TRY(ctx, cudaEventCreateWithFlags(&x.ev, cudaEventDisableTiming));
     if (x.parts) {
-      VTRY(cudaMalloc(&x.d_sc, max_pts * 32 + 16));
-      VTRY(cudaMalloc(&x.d_scratch, scratch));
-      VTRY(cudaMalloc((void**)&x.d_parts, (size_t)x.parts * 256));
+      CUDA_TRY(ctx, cudaMalloc(&x.d_sc, max_pts * 32 + 16));
+      CUDA_TRY(ctx, cudaMalloc(&x.d_scratch, scratch));
+      CUDA_TRY(ctx, cudaMalloc((void**)&x.d_parts, (size_t)x.parts * 256));
     }
-    VTRY(cudaMemcpyAsync(x.d_status, none_v.data(), nsec * 8, cudaMemcpyHostToDevice, s.stream[0]));
-    VTRY(cudaStreamSynchronize(s.stream[0]));  // none_v is a local; stream[1] must also see the initialised words
+    CUDA_TRY(ctx, cudaMemcpyAsync(x.d_status, none_v.data(), nsec * 8, cudaMemcpyHostToDevice, s.stream[0]));
+    // none_v is a local; stream[1] must also see the initialised words
+    CUDA_TRY(ctx, cudaStreamSynchronize(s.stream[0]));
   }
   uint64_t launches = 0, h2d = 0;
 
   // ---- key points on GPU 0 (their checks are the main pass's; this status word is not read)
   {
     GpuSlot& s = ctx->gpu[0];
-    VTRY(cudaSetDevice(s.device));
-    VTRY(cudaMalloc(&run.d_keys, kKeyWords * 4));
-    VTRY(cudaMalloc(&run.d_keys_in, 256));
-    VTRY(cudaMalloc((void**)&run.d_key_status, 8));
-    VTRY(cudaMemsetAsync(run.d_keys, 0, kKeyWords * 4, s.stream[0]));
+    CUDA_TRY(ctx, cudaSetDevice(s.device));
+    CUDA_TRY(ctx, cudaMalloc(&run.d_keys, kKeyWords * 4));
+    CUDA_TRY(ctx, cudaMalloc(&run.d_keys_in, 256));
+    CUDA_TRY(ctx, cudaMalloc((void**)&run.d_key_status, 8));
+    CUDA_TRY(ctx, cudaMemsetAsync(run.d_keys, 0, kKeyWords * 4, s.stream[0]));
     for (const KeyPoint& kp : keys) {
       const Sec& sc = secs[kp.sec];
-      const int ri = rec_bytes(sc.group, fmt);
+      const int ri = rec_size(sc.group, fmt);
       uint32_t* dst = (uint32_t*)run.d_keys + (sc.group == PTAU_G1 ? kp.slot * 32 : K1_N * 32 + kp.slot * 64);
-      VTRY(cudaMemcpyAsync(run.d_keys_in, sc.data + kp.index * ri, ri, cudaMemcpyHostToDevice, s.stream[0]));
-      VTRY(launch_convert(sc.group, fmt, PTAU_FMT_ARK_MONT_LIMBS, run.d_keys_in, dst, 1, PTAU_CHECKS_STRICT, 0,
-                          run.d_key_status, s.stream[0]));
+      CUDA_TRY(ctx, cudaMemcpyAsync(run.d_keys_in, sc.data + kp.index * ri, ri, cudaMemcpyHostToDevice, s.stream[0]));
+      CUDA_TRY(ctx, launch_convert(sc.group, fmt, PTAU_FMT_ARK_MONT_LIMBS, run.d_keys_in, dst, 1, PTAU_CHECKS_STRICT, 0,
+                                   run.d_key_status, s.stream[0]));
       launches++;
     }
   }
@@ -380,36 +364,38 @@ extern "C" int ptau_verify_powers(ptau_ctx* ctx, int kind, const void* data, uin
       const Job& jb = jobs[per_gpu[g][next[g]++]];
       const Piece& pc = pieces[jb.piece];
       const Sec& sc = secs[pc.sec];
-      const int ri = rec_bytes(sc.group, fmt), rb = sc.group == PTAU_G1 ? 104 : 200;
+      const int ri = rec_size(sc.group, fmt), rb = sc.group == PTAU_G1 ? kMontG1 : kMontG2;
       GpuSlot& s = ctx->gpu[g];
       GpuWork& x = run.w[g];
-      VTRY(cudaSetDevice(s.device));
+      CUDA_TRY(ctx, cudaSetDevice(s.device));
       // the previous slab's MSMs (stream 0) read d_rec: stream 1 starts converting only after them
-      VTRY(cudaEventRecord(x.ev, s.stream[0]));
-      VTRY(cudaStreamWaitEvent(s.stream[1], x.ev, 0));
+      CUDA_TRY(ctx, cudaEventRecord(x.ev, s.stream[0]));
+      CUDA_TRY(ctx, cudaStreamWaitEvent(s.stream[1], x.ev, 0));
       int c = 0;
       for (uint64_t o = jb.a; o < jb.b; o += chunk, c++) {
         const uint64_t m = jb.b - o < chunk ? jb.b - o : chunk;
         const uint64_t idx = pc.first + o;  // section-relative
         cudaStream_t st = s.stream[c & 1];
-        VTRY(cudaMemcpyAsync(x.d_in[c & 1], sc.data + idx * ri, m * ri, cudaMemcpyHostToDevice, st));
-        VTRY(launch_convert(sc.group, fmt, PTAU_FMT_ARK_MONT_LIMBS, x.d_in[c & 1], (uint8_t*)x.d_rec + (o - jb.a) * rb, m,
-                            PTAU_CHECKS_STRICT, idx, x.d_status + pc.sec, st));
+        CUDA_TRY(ctx, cudaMemcpyAsync(x.d_in[c & 1], sc.data + idx * ri, m * ri, cudaMemcpyHostToDevice, st));
+        uint8_t* dst = (uint8_t*)x.d_rec + (o - jb.a) * rb;
+        CUDA_TRY(ctx, launch_convert(sc.group, fmt, PTAU_FMT_ARK_MONT_LIMBS, x.d_in[c & 1], dst, m, PTAU_CHECKS_STRICT,
+                                     idx, x.d_status + pc.sec, st));
         launches++;
         h2d += m * ri;
       }
-      VTRY(cudaEventRecord(x.ev, s.stream[1]));
-      VTRY(cudaStreamWaitEvent(s.stream[0], x.ev, 0));
+      CUDA_TRY(ctx, cudaEventRecord(x.ev, s.stream[1]));
+      CUDA_TRY(ctx, cudaStreamWaitEvent(s.stream[0], x.ev, 0));
       if (jb.part < 0) continue;
       const uint64_t np = jb.b - 1 - jb.a;
       ratio_coeff_kernel<<<(unsigned)((np + 255) / 256), 256, 0, s.stream[0]>>>(key, (uint32_t)pc.rel, jb.a, np,
                                                                                   (uint32_t*)x.d_sc);
-      VTRY(cudaGetLastError());
+      CUDA_TRY(ctx, cudaGetLastError());
       auto msm = sc.group == PTAU_G1 ? launch_msm_g1 : launch_msm_g2;
       int nl = 0;
-      VTRY(msm(x.d_rec, x.d_sc, np, x.d_scratch, x.d_parts + (size_t)jb.part * 256, &nl, s.stream[0]));
+      CUDA_TRY(ctx, msm(x.d_rec, x.d_sc, np, x.d_scratch, x.d_parts + (size_t)jb.part * 256, &nl, s.stream[0]));
       launches += nl + 1;
-      VTRY(msm((uint8_t*)x.d_rec + rb, x.d_sc, np, x.d_scratch, x.d_parts + (size_t)(jb.part + 1) * 256, &nl, s.stream[0]));
+      CUDA_TRY(ctx, msm((uint8_t*)x.d_rec + rb, x.d_sc, np, x.d_scratch, x.d_parts + (size_t)(jb.part + 1) * 256, &nl,
+                        s.stream[0]));
       launches += nl;
     }
   }
@@ -421,18 +407,18 @@ extern "C" int ptau_verify_powers(ptau_ctx* ctx, int kind, const void* data, uin
   for (int g = 0; g < G; g++) {
     GpuSlot& s = ctx->gpu[g];
     GpuWork& x = run.w[g];
-    VTRY(cudaSetDevice(s.device));
-    VTRY(cudaStreamSynchronize(s.stream[1]));
+    CUDA_TRY(ctx, cudaSetDevice(s.device));
+    CUDA_TRY(ctx, cudaStreamSynchronize(s.stream[1]));
     unsigned long long st[8];
-    VTRY(cudaMemcpyAsync(st, x.d_status, nsec * 8, cudaMemcpyDeviceToHost, s.stream[0]));
+    CUDA_TRY(ctx, cudaMemcpyAsync(st, x.d_status, nsec * 8, cudaMemcpyDeviceToHost, s.stream[0]));
     parts[g].resize((size_t)x.parts * 256);
-    if (x.parts) VTRY(cudaMemcpyAsync(parts[g].data(), x.d_parts, parts[g].size(), cudaMemcpyDeviceToHost, s.stream[0]));
-    VTRY(cudaStreamSynchronize(s.stream[0]));
+    if (x.parts)
+      CUDA_TRY(ctx, cudaMemcpyAsync(parts[g].data(), x.d_parts, parts[g].size(), cudaMemcpyDeviceToHost, s.stream[0]));
+    CUDA_TRY(ctx, cudaStreamSynchronize(s.stream[0]));
     for (int i = 0; i < nsec; i++)
       if (st[i] < st_min[i]) st_min[i] = st[i];
   }
-  memset(&ctx->timing, 0, sizeof(ctx->timing));
-  ctx->timing.n_gpus = ctx->n_gpus;
+  timing_reset(ctx);
   for (int i = 0; i < nsec; i++) {
     if (st_min[i] == none) continue;
     uint64_t idx = st_min[i] >> 8;
@@ -451,16 +437,16 @@ extern "C" int ptau_verify_powers(ptau_ctx* ctx, int kind, const void* data, uin
     const int rel = pieces[pi].rel;
     if (!rel) continue;
     const bool g1 = secs[pieces[pi].sec].group == PTAU_G1;
-    const int rb = g1 ? 104 : 200, rw = g1 ? 26 : 50;
+    const int rb = g1 ? kMontG1 : kMontG2;
     for (int ab = 0; ab < 2; ab++) {
       std::vector<uint8_t> recs;
       for (const Job& jb : jobs) {
         if (jb.piece != pi || jb.part < 0) continue;
         const uint8_t* slot = parts[jb.gpu].data() + (size_t)(jb.part + ab) * 256;
         uint32_t bad;
-        memcpy(&bad, slot + rw * 4, 4);
+        memcpy(&bad, slot + rb, 4);
         if (bad) {  // coefficients are < 2^127: cannot happen unless the MSM misread them
-          ctx->last_error = "verify_powers: coefficient rejected by the MSM";
+          ctx->last_error = "ptau_verify_powers: coefficient rejected by the MSM";
           return PTAU_ERR_CUDA;
         }
         recs.insert(recs.end(), slot, slot + rb);
@@ -484,26 +470,25 @@ extern "C" int ptau_verify_powers(ptau_ctx* ctx, int kind, const void* data, uin
   uint8_t is_one[kItems];
   {
     GpuSlot& s = ctx->gpu[0];
-    VTRY(cudaSetDevice(s.device));
-    VTRY(cudaMalloc(&run.d_combo, combo.size()));
-    VTRY(cudaMalloc(&run.d_g1, kItems * 2 * 104));
-    VTRY(cudaMalloc(&run.d_g2, kItems * 2 * 200));
-    VTRY(cudaMalloc(&run.d_flags, 8));
-    VTRY(cudaMalloc(&run.d_one, kItems));
-    VTRY(cudaMemcpyAsync(run.d_combo, combo.data(), combo.size(), cudaMemcpyHostToDevice, s.stream[0]));
+    CUDA_TRY(ctx, cudaSetDevice(s.device));
+    CUDA_TRY(ctx, cudaMalloc(&run.d_combo, combo.size()));
+    CUDA_TRY(ctx, cudaMalloc(&run.d_g1, kItems * 2 * kMontG1));
+    CUDA_TRY(ctx, cudaMalloc(&run.d_g2, kItems * 2 * kMontG2));
+    CUDA_TRY(ctx, cudaMalloc(&run.d_flags, 8));
+    CUDA_TRY(ctx, cudaMalloc(&run.d_one, kItems));
+    CUDA_TRY(ctx, cudaMemcpyAsync(run.d_combo, combo.data(), combo.size(), cudaMemcpyHostToDevice, s.stream[0]));
     verify_assemble_kernel<<<1, 32, 0, s.stream[0]>>>((const uint32_t*)run.d_keys, (const uint32_t*)run.d_combo, kind,
                                                      rel_mask, (uint32_t*)run.d_g1, (uint32_t*)run.d_g2,
                                                      (uint32_t*)run.d_flags);
-    VTRY(cudaGetLastError());
-    VTRY(launch_pairing_product2(run.d_g1, run.d_g2, kItems, nullptr, run.d_one, s.stream[0]));
+    CUDA_TRY(ctx, cudaGetLastError());
+    CUDA_TRY(ctx, launch_pairing_product2(run.d_g1, run.d_g2, kItems, nullptr, run.d_one, s.stream[0]));
     launches += 2;
-    VTRY(cudaMemcpyAsync(flags, run.d_flags, 8, cudaMemcpyDeviceToHost, s.stream[0]));
-    VTRY(cudaMemcpyAsync(is_one, run.d_one, kItems, cudaMemcpyDeviceToHost, s.stream[0]));
-    VTRY(cudaStreamSynchronize(s.stream[0]));
+    CUDA_TRY(ctx, cudaMemcpyAsync(flags, run.d_flags, 8, cudaMemcpyDeviceToHost, s.stream[0]));
+    CUDA_TRY(ctx, cudaMemcpyAsync(is_one, run.d_one, kItems, cudaMemcpyDeviceToHost, s.stream[0]));
+    CUDA_TRY(ctx, cudaStreamSynchronize(s.stream[0]));
   }
   if (combos_out) memcpy(combos_out, combo.data(), combo.size());
-  memset(&ctx->timing, 0, sizeof(ctx->timing));
-  ctx->timing.n_gpus = ctx->n_gpus;
+  timing_reset(ctx);
   ctx->timing.wall_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
   ctx->timing.kernel_launches = launches;
   ctx->timing.h2d_bytes[0] = h2d;
