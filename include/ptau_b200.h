@@ -318,6 +318,44 @@ int ptau_verify_powers(ptau_ctx* ctx, int kind, const void* data, uint64_t len, 
                        const uint8_t seed[32], uint64_t* bad_index, int* bad_kind, int* bad_section, int* bad_relation,
                        void* combos_out);
 
+/* ---- a Powers-of-Tau contribution (powersoftau `compute`) and its check (`verify_transform`) --------------- */
+/* A challenge is the 64-byte BLAKE2b-512 of the previous response followed by the accumulator in uncompressed zcash
+ * records, the sections of ptau_uncompressed_size.  A response is BLAKE2b-512 of the whole challenge, the transformed
+ * accumulator in compressed records and the contributor's public key (1152 bytes, uncompressed): ptau_response_size. */
+uint64_t ptau_challenge_size(uint64_t n_powers);
+/* Transforms the challenge's accumulator with secrets (tau, alpha, beta): tau_g1[i], tau_g2[i] times tau^i, alpha_g1[i]
+ * times alpha tau^i, beta_g1[i] times beta tau^i, beta_g2 times beta; writes the response with the public key of
+ * (tau, alpha, beta) and (s_tau, s_alpha, s_beta), where g1_s = [s]G1 (powersoftau keypair).
+ * secrets: NULL (drawn with getrandom) or 6 x 32-byte little-endian scalars in (0, r): tau, alpha, beta, s_tau, s_alpha,
+ * s_beta.  Every challenge point is read with `checks` and a bad one is reported exactly as ptau_preprocess reports the
+ * same bytes (*bad_section 0-4, *bad_index within it, *bad_kind).  Without PTAU_CHECK_SUBGROUP (or the on-curve check)
+ * the output record of a point outside the subgroup is unspecified; a point at infinity (allowed without
+ * PTAU_CHECK_REJECT_INFINITY) stays infinity.  The secrets and the values derived from them are wiped from host memory
+ * before the call returns.  Device memory per GPU depends on the context's chunk_points only.
+ * A zero or non-canonical secret, n_powers < 2: PTAU_ERR_ARG; a length that does not match n_powers: PTAU_ERR_SIZE. */
+int ptau_contribute(ptau_ctx* ctx, const void* challenge, uint64_t challenge_len, uint64_t n_powers,
+                    const uint8_t* secrets, unsigned checks, void* response_out, uint64_t response_len,
+                    uint64_t* bad_index, int* bad_kind, int* bad_section);
+/* relations of ptau_verify_contribution beyond those of ptau_verify_powers (same_ratio = the pairing ratio check) */
+#define PTAU_REL_HASH 7          /* the response's first 64 bytes are BLAKE2b-512 of the challenge                 */
+#define PTAU_REL_POK_TAU 8       /* same_ratio(key.tau_g1, (g2_s, key.tau_g2)), g2_s = hash_to_g2 of the key      */
+#define PTAU_REL_POK_ALPHA 9     /* the same for alpha                                                            */
+#define PTAU_REL_POK_BETA 10     /* the same for beta                                                             */
+#define PTAU_REL_CHAIN_TAU 11    /* same_ratio((before.tau_g1[1], after.tau_g1[1]), (g2_s, key.tau_g2))           */
+#define PTAU_REL_CHAIN_ALPHA 12  /* same_ratio((before.alpha_g1[0], after.alpha_g1[0]), (g2_s, key.alpha_g2))     */
+#define PTAU_REL_CHAIN_BETA 13   /* same_ratio((before.beta_g1[0], after.beta_g1[0]), (g2_s, key.beta_g2))        */
+#define PTAU_REL_CHAIN_BETA_G2 14 /* same_ratio((before.beta_g1[0], after.beta_g1[0]), (before.beta_g2, after.beta_g2)) */
+/* powersoftau verify_transform of a response against its challenge.  Point checks first, all strict: the public key's
+ * nine points (*bad_section 5, *bad_index 0-5 for its G1 points, 6-8 for its G2 points); the challenge points the
+ * relations read, tau_g1[1], alpha_g1[0], beta_g1[0] and beta_g2 (*bad_section 6 + their section); then the response as
+ * ptau_verify_powers checks it (its points as sections 0-4, its powers relations 0-5, with `seed` as there).  Then
+ * HASH, POK_* and CHAIN_*; the lowest failing relation goes to *bad_relation with PTAU_BAD_NOT_POWERS.
+ * challenge may be NULL: then only the response's own relations are checked (public key + powers), HASH and CHAIN_*
+ * are skipped and the digest the key was made with is the response's first 64 bytes. */
+int ptau_verify_contribution(ptau_ctx* ctx, const void* challenge, uint64_t challenge_len, const void* response,
+                             uint64_t response_len, uint64_t n_powers, const uint8_t seed[32], uint64_t* bad_index,
+                             int* bad_kind, int* bad_section, int* bad_relation);
+
 /* ---- self-test hook --------------------------------------------------------------- */
 /* Raw Fq operations on n pairs of 48-byte Montgomery-limb values (host pointers), computed by
  * the kernels' own field code on the GPU: op 0 mul, 1 add, 2 sub, 3 neg, 4 sqr, 5 a^((p-3)/4),

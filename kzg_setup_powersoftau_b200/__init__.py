@@ -29,6 +29,7 @@ from ._ffi import (  # noqa: F401  (re-exported constants)
     G1, G2, STATUS_NONE, VARIANT_FASTKGZ, VARIANT_KGZ,
     BAD_NOT_POWERS, POWERS_FASTKGZ, POWERS_KGZ, POWERS_RESPONSE, REL_ALPHA_G1, REL_BETA_G1, REL_BETA_G2,
     REL_GENERATORS, REL_KEY, REL_NAMES, REL_TAU_G1, REL_TAU_G2,
+    REL_HASH, REL_POK_TAU, REL_POK_ALPHA, REL_POK_BETA, REL_CHAIN_TAU, REL_CHAIN_ALPHA, REL_CHAIN_BETA, REL_CHAIN_BETA_G2,
 )
 
 # ---- reference constants (src/lib.rs:20-28, src/bin/preprocess-kgz.rs:18-23) --
@@ -297,6 +298,48 @@ class Context:
             section = bad_s.value if (rc > 0 and kind == POWERS_RESPONSE) else None
             self._raise(rc, bad_i.value if rc > 0 else None, section)
         return out
+
+    def contribute(self, challenge, n_powers: int, secrets=None, checks: int = CHECKS_STRICT, out=None) -> np.ndarray:
+        """ptau_contribute: the response of powersoftau `compute` on a challenge (64-byte hash + uncompressed
+        accumulator).  secrets: None (drawn from the OS) or (tau, alpha, beta, s_tau, s_alpha, s_beta) as ints in
+        (0, r), or their 192 bytes (6 x 32, little-endian).  The library wipes its own copies of the secrets before it
+        returns; the Python objects passed in (and the bytes built from them here) are not wiped.  Returns the response
+        bytes (or fills `out`).  A bad
+        challenge point raises PtauError with its section and index, as preprocess reports it."""
+        L = _ffi.lib()
+        src = _as_u8(challenge)
+        sec = None
+        if secrets is not None:
+            sec = bytes(secrets) if isinstance(secrets, (bytes, bytearray)) else b"".join(
+                int(v).to_bytes(32, "little") if 0 <= int(v) < (1 << 256) else b"" for v in secrets)
+            if len(sec) != 192:
+                raise PtauError(_ffi.ERR_ARG, detail="secrets must be six scalars")
+        size = L.ptau_response_size(n_powers)
+        dst = _as_u8(out) if out is not None else np.empty(size, dtype=np.uint8)
+        bad_i, bad_k, bad_s = C.c_uint64(0), C.c_int(0), C.c_int(-1)
+        rc = L.ptau_contribute(self._h, _ptr(src), src.size, n_powers, sec, checks, _ptr(dst), dst.size,
+                               C.byref(bad_i), C.byref(bad_k), C.byref(bad_s))
+        if rc != 0:
+            self._raise(rc, bad_i.value if rc > 0 else None, bad_s.value if rc > 0 else None)
+        return dst
+
+    def verify_contribution(self, challenge, response, n_powers: int, seed: Optional[bytes] = None) -> None:
+        """ptau_verify_contribution (powersoftau verify_transform).  challenge None: the response's own relations only
+        (public key and powers).  Raises PtauError: a bad point with .section (0-4 response, 5 public key, 6 + s the
+        challenge's section s) and .index, or BAD_NOT_POWERS with .relation."""
+        resp = _as_u8(response)
+        chal = _as_u8(challenge) if challenge is not None else None
+        if seed is not None and len(seed) != 32:
+            raise PtauError(_ffi.ERR_ARG, detail="seed must be 32 bytes")
+        bad_i, bad_k, bad_s, bad_r = C.c_uint64(0), C.c_int(0), C.c_int(-1), C.c_int(-1)
+        rc = _ffi.lib().ptau_verify_contribution(self._h, _ptr(chal) if chal is not None else None,
+                                                 chal.size if chal is not None else 0, _ptr(resp), resp.size, n_powers,
+                                                 bytes(seed) if seed is not None else None, C.byref(bad_i),
+                                                 C.byref(bad_k), C.byref(bad_s), C.byref(bad_r))
+        if rc == BAD_NOT_POWERS:
+            raise PtauError(rc, relation=bad_r.value)
+        if rc != 0:
+            self._raise(rc, bad_i.value if rc > 0 else None, bad_s.value if rc > 0 else None)
 
     def msm_g2(self, points, scalars) -> np.ndarray:
         """sum_i scalars[i] * points[i] over G2 (ptau_msm_g2): points [n, 200] Montgomery-limb records, scalars ints
@@ -878,3 +921,104 @@ def preprocess_fastkgz(directory: str = ".", log2_powers: int = DEFAULT_LOG2_POW
                        checks: int = CHECKS_STRICT, ctx: Optional[Context] = None) -> str:
     """main() of src/bin/preprocess-fastkgz.rs:180-214."""
     return _preprocess_main(VARIANT_FASTKGZ, directory, log2_powers, expected_digest, emit_uncompressed, checks, ctx)
+
+
+# ---- a Powers-of-Tau contribution (powersoftau compute / verify_transform / new_challenge) -------------------------
+def _write_new(path: str, size: int, fill) -> None:
+    """Creates `path` atomically: `fill` writes a memory-mapped temporary file of `size` bytes in the same directory,
+    which is then linked to `path` (never replacing an existing file: FileExistsError) and removed."""
+    if os.path.exists(path):
+        raise FileExistsError(path)
+    tmp = "%s.tmp-%d" % (path, os.getpid())
+    try:
+        with open(tmp, "wb") as f:
+            f.truncate(size)
+        m = np.memmap(tmp, dtype=np.uint8, mode="r+", shape=(size,))
+        try:
+            fill(m)
+            m.flush()
+        finally:
+            del m
+        os.link(tmp, path)
+    finally:
+        if os.path.exists(tmp):
+            os.unlink(tmp)
+
+
+def _read_map(path: str) -> np.ndarray:
+    if not os.path.exists(path):
+        raise FileNotFoundError(path)
+    return np.memmap(path, dtype=np.uint8, mode="r")
+
+
+def challenge_from_response(response_path: str, challenge_path: str, log2_powers: int = DEFAULT_LOG2_POWERS,
+                            ctx: Optional[Context] = None, checks: int = CHECKS_STRICT) -> bytes:
+    """powersoftau new_challenge: writes BLAKE2b(response) || the response's accumulator in uncompressed records to
+    `challenge_path` (created new).  This is how a downloaded response becomes the challenge of one's own
+    contribution.  Returns the new challenge's 64-byte prefix."""
+    L = _ffi.lib()
+    n = 1 << log2_powers
+    ctx = ctx or default_context()
+    resp = _read_map(response_path)
+    if resp.size != L.ptau_response_size(n):
+        raise PtauError(_ffi.ERR_SIZE, detail="%s is not a response of 2^%d powers" % (response_path, log2_powers))
+    hx = C.create_string_buffer(129)
+    rc = L.ptau_blake2b_file(response_path.encode(), hx)
+    if rc != 0:
+        raise PtauError(rc, detail=response_path)
+    digest = bytes.fromhex(hx.value.decode())
+
+    def fill(m):
+        m[:64] = np.frombuffer(digest, dtype=np.uint8)
+        ri, ro = 64, 64
+        for s, (group, count) in enumerate(((G1, 2 * n - 1), (G2, n), (G1, n), (G1, n), (G2, 1))):
+            ci, cu = L.ptau_record_size(group, FMT_ZCASH_COMPRESSED), L.ptau_record_size(group, FMT_ZCASH_UNCOMPRESSED)
+            try:
+                ctx.convert(group, FMT_ZCASH_COMPRESSED, resp[ri:ri + count * ci], FMT_ZCASH_UNCOMPRESSED, checks,
+                            out=m[ro:ro + count * cu])
+            except PtauError as e:
+                e.section = s
+                raise
+            ri += count * ci
+            ro += count * cu
+
+    try:
+        _write_new(challenge_path, L.ptau_challenge_size(n), fill)
+    finally:
+        del resp
+    return digest
+
+
+def contribute(challenge_path: str, response_path: str, log2_powers: int = DEFAULT_LOG2_POWERS,
+               ctx: Optional[Context] = None, secrets=None, checks: int = CHECKS_STRICT) -> bytes:
+    """powersoftau compute: reads `challenge_path`, writes the response to `response_path` (created new) and returns
+    the response's 64-byte prefix (BLAKE2b of the challenge).  secrets: None draws them from the OS inside the
+    library, which wipes its copies before returning; secrets passed in as Python ints or bytes stay in the caller's
+    objects, which Python cannot wipe."""
+    L = _ffi.lib()
+    n = 1 << log2_powers
+    ctx = ctx or default_context()
+    chal = _read_map(challenge_path)
+    if chal.size != L.ptau_challenge_size(n):
+        raise PtauError(_ffi.ERR_SIZE, detail="%s is not a challenge of 2^%d powers" % (challenge_path, log2_powers))
+    try:
+        _write_new(response_path, L.ptau_response_size(n),
+                   lambda m: ctx.contribute(chal, n, secrets=secrets, checks=checks, out=m))
+    finally:
+        del chal
+    with open(response_path, "rb") as f:
+        return f.read(64)
+
+
+def verify_contribution(challenge_path: Optional[str], response_path: str, log2_powers: int = DEFAULT_LOG2_POWERS,
+                        ctx: Optional[Context] = None, seed: Optional[bytes] = None) -> None:
+    """powersoftau verify_transform of `response_path` against `challenge_path` (None: the response's public key and
+    powers only).  Raises PtauError on failure."""
+    n = 1 << log2_powers
+    ctx = ctx or default_context()
+    resp = _read_map(response_path)
+    chal = _read_map(challenge_path) if challenge_path is not None else None
+    try:
+        ctx.verify_contribution(chal, resp, n, seed=seed)
+    finally:
+        del resp, chal

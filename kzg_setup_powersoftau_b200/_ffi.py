@@ -30,6 +30,8 @@ VARIANT_KGZ, VARIANT_FASTKGZ = 1, 2
 STATUS_NONE = 0xFFFFFFFFFFFFFFFF
 POWERS_RESPONSE, POWERS_KGZ, POWERS_FASTKGZ = 1, 2, 3
 REL_GENERATORS, REL_TAU_G1, REL_TAU_G2, REL_ALPHA_G1, REL_BETA_G1, REL_BETA_G2, REL_KEY = 0, 1, 2, 3, 4, 5, 6
+REL_HASH, REL_POK_TAU, REL_POK_ALPHA, REL_POK_BETA = 7, 8, 9, 10
+REL_CHAIN_TAU, REL_CHAIN_ALPHA, REL_CHAIN_BETA, REL_CHAIN_BETA_G2 = 11, 12, 13, 14
 
 BAD_NAMES = {
     BAD_NON_CANONICAL: "NON_CANONICAL",
@@ -39,7 +41,8 @@ BAD_NAMES = {
     BAD_NOT_IN_SUBGROUP: "NOT_IN_SUBGROUP",
     BAD_NOT_POWERS: "NOT_POWERS",
 }
-REL_NAMES = ("GENERATORS", "TAU_G1", "TAU_G2", "ALPHA_G1", "BETA_G1", "BETA_G2", "KEY")
+REL_NAMES = ("GENERATORS", "TAU_G1", "TAU_G2", "ALPHA_G1", "BETA_G1", "BETA_G2", "KEY", "HASH", "POK_TAU", "POK_ALPHA",
+             "POK_BETA", "CHAIN_TAU", "CHAIN_ALPHA", "CHAIN_BETA", "CHAIN_BETA_G2")
 
 
 class Timing(C.Structure):
@@ -138,6 +141,17 @@ _SIGNATURES = {
         C.c_int,
         [C.c_void_p, C.c_int, C.c_void_p, C.c_uint64, C.c_uint64, C.c_char_p, C.POINTER(C.c_uint64), C.POINTER(C.c_int),
          C.POINTER(C.c_int), C.POINTER(C.c_int), C.c_void_p],
+    ),
+    "ptau_challenge_size": (C.c_uint64, [C.c_uint64]),
+    "ptau_contribute": (
+        C.c_int,
+        [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_char_p, C.c_uint, C.c_void_p, C.c_uint64,
+         C.POINTER(C.c_uint64), C.POINTER(C.c_int), C.POINTER(C.c_int)],
+    ),
+    "ptau_verify_contribution": (
+        C.c_int,
+        [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_uint64, C.c_char_p, C.POINTER(C.c_uint64),
+         C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)],
     ),
     "ptau_selftest_fq_op": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t]),
     "ptau_microbench": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double)]),

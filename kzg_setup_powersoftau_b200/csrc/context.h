@@ -61,6 +61,21 @@ inline void timing_reset(ptau_ctx* ctx) {
   ctx->timing.n_gpus = ctx->n_gpus;
 }
 
+// the double buffers d_in or d_out of a slot, each at least `need` bytes; the capacity reads 0 until all of them are
+// allocated, so a failed call leaves no buffer a later call would trust
+inline cudaError_t ensure_buffers(void* (&d)[kBufs], size_t* cap, size_t need) {
+  if (need <= *cap) return cudaSuccess;
+  *cap = 0;
+  for (int b = 0; b < kBufs; b++) {
+    cudaError_t e = d[b] ? cudaFree(d[b]) : cudaSuccess;
+    d[b] = nullptr;
+    if (e == cudaSuccess) e = cudaMalloc(&d[b], need);
+    if (e != cudaSuccess) return e;
+  }
+  *cap = need;
+  return cudaSuccess;
+}
+
 // [lo, hi): the g-th of G contiguous index ranges that split [0, n) over the context's GPUs
 struct Shard {
   uint64_t lo, hi;

@@ -91,15 +91,10 @@ __device__ __forceinline__ void stage_out(uint32_t* __restrict__ g, const uint32
   }
 }
 
-// shared -> global, flat (the generators: records written at their natural stride)
-template <int BLK>
-__device__ __forceinline__ void stage_out_flat(uint32_t* __restrict__ g, const uint32_t* sm, int nwords) {
-  int nvec = nwords >> 2;
-  uint4* g4 = reinterpret_cast<uint4*>(g);
-  const uint4* s4 = reinterpret_cast<const uint4*>(sm);
-  for (int i = threadIdx.x; i < nvec; i += BLK) g4[i] = s4[i];
-  for (int i = (nvec << 2) + threadIdx.x; i < nwords; i += BLK) g[i] = sm[i];
-}
+}  // namespace ptau
+// stage_out_flat and the affine + encode tail of the generator, shared with the contribution kernel
+#include "gen_tail.cuh"
+namespace ptau {
 
 // shared memory of one block: the record staging buffer (BLK x max(stride_in, stride_out)) and, for the G2 kernels
 // with curve checks, the operand file of the subgroup ladder (PTAU_PARK_WORDS per thread, transposed: conflict-free)
@@ -401,13 +396,6 @@ cudaError_t launch_generate(int group, int fmt, const uint32_t* d_scalars, void*
 // with the v1 kernel.  No exceptional cases: the partial sums are < 256^w <= d*256^w and
 // k < r, so an addition never meets equal or opposite points.
 // =============================================================================
-#define PTAU_GEN_B 8
-
-struct FrParams {
-  uint32_t s0[8];         // scalar0, Montgomery form
-  uint32_t pw[64][8];     // step^(2^j), Montgomery form
-};
-
 }  // namespace ptau
 // K_FR_MOD, fr_mul; included here so that the constant bank keeps its layout
 #include "fr.cuh"
@@ -520,57 +508,8 @@ __global__ void __launch_bounds__(PTAU_BLOCK)
     pts[j] = acc;
     pre[j] = (j == 0) ? acc.Z : fmul(pre[j - 1], acc.Z);
   }
-  // ---- batch inversion (Montgomery's trick) ----
-  F inv = FieldInv<F>::inv(pre[PTAU_GEN_B - 1]);
-#pragma unroll 1
-  for (int j = PTAU_GEN_B - 1; j >= 0; j--) {
-    F zi = (j == 0) ? inv : fmul(inv, pre[j - 1]);
-    if (j) inv = fmul(inv, pts[j].Z);
-    F zi2 = fsqr(zi);
-    F xm = fmul(pts[j].X, zi2);
-    F ym = fmul(pts[j].Y, fmul(zi2, zi));
-    const uint64_t rec0 = blk0 + (uint64_t)j * PTAU_BLOCK;
-    uint32_t* o = sm + tid * WOUT;
-    if (rec0 + tid < n) {
-      if (G == PTAU_G1) {
-        const Fq& xq = reinterpret_cast<const Fq&>(xm);
-        const Fq& yq = reinterpret_cast<const Fq&>(ym);
-        Fq xp = fq_from_mont(xq), yp = fq_from_mont(yq);
-        if (OUTFMT == PTAU_FMT_ZCASH_COMPRESSED) {
-          xp.l[11] |= 0x80000000u | (fq_plain_is_largest(yp) ? 0x20000000u : 0u);
-          fq_to_be_words(xp, o);
-        } else {
-          fq_to_be_words(xp, o);
-          fq_to_be_words(yp, o + 12);
-        }
-      } else {
-        const Fq2& xq = reinterpret_cast<const Fq2&>(xm);
-        const Fq2& yq = reinterpret_cast<const Fq2&>(ym);
-        Fq2 xp, yp;
-        xp.c0 = fq_from_mont(xq.c0);
-        xp.c1 = fq_from_mont(xq.c1);
-        yp.c0 = fq_from_mont(yq.c0);
-        yp.c1 = fq_from_mont(yq.c1);
-        if (OUTFMT == PTAU_FMT_ZCASH_COMPRESSED) {
-          bool largest = fq_is_zero(yp.c1) ? fq_plain_is_largest(yp.c0) : fq_plain_is_largest(yp.c1);
-          xp.c1.l[11] |= 0x80000000u | (largest ? 0x20000000u : 0u);
-          fq_to_be_words(xp.c1, o);
-          fq_to_be_words(xp.c0, o + 12);
-        } else {
-          fq_to_be_words(xp.c1, o);
-          fq_to_be_words(xp.c0, o + 12);
-          fq_to_be_words(yp.c1, o + 24);
-          fq_to_be_words(yp.c0, o + 36);
-        }
-      }
-    }
-    __syncthreads();
-    if (rec0 < n) {
-      const int nrec = (int)((n - rec0) < (uint64_t)PTAU_BLOCK ? (n - rec0) : (uint64_t)PTAU_BLOCK);
-      stage_out_flat<PTAU_BLOCK>(out + rec0 * WOUT, sm, nrec * WOUT);
-    }
-    __syncthreads();
-  }
+  // ---- batch inversion (Montgomery's trick), affine, encode, store ----
+  affine_encode_tail<G, OUTFMT, FieldInv<F>>(pts, pre, sm, out, tid, blk0, n);
 }
 
 cudaError_t launch_generate_win(int group, int fmt, const uint32_t* s0_mont, const uint32_t (*pw_mont)[8],

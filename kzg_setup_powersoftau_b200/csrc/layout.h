@@ -52,6 +52,13 @@ inline uint64_t response_bytes(uint64_t n, int fmt) {
   for (const Section& s : response_sections(n)) b += s.count * rec_size(s.group, fmt);
   return b;
 }
+// byte offset of section `sec` (0..4) within the sections of a response / accumulator in records of `fmt`
+inline uint64_t section_offset(uint64_t n, int fmt, int sec) {
+  const auto secs = response_sections(n);
+  uint64_t b = 0;
+  for (int s = 0; s < sec; s++) b += secs[s].count * rec_size(secs[s].group, fmt);
+  return b;
+}
 
 // `kzg_setup` in ark uncompressed records: every G1 record, then every G2 record.  Positions are record indices
 // within their group; g1() and g2() turn them into byte offsets.

@@ -103,4 +103,14 @@ extern "C" {
         ctx: *mut ptau_ctx, g1: *const c_void, g2: *const c_void, n: usize, gt_out: *mut c_void, is_one: *mut u8,
     ) -> c_int;
     pub fn ptau_g2_prepare(ctx: *mut ptau_ctx, g2: *const c_void, n: usize, coeffs_out: *mut c_void, infinity_out: *mut u8) -> c_int;
+    pub fn ptau_challenge_size(n_powers: u64) -> u64;
+    pub fn ptau_contribute(
+        ctx: *mut ptau_ctx, challenge: *const c_void, challenge_len: u64, n_powers: u64, secrets: *const u8, checks: c_uint,
+        response_out: *mut c_void, response_len: u64, bad_index: *mut u64, bad_kind: *mut c_int, bad_section: *mut c_int,
+    ) -> c_int;
+    pub fn ptau_verify_contribution(
+        ctx: *mut ptau_ctx, challenge: *const c_void, challenge_len: u64, response: *const c_void, response_len: u64,
+        n_powers: u64, seed: *const u8, bad_index: *mut u64, bad_kind: *mut c_int, bad_section: *mut c_int,
+        bad_relation: *mut c_int,
+    ) -> c_int;
 }

@@ -16,6 +16,8 @@
 //!   * edge_cases.json: every malformed / boundary record with the status the oracle expects in the three check modes;
 //!     `read` = what read_g1/read_g2 (ark 0.2 deserialize_uncompressed) answers, `nocheck` = deserialize_unchecked
 //!     resp. pairing's into_affine_unchecked.
+//!   * n8_challenge.bin -> n8_contribution.bin: a contribution with fixed secrets, checked with the `powersoftau`
+//!     crate's hash_to_g2 and PublicKey::deserialize and pairing 0.14.2's pairing (contribution_matches_powersoftau_crate)
 //! Each [dagger] assumption of SURVEY.md 8a-3/5/6/7/9 is named at the assertion that would flip if it were wrong;
 //! tests/test_dagger_assumptions.py holds the same list on the oracle side.
 use ark_bls12_381::Bls12_381;
@@ -276,4 +278,84 @@ fn shim_g2_prepare_equals_ark() {
         assert_eq!(want.infinity, *inf);
         assert_eq!(&want.ell_coeffs, coeffs);
     }
+}
+
+/// The golden contribution (tests/golden/n8_challenge.bin -> n8_contribution.bin, tools/make_golden.py) against the
+/// real `powersoftau` crate and pairing 0.14.2: its prefix is BLAKE2b of the challenge, its public key deserializes
+/// with the crate's strict checks, every G2 element is [x] hash_to_g2(BLAKE2b(personalization || digest || g1_s ||
+/// g1_s_x)) computed by the crate's own `hash_to_g2` (rand 0.4 ChaChaRng, `G2::rand`), the proofs of knowledge hold
+/// by pairing, and the transformed accumulator is the challenge's times the known secrets.  This is what pins the
+/// recalled rand 0.4 / `Fq::rand` / `G2::rand` behaviour of csrc/contribute.cuh; the crate's `verify_transform` is
+/// fixed at 2^21 powers and cannot take N = 8.
+#[test]
+fn contribution_matches_powersoftau_crate() {
+    use pairing::bls12_381::{Fr, FrRepr, G1Affine, G2Affine};
+    use pairing::{CurveProjective, Field, PrimeField};
+    // tau, alpha, beta, s_tau, s_alpha, s_beta: tests/contribute_oracle.py GOLDEN_SECRETS
+    const SECRETS: [u64; 6] = [0x2A5F3C91D7E04B86, 0x6C1E9A74B3F2D058, 0x1F8B6E3D5A7C9042, 0x3B7D1F5E9C2A6084,
+                               0x5E2C8A4F1D6B3097, 0x7A4E2C6F8B1D5039];
+    let fr = |v: u64| Fr::from_repr(FrRepr([v, 0, 0, 0])).unwrap();
+    let chal = golden("n8_challenge.bin");
+    let resp = golden("n8_contribution.bin");
+    let digest = blake2b_simd::blake2b(&chal);
+    assert_eq!(&resp[..64], digest.as_bytes());
+    let pk = &resp[resp.len() - powersoftau::PUBLIC_KEY_SIZE..];
+    powersoftau::PublicKey::deserialize(&mut &pk[..]).expect("strict public key");
+    let g1 = |i: usize| {
+        let mut e = G1Uncompressed::empty();
+        e.as_mut().copy_from_slice(&pk[96 * i..96 * (i + 1)]);
+        e.into_affine().unwrap()
+    };
+    let g2 = |i: usize| {
+        let mut e = G2Uncompressed::empty();
+        e.as_mut().copy_from_slice(&pk[576 + 192 * i..576 + 192 * (i + 1)]);
+        e.into_affine().unwrap()
+    };
+    for i in 0..3 {
+        let (s, sx, x_g2s) = (g1(2 * i), g1(2 * i + 1), g2(i));
+        let (x, sv) = (fr(SECRETS[i]), fr(SECRETS[3 + i]));
+        assert_eq!(s, G1Affine::one().mul(sv).into_affine());
+        assert_eq!(sx, s.mul(x).into_affine());
+        let mut h = blake2b_simd::State::new();
+        h.update(&[i as u8]);
+        h.update(digest.as_bytes());
+        h.update(s.into_uncompressed().as_ref());
+        h.update(sx.into_uncompressed().as_ref());
+        let g2_s: G2Affine = powersoftau::hash_to_g2(h.finalize().as_bytes()).into_affine();
+        assert_eq!(x_g2s, g2_s.mul(x).into_affine(), "hash_to_g2 of key pair {}", i);
+        assert_eq!(s.pairing_with(&x_g2s), sx.pairing_with(&g2_s), "proof of knowledge {}", i);
+    }
+    // the body: tau_g1[i] * tau^i ... beta_g2 * beta, section by section (decompressed with pairing's own code)
+    let (tau, alpha, beta) = (fr(SECRETS[0]), fr(SECRETS[1]), fr(SECRETS[2]));
+    let (mut off_u, mut off_c) = (64usize, 64usize);
+    for (sec, count) in [(0usize, 2 * N - 1), (1, N), (2, N), (3, N), (4, 1)].iter() {
+        let mut t = Fr::one();
+        for _ in 0..*count {
+            let mut k = t;
+            if *sec == 2 {
+                k.mul_assign(&alpha);
+            } else if *sec >= 3 {
+                k.mul_assign(&beta);
+            }
+            if *sec == 1 || *sec == 4 {
+                let mut u = G2Uncompressed::empty();
+                u.as_mut().copy_from_slice(&chal[off_u..off_u + 192]);
+                let mut c = G2Compressed::empty();
+                c.as_mut().copy_from_slice(&resp[off_c..off_c + 96]);
+                assert_eq!(c.into_affine().unwrap(), u.into_affine().unwrap().mul(k).into_affine());
+                off_u += 192;
+                off_c += 96;
+            } else {
+                let mut u = G1Uncompressed::empty();
+                u.as_mut().copy_from_slice(&chal[off_u..off_u + 96]);
+                let mut c = G1Compressed::empty();
+                c.as_mut().copy_from_slice(&resp[off_c..off_c + 48]);
+                assert_eq!(c.into_affine().unwrap(), u.into_affine().unwrap().mul(k).into_affine());
+                off_u += 96;
+                off_c += 48;
+            }
+            t.mul_assign(&tau);
+        }
+    }
+    assert_eq!(off_c + powersoftau::PUBLIC_KEY_SIZE, resp.len());
 }

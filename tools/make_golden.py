@@ -7,6 +7,7 @@ artefact the reference binaries/loaders derive from it, plus a table of malforme
 records with the status each check mode must report.  Committed together with this
 script; regenerate with `python tools/make_golden.py`.
 """
+import hashlib
 import json
 import os
 import random
@@ -267,4 +268,13 @@ while True:
 with open(os.path.join(OUT, "edge_cases.json"), "w") as f:
     json.dump({"seed": SEED, "n_powers": N, "scalars": [hex(v) for v in o.derive_scalars(SEED)], "cases": cases}, f,
               indent=1)
+# ---- a contribution (powersoftau new_challenge + compute) to the response above, with fixed secrets ------------
+sys.path.insert(0, os.path.join(ROOT, "tests"))
+import contribute_oracle as co  # noqa: E402
+
+challenge = hashlib.blake2b(resp).digest() + unc
+assert len(challenge) == 64 + o.uncompressed_size(N)
+w("n8_challenge.bin", challenge)
+w("n8_contribution.bin", co.contribute(challenge, N, co.GOLDEN_SECRETS))
+
 print("golden files written:", sorted(os.listdir(OUT)), "edge cases:", len(cases))
