@@ -248,6 +248,31 @@ int ptau_kzg_open(ptau_ctx* ctx, const ptau_kzg_powers* powers, const ptau_kzg_p
                   const void* coeffs, size_t n, const void* blinding, size_t n_b, const void* points, size_t k,
                   void* proofs_out, void* values_out, void* random_v_out);
 
+/* KZG10 opening of one polynomial on whole cosets, one proof per coset.  For k = 2^log2_k (0 <= log2_k <= 20),
+ * omega_k = omega^(2^(32 - log2_k)) with omega = 7^((r - 1) / 2^32) mod r, and each shift h_i (0 < h_i < r):
+ *   p = (X^k - c_i) q_i + r_i with c_i = h_i^k,   proofs_out[i] = sum_{j < n - k} q_{i,j} powers_of_g[j]
+ *   (the infinity record when n <= k),   values_out[i][m] = p(h_i omega_k^m) for m < k, natural order.
+ * powers: device-resident (ptau_kzg_powers_upload); coeffs: n scalars, shifts: m scalars (32 B LE, < r).
+ * proofs_out m x 104 (ARK_MONT_LIMBS), values_out m x k x 32.  log2_k outside [0, 20], n > powers' count, a shift
+ * that is 0 or >= r, a coefficient >= r, a handle of another context or a NULL output: PTAU_ERR_ARG.
+ * The quotient is an exact strided scan on the device straight into the MSM's scalars; the values are one batched
+ * NTT per GPU of the remainders scaled by h_i^j; the cosets are split in contiguous ranges over the context's GPUs. */
+int ptau_kzg_open_cosets(ptau_ctx* ctx, const ptau_kzg_powers* powers, const void* coeffs, size_t n, int log2_k,
+                         const void* shifts, size_t m, void* proofs_out, void* values_out);
+
+/* Batched check of m coset openings with one k = 2^log2_k: item i is (comms[i], shifts[i], values[i][0..k),
+ * proofs[i]) as ptau_kzg_open_cosets returns them.  With I_i the interpolant of the values on the coset,
+ * c_i = h_i^k and 127-bit randomizers rho_i (BLAKE2b keyed with the 32-byte seed, as ptau_verify_powers derives its
+ * coefficients, domain byte 0x20; seed NULL: 32 bytes from getrandom), *ok = 1 iff
+ *   e(sum rho_i (C_i + [c_i] pi_i) - [sum_j (sum_i rho_i I_{i,j}) tau^j] G, h) e(-sum rho_i pi_i, tau_k_h) = 1.
+ * powers: >= k resident G1 powers (powers_of_g); h, tau_k_h: 200-byte G2 records h and [tau^k] h (fastkgz
+ * powers_of_h[0] and powers_of_h[k]; a kgz setup's beta_h serves k = 1).  comms, proofs m x 104; shifts m x 32;
+ * values m x k x 32.  A false item passes with probability at most 2^-127 over a fresh seed.  The same argument
+ * errors as ptau_kzg_open_cosets (k > powers' count, a value >= r).  m = 0: *ok = 1.  GPU 0 only. */
+int ptau_kzg_check_cosets(ptau_ctx* ctx, const ptau_kzg_powers* powers, const void* h, const void* tau_k_h, int log2_k,
+                          const void* comms, const void* shifts, const void* values, const void* proofs, size_t m,
+                          const uint8_t* seed, uint8_t* ok);
+
 /* KZG10::check for n openings in parallel -- ark-poly-commit 0.2 kzg10 `check`, the call the reference's
  * consumer code makes at /root/reference/src/lib.rs:276-286:
  *     e(C_i - [v_i] g - [rv_i] gamma_g, h) == e(w_i, beta_h - [z_i] h)

@@ -364,6 +364,18 @@ class Context:
 
 
 R_ORDER = 0x73EDA753299D7D483339D80809A1D80553BDA402FFFE5BFEFFFFFFFF00000001  # Fr modulus
+# 7^((r - 1) / 2^32) mod r: a root of unity of order 2^32 (ark-bls12-381 Fr TWO_ADIC_ROOT_OF_UNITY, GENERATOR 7)
+FR_ROOT_OF_UNITY = 0x16A2A19EDFE81F20D09B681922C813B4B63683508C2280B93829971F439F0D2B
+
+
+def coset_points(log2_k: int, h: int) -> list:
+    """The points h omega_k^m, m < k = 2^log2_k, of the coset KZG10.open_cosets opens, in its order."""
+    w = pow(FR_ROOT_OF_UNITY, 1 << (32 - log2_k), R_ORDER)
+    pts, x = [], int(h) % R_ORDER
+    for _ in range(1 << log2_k):
+        pts.append(x)
+        x = x * w % R_ORDER
+    return pts
 
 
 class KZG10:
@@ -482,6 +494,67 @@ class KZG10:
             return [int.from_bytes(raw[32 * i:32 * i + 32], "little") for i in range(k)]
 
         return ints(vals), proofs, None if rvs is None else ints(rvs)
+
+    @staticmethod
+    def open_cosets(powers: "Powers", coeffs, log2_k: int, shifts, ctx: Optional["Context"] = None):
+        """Open one polynomial on whole cosets {h omega_k^m : m < k}, k = 2^log2_k (0 <= log2_k <= 20), one proof per
+        shift h (ptau_kzg_open_cosets): the proof commits to q with p = (X^k - h^k) q + r, the values are p at the
+        coset's points in natural order (coset_points(log2_k, h)).  powers: Powers of arrays (the first len(coeffs)
+        powers_of_g are uploaded for the call) or Powers.to_device().  coeffs / shifts: ints or [m, 32] u8 arrays.
+        Returns (values: m lists of k ints, proofs: u8 [m, 104])."""
+        ctx = ctx or default_context()
+        c, h = KZG10._scalars(coeffs), KZG10._scalars(shifts)
+        n, m, k = c.size // 32, h.size // 32, 1 << log2_k if 0 <= log2_k <= 20 else 0
+        pg = powers.powers_of_g
+        if not isinstance(pg, ResidentPoints):
+            if n > len(pg):
+                raise PtauError(_ffi.ERR_ARG, detail="polynomial degree exceeds the supported degree")  # TooManyCoefficients
+            pg = ResidentPoints(ctx, np.asarray(pg)[:n])
+        proofs = np.zeros((m, 104), dtype=np.uint8)
+        vals = np.zeros(m * k * 32, dtype=np.uint8)
+        rc = _ffi.lib().ptau_kzg_open_cosets(ctx._h, pg._h, _ptr(c) if n else None, n, log2_k, _ptr(h) if m else None, m,
+                                             _ptr(proofs) if m else None, _ptr(vals) if m else None)
+        if rc != 0:
+            ctx._raise(rc)
+        raw = vals.tobytes()
+        return [[int.from_bytes(raw[32 * (i * k + j):32 * (i * k + j + 1)], "little") for j in range(k)]
+                for i in range(m)], proofs
+
+    @staticmethod
+    def check_cosets(powers_of_g, h, tau_k_h, log2_k: int, comms, shifts, values, proofs, seed: Optional[bytes] = None,
+                     ctx: Optional["Context"] = None) -> bool:
+        """Batched check of coset openings with one k = 2^log2_k (ptau_kzg_check_cosets): item i is (comms[i],
+        shifts[i], values[i] (k ints or a [k, 32] u8 array), proofs[i]).  powers_of_g: >= k G1 powers as an array
+        (its first k are uploaded for the call) or ResidentPoints; h, tau_k_h: 200-byte G2 records h and [tau^k] h
+        (fastkgz powers_of_h[0] and powers_of_h[k]).  One random linear combination of the items (127-bit
+        randomizers from the 32-byte seed, or from getrandom when None) and one pairing product decide: a false item
+        passes with probability at most 2^-127."""
+        ctx = ctx or default_context()
+        m, k = len(shifts), 1 << log2_k if 0 <= log2_k <= 20 else 0
+        if not isinstance(powers_of_g, ResidentPoints):
+            if k > len(powers_of_g):
+                raise PtauError(_ffi.ERR_ARG, detail="fewer powers than the coset size")
+            powers_of_g = ResidentPoints(ctx, np.asarray(powers_of_g)[:k])
+        c = np.ascontiguousarray(np.asarray(comms, dtype=np.uint8).reshape(m, 104))
+        w = np.ascontiguousarray(np.asarray(proofs, dtype=np.uint8).reshape(m, 104))
+        z = KZG10._scalars(shifts)
+        if isinstance(values, np.ndarray) and values.dtype == np.uint8:
+            v = np.ascontiguousarray(values).reshape(-1)
+        else:
+            v = KZG10._scalars([x for row in values for x in row])
+        if v.size != m * k * 32:
+            raise PtauError(_ffi.ERR_ARG, detail="expected k values per item")
+        g2 = np.ascontiguousarray(np.concatenate([np.asarray(h, dtype=np.uint8).reshape(-1),
+                                                  np.asarray(tau_k_h, dtype=np.uint8).reshape(-1)]))
+        if seed is not None and len(seed) != 32:
+            raise PtauError(_ffi.ERR_ARG, detail="seed must be 32 bytes")
+        ok = np.zeros(1, dtype=np.uint8)
+        rc = _ffi.lib().ptau_kzg_check_cosets(ctx._h, powers_of_g._h, _ptr(g2), _ptr(g2[200:]), log2_k,
+                                              _ptr(c) if m else None, _ptr(z) if m else None, _ptr(v) if m else None,
+                                              _ptr(w) if m else None, m, seed, _ptr(ok))
+        if rc != 0:
+            ctx._raise(rc)
+        return bool(ok[0])
 
     @staticmethod
     def _scalars(vals) -> np.ndarray:

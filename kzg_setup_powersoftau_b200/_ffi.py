@@ -133,6 +133,15 @@ _SIGNATURES = {
         [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t,
          C.c_void_p, C.c_void_p, C.c_void_p],
     ),
+    "ptau_kzg_open_cosets": (
+        C.c_int,
+        [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p],
+    ),
+    "ptau_kzg_check_cosets": (
+        C.c_int,
+        [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+         C.c_size_t, C.c_char_p, C.c_void_p],
+    ),
     "ptau_kzg_check": (C.c_int, [C.c_void_p] * 8 + [C.c_size_t, C.c_void_p]),
     "ptau_pairing_product2": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]),
     "ptau_g2_prepare": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]),

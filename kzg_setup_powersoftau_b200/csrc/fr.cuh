@@ -1,6 +1,6 @@
 // BLS12-381 scalar field Fr, 8 x u32 limbs: the Montgomery product (R = 2^256) of the synthetic generator
 // (kernels.cu) and what the KZG10 quotient scan (kzg_open.cu) adds to it: addition, the canonical check and 32-byte
-// little-endian load / store.
+// little-endian load / store; the coset openings (kzg_coset.cu) add subtraction and powers from a table of squares.
 //
 // Scalars in memory stay canonical (< r), not Montgomery: fr_mul(a, bR) = a b mod r, so a canonical value times a
 // constant kept in Montgomery form (z R mod r, prepared once on the host) is again canonical.
@@ -89,6 +89,41 @@ PTAU_FR_HD void fr_add(uint32_t* r, const uint32_t* a, const uint32_t* b) {
   const bool ge = bw == 0;
 #pragma unroll
   for (int i = 0; i < 8; i++) r[i] = ge ? d[i] : s[i];
+}
+
+// r = a - b mod r for canonical a, b (r may alias either)
+PTAU_FR_HD void fr_sub(uint32_t* r, const uint32_t* a, const uint32_t* b) {
+  uint32_t d[8], s[8];
+  uint32_t bw = 0;
+#pragma unroll
+  for (int i = 0; i < 8; i++) {
+    uint64_t x = (uint64_t)a[i] - b[i] - bw;
+    d[i] = (uint32_t)x;
+    bw = (uint32_t)(x >> 63);
+  }
+  // a < b: the difference wrapped by 2^256; adding r brings it back into [0, r)
+  uint64_t c = 0;
+#pragma unroll
+  for (int i = 0; i < 8; i++) {
+    c += (uint64_t)d[i] + K_FR_MOD[i];
+    s[i] = (uint32_t)c;
+    c >>= 32;
+  }
+#pragma unroll
+  for (int i = 0; i < 8; i++) r[i] = bw ? s[i] : d[i];
+}
+
+// R mod r: 1 in Montgomery form
+PTAU_FR_HD void fr_mont_one(uint32_t* a) {
+  a[0] = 0xfffffffeu, a[1] = 0x00000001u, a[2] = 0x00034802u, a[3] = 0x5884b7fau;
+  a[4] = 0xecbc4ff5u, a[5] = 0x998c4fefu, a[6] = 0xacc5056fu, a[7] = 0x1824b159u;
+}
+
+// out = prod of tbl[s] over the set bits s < bits of x, in Montgomery form (tbl[s] = w^(2^s) R gives w^x R)
+PTAU_FR_HD void fr_pow_bits(uint32_t* out, const uint32_t (*tbl)[8], uint64_t x, int bits) {
+  fr_mont_one(out);
+  for (int s = 0; s < bits; s++)
+    if ((x >> s) & 1) fr_mul(out, out, tbl[s]);
 }
 
 // a < r

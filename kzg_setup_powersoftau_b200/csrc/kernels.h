@@ -60,6 +60,29 @@ size_t kzg_quotient_sums_bytes(uint64_t n);
 cudaError_t launch_kzg_quotient(const void* d_coeffs, uint64_t n, const uint32_t (*zpow)[8], void* d_sums, void* d_q,
                                 void* d_value, uint32_t* d_bad, int* launches, cudaStream_t stream);
 
+// kzg_coset.cu, for k = 2^lg_k, lg_k <= kCosetLgKMax.
+// launch_coset_quotient: p = (X^k - c) q + r for n > 0 canonical scalars d_coeffs; q (n - k scalars when n > k) into d_q,
+// r (k scalars) into d_rem; cpow[s] = c^(2^s) R mod r for s < kKzgZPowCount; d_sums: coset_quotient_sums_bytes(n, lg_k)
+// of scratch; *d_bad is set to 1 when a coefficient is >= r.  n == 0: r = 0, no launch but a memset.
+constexpr int kCosetLgKMax = 20;
+constexpr uint32_t kCosetRhoDomain = 0x20;  // BLAKE2b domain byte of the coset check's randomizers (ratio_coeff)
+size_t coset_quotient_sums_bytes(uint64_t n, int lg_k);
+cudaError_t launch_coset_quotient(const void* d_coeffs, uint64_t n, int lg_k, const uint32_t (*cpow)[8], void* d_sums,
+                                  void* d_q, void* d_rem, uint32_t* d_bad, int* launches, cudaStream_t stream);
+// d_tw: k/2 twiddles w^i R for the NTT of size k, from wpow[s] = w^(2^s) R, s < lg_k
+cudaError_t launch_ntt_twiddles(void* d_tw, int lg_k, const uint32_t (*wpow)[8], cudaStream_t stream);
+// per item: d_out = NTT_k(in_j h^j) in natural order, over the twiddles d_tw (d_in != d_out); d_hpow: items x
+// kCosetLgKMax rows h^(2^s) R, or null (h = 1)
+cudaError_t launch_ntt(const void* d_in, void* d_out, uint64_t items, int lg_k, const void* d_hpow, const void* d_tw,
+                       int* launches, cudaStream_t stream);
+// the check's scalars of m items: srm[i] = rho_i k^-1 R, sc[i] = rho_i, sc[m + i] = rho_i c_i, neg[i] = -rho_i, where
+// rho_i = ratio_coeff(key, kCosetRhoDomain, i), d_cm[i] = c_i R and kinv_r2 = k^-1 R^2
+cudaError_t launch_coset_check_scalars(const uint64_t* key_h, uint64_t m, const void* d_cm, const uint32_t* kinv_r2,
+                                       void* d_srm, void* d_sc, void* d_neg, cudaStream_t stream);
+// d_out[j] = -sum_i d_x[i][j] h_i^-j rho_i k^-1 (d_hinv: m x kCosetLgKMax rows h_i^(-2^s) R, d_srm from above)
+cudaError_t launch_coset_interp_sum(const void* d_x, uint64_t m, int lg_k, const void* d_hinv, const void* d_srm,
+                                    void* d_out, cudaStream_t stream);
+
 // G2Prepared (ark-ec 0.2): n x 68 x 288 bytes of line coefficients + n infinity bytes
 cudaError_t launch_g2_prepare(const void* d_g2, uint64_t n, void* d_coeffs, void* d_infinity, cudaStream_t stream);
 

@@ -95,6 +95,15 @@ extern "C" {
         n: usize, blinding: *const c_void, n_b: usize, points: *const c_void, k: usize, proofs_out: *mut c_void,
         values_out: *mut c_void, random_v_out: *mut c_void,
     ) -> c_int;
+    pub fn ptau_kzg_open_cosets(
+        ctx: *mut ptau_ctx, powers: *const ptau_kzg_powers, coeffs: *const c_void, n: usize, log2_k: c_int,
+        shifts: *const c_void, m: usize, proofs_out: *mut c_void, values_out: *mut c_void,
+    ) -> c_int;
+    pub fn ptau_kzg_check_cosets(
+        ctx: *mut ptau_ctx, powers: *const ptau_kzg_powers, h: *const c_void, tau_k_h: *const c_void, log2_k: c_int,
+        comms: *const c_void, shifts: *const c_void, values: *const c_void, proofs: *const c_void, m: usize,
+        seed: *const u8, ok: *mut u8,
+    ) -> c_int;
     pub fn ptau_kzg_check(
         ctx: *mut ptau_ctx, vk_g1: *const c_void, vk_g2: *const c_void, comms: *const c_void, points: *const c_void,
         values: *const c_void, proofs_w: *const c_void, random_v: *const c_void, n: usize, ok: *mut u8,
