@@ -904,140 +904,7 @@ int ptau_kzg_quotient(const void* coeffs, size_t n, const void* point, void* quo
 }
 
 namespace {
-// the multipliers of the quotient scan for the point z: out[s] = z^(2^s) R mod r
-void kzg_zpow(const void* z, uint32_t (*out)[8]) {
-  Fr p = fr_to_mont(fr_from_le32((const uint8_t*)z));
-  for (int s = 0; s < ptau::kKzgZPowCount; s++) {
-    memcpy(out[s], p.l, 32);
-    p = fr_mont_mul(p, p);
-  }
-}
 size_t up256(size_t v) { return (v + 255) & ~(size_t)255; }
-}  // namespace
-
-// Per GPU, for its contiguous range of the points: the coefficients (and blinding coefficients) are uploaded once;
-// then, per point and on one stream with no host round trip, the quotient kernels write (p - p(z)) / (X - z) into the
-// MSM's scalar buffer and the bucket MSM runs over the resident powers.  With blinding the same follows for b over
-// gamma_powers, and a 2-term MSM with unit scalars adds the two results.  Values, proofs and the "coefficient >= r"
-// word come back once at the end.
-int ptau_kzg_open(ptau_ctx* ctx, const ptau_kzg_powers* powers, const ptau_kzg_powers* gamma_powers, const void* coeffs,
-                  size_t n, const void* blinding, size_t n_b, const void* points, size_t k, void* proofs_out,
-                  void* values_out, void* random_v_out) {
-  if (!ctx || !powers || powers->ctx != ctx || (gamma_powers && gamma_powers->ctx != ctx)) return PTAU_ERR_ARG;
-  if (n > powers->n || (n_b && (!gamma_powers || n_b > gamma_powers->n))) return PTAU_ERR_ARG;  // TooManyCoefficients
-  if ((n && !coeffs) || (n_b && !blinding)) return PTAU_ERR_ARG;
-  if (k && (!points || !proofs_out || !values_out || (n_b > 0) != (random_v_out != nullptr))) return PTAU_ERR_ARG;
-  if (!msm_fits(n) || !msm_fits(n_b)) return PTAU_ERR_ARG;
-  auto t0 = std::chrono::steady_clock::now();
-  timing_reset(ctx);
-  if (k == 0) return PTAU_OK;
-  if (!scalars_canonical(points, k)) return PTAU_ERR_ARG;
-  const int G = (size_t)ctx->n_gpus < k ? ctx->n_gpus : (int)k;
-  const size_t n_max = n > n_b ? n : n_b, nq = n > 1 ? n - 1 : 0, nbq = n_b > 1 ? n_b - 1 : 0;
-  size_t scratch = 0;
-  for (size_t m : {nq, nbq, (size_t)2}) {
-    ptau::MsmPlan plan;
-    ptau::msm_g1_plan(m, &plan);
-    scratch = plan.scratch_bytes > scratch ? plan.scratch_bytes : scratch;
-  }
-  // staging in GPU 0's pinned scalar buffer (portable: every GPU copies from it): coefficients | blinding | 1, 1
-  GpuSlot& s0 = ctx->gpu[0];
-  const size_t h_b = n * 32, h_one = h_b + n_b * 32, h_len = h_one + 64;
-  cudaError_t e = cudaSetDevice(s0.device);
-  if (e == cudaSuccess) e = grow(&s0.h_msm_sc, &s0.cap_h_msm_sc, h_len, true);
-  if (e != cudaSuccess) return cuda_fail(ctx, __func__, e);
-  uint8_t* stage = (uint8_t*)s0.h_msm_sc;
-  if (n) copy_parts(stage, coeffs, n * 32);
-  if (n_b) copy_parts(stage + h_b, blinding, n_b * 32);
-  memset(stage + h_one, 0, 64);
-  stage[h_one] = stage[h_one + 32] = 1;
-  // device layout of d_open, per GPU: coefficients | blinding | 1, 1 | chunk sums | MSM results r0, r1 | the pair
-  // (r0, r1) as consecutive records | "coefficient >= r" word | values | random values | proofs
-  const size_t d_b = up256(n * 32), d_one = d_b + up256(n_b * 32), d_sums = d_one + 256,
-               d_r0 = d_sums + up256(ptau::kzg_quotient_sums_bytes(n_max)), d_r1 = d_r0 + 256, d_pair = d_r1 + 256,
-               d_bad = d_pair + 256, d_val = d_bad + 256;
-  int launches = 0;
-  for (int g = 0; g < G && e == cudaSuccess; g++) {
-    GpuSlot& s = ctx->gpu[g];
-    const ptau::Shard sh = shard(k, g, G);
-    const size_t lo = sh.lo, cnt = sh.hi - sh.lo;
-    const size_t d_rv = d_val + up256(cnt * 32), d_pf = d_rv + up256(cnt * 32), d_len = d_pf + cnt * kMontG1;
-    cudaStream_t st = s.stream[0];
-    e = cudaSetDevice(s.device);
-    if (e == cudaSuccess) e = grow(&s.d_open, &s.cap_open, d_len);
-    if (e == cudaSuccess) e = grow(&s.d_msm_sc, &s.cap_msm_sc, n_max * 32 + 16);
-    if (e == cudaSuccess) e = grow(&s.d_msm_scratch, &s.cap_msm_scratch, scratch);
-    if (e == cudaSuccess && !s.h_msm_out) e = cudaHostAlloc((void**)&s.h_msm_out, 256, cudaHostAllocPortable);
-    if (e != cudaSuccess) break;
-    uint8_t* d = (uint8_t*)s.d_open;
-    uint32_t* bad = (uint32_t*)(d + d_bad);
-    e = cudaEventRecord(s.ev_first, st);
-    if (e == cudaSuccess && n) e = cudaMemcpyAsync(d, stage, n * 32, cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess && n_b) e = cudaMemcpyAsync(d + d_b, stage + h_b, n_b * 32, cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d + d_one, stage + h_one, 64, cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess) e = cudaMemsetAsync(bad, 0, 4, st);
-    if (e == cudaSuccess) e = cudaEventRecord(s.ev_k0[0], st);
-    for (size_t j = 0; j < cnt && e == cudaSuccess; j++) {
-      uint32_t zp[ptau::kKzgZPowCount][8];
-      kzg_zpow((const uint8_t*)points + (lo + j) * 32, zp);
-      int nl = 0;
-      e = ptau::launch_kzg_quotient(d, n, zp, d + d_sums, s.d_msm_sc, d + d_val + j * 32, bad, &nl, st);
-      launches += nl;
-      if (e == cudaSuccess) e = ptau::launch_msm_g1(powers->d_pts[g], s.d_msm_sc, nq, s.d_msm_scratch, d + d_r0, &nl, st);
-      launches += nl;
-      if (n_b) {
-        if (e == cudaSuccess)
-          e = ptau::launch_kzg_quotient(d + d_b, n_b, zp, d + d_sums, s.d_msm_sc, d + d_rv + j * 32, bad, &nl, st);
-        launches += nl;
-        if (e == cudaSuccess)
-          e = ptau::launch_msm_g1(gamma_powers->d_pts[g], s.d_msm_sc, nbq, s.d_msm_scratch, d + d_r1, &nl, st);
-        launches += nl;
-        if (e == cudaSuccess) e = cudaMemcpyAsync(d + d_pair, d + d_r0, kMontG1, cudaMemcpyDeviceToDevice, st);
-        if (e == cudaSuccess)
-          e = cudaMemcpyAsync(d + d_pair + kMontG1, d + d_r1, kMontG1, cudaMemcpyDeviceToDevice, st);
-        if (e == cudaSuccess) e = ptau::launch_msm_g1(d + d_pair, d + d_one, 2, s.d_msm_scratch, d + d_r0, &nl, st);
-        launches += nl;
-      }
-      if (e == cudaSuccess)
-        e = cudaMemcpyAsync(d + d_pf + j * kMontG1, d + d_r0, kMontG1, cudaMemcpyDeviceToDevice, st);
-    }
-    if (e == cudaSuccess) e = cudaEventRecord(s.ev_k1[0], st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(s.h_msm_out, bad, 4, cudaMemcpyDeviceToHost, st);
-    ctx->timing.h2d_bytes[g] = (n + n_b) * 32 + 64;
-    ctx->timing.d2h_bytes[g] = cnt * (kMontG1 + 32 + (n_b ? 32 : 0)) + 4;
-  }
-  ctx->timing.kernel_launches = launches;
-  // results to the caller's (pageable) memory only once every GPU has its work queued
-  bool bad_coeff = false;
-  for (int g = 0; g < G && e == cudaSuccess; g++) {
-    GpuSlot& s = ctx->gpu[g];
-    const ptau::Shard sh = shard(k, g, G);
-    const size_t lo = sh.lo, cnt = sh.hi - sh.lo;
-    const size_t d_rv = d_val + up256(cnt * 32), d_pf = d_rv + up256(cnt * 32);
-    const uint8_t* d = (const uint8_t*)s.d_open;
-    cudaStream_t st = s.stream[0];
-    e = cudaSetDevice(s.device);
-    if (e == cudaSuccess)
-      e = cudaMemcpyAsync((uint8_t*)proofs_out + lo * kMontG1, d + d_pf, cnt * kMontG1, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess)
-      e = cudaMemcpyAsync((uint8_t*)values_out + lo * 32, d + d_val, cnt * 32, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess && n_b)
-      e = cudaMemcpyAsync((uint8_t*)random_v_out + lo * 32, d + d_rv, cnt * 32, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaEventRecord(s.ev_last, st);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    float kms = 0, gms = 0;
-    if (e == cudaSuccess) e = cudaEventElapsedTime(&kms, s.ev_k0[0], s.ev_k1[0]);
-    if (e == cudaSuccess) e = cudaEventElapsedTime(&gms, s.ev_first, s.ev_last);
-    ctx->timing.kernel_ms[g] = kms;
-    ctx->timing.gpu_ms[g] = gms;
-    bad_coeff = bad_coeff || s.h_msm_out[0] != 0;
-  }
-  if (e != cudaSuccess) return drain_fail(ctx, G, __func__, e);
-  ctx->timing.wall_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-  return bad_coeff ? PTAU_ERR_ARG : PTAU_OK;
-}
-
-namespace {
 // omega_{2^32} = 7^((r - 1) / 2^32) mod r (ark-bls12-381 Fr TWO_ADIC_ROOT_OF_UNITY), canonical limbs
 constexpr uint64_t kFrRootOfUnity[4] = {0x3829971f439f0d2bull, 0xb63683508c2280b9ull, 0xd09b681922c813b4ull,
                                         0x16a2a19edfe81f20ull};
@@ -1078,107 +945,145 @@ bool shifts_valid(const void* p, size_t m) {
   }
   return true;
 }
-}  // namespace
 
-// Per GPU, for its contiguous range of the cosets: the coefficients and the cosets' tables h^(2^s) R are uploaded once;
-// then, per coset and on one stream with no host round trip, the strided quotient kernels write q = p div (X^k - h^k)
-// into the MSM's scalar buffer and r into the remainder buffer, and the bucket MSM commits to q over the resident
-// powers.  One batched NTT of all the GPU's remainders (scaled by h^j) gives the values; values, proofs and the
-// "coefficient >= r" word come back once at the end.
-int ptau_kzg_open_cosets(ptau_ctx* ctx, const ptau_kzg_powers* powers, const void* coeffs, size_t n, int log2_k,
-                         const void* shifts, size_t m, void* proofs_out, void* values_out) {
-  if (!ctx || !powers || powers->ctx != ctx || log2_k < 0 || log2_k > ptau::kCosetLgKMax) return PTAU_ERR_ARG;
-  if (n > powers->n || (n && !coeffs) || (m && (!shifts || !proofs_out || !values_out))) return PTAU_ERR_ARG;
-  const uint64_t k = 1ull << log2_k;
-  const size_t nq = n > k ? n - k : 0;
-  if (!msm_fits(nq)) return PTAU_ERR_ARG;
+// Both openings, per GPU for its contiguous range of the shifts h (the points of ptau_kzg_open, the cosets' shifts of
+// ptau_kzg_open_cosets): the coefficients, the blinding coefficients and, for k > 1, the shifts' tables h^(2^s) R are
+// uploaded once; then, per shift and on one stream with no host round trip, the quotient kernels write
+// q = p div (X^k - h^k) into the MSM's scalar buffer and the remainder r into its slot, and the bucket MSM commits to q
+// over the resident powers.  With blinding (only at k = 1) the same follows for b over gamma_powers, and a 2-term MSM
+// with unit scalars adds the two results.  For k > 1 one batched NTT of all the GPU's remainders (scaled by h^j) gives
+// the values; for k = 1 the remainder is the value p(h) and is written straight into the values.  Values, proofs and
+// the "coefficient >= r" word come back once at the end.  `where` names the entry point in the last-error text.
+int kzg_open_impl(ptau_ctx* ctx, const char* where, const ptau_kzg_powers* powers, const ptau_kzg_powers* gamma_powers,
+                  const void* coeffs, size_t n, const void* blinding, size_t n_b, int log2_k, const void* shifts, size_t m,
+                  void* proofs_out, void* values_out, void* random_v_out) {
   auto t0 = std::chrono::steady_clock::now();
-  timing_reset(ctx);
-  if (m == 0) return PTAU_OK;
-  if (!shifts_valid(shifts, m)) return PTAU_ERR_ARG;
+  const uint64_t k = 1ull << log2_k;
   const int G = (size_t)ctx->n_gpus < m ? ctx->n_gpus : (int)m;
-  ptau::MsmPlan plan;
-  ptau::msm_g1_plan(nq, &plan);
-  // host tables: c = h^k as the scan's multipliers (per coset, built while queueing), h^(2^s) R for the NTT's scale
+  const size_t n_max = n > n_b ? n : n_b, nq = n > k ? n - k : 0, nbq = n_b > k ? n_b - k : 0;
+  size_t scratch = 0;
+  for (size_t len : {nq, nbq, n_b ? (size_t)2 : 0}) {
+    ptau::MsmPlan plan;
+    ptau::msm_g1_plan(len, &plan);
+    scratch = plan.scratch_bytes > scratch ? plan.scratch_bytes : scratch;
+  }
+  // staging in GPU 0's pinned scalar buffer (portable: every GPU copies from it): coefficients | blinding | 1, 1 |
+  // per shift, h^(2^s) R for the NTT's coset scale (k > 1)
   constexpr int kTbl = ptau::kCosetLgKMax;
+  const size_t tbl = log2_k ? kTbl * 32 : 0;
   GpuSlot& s0 = ctx->gpu[0];
-  const size_t h_tbl = n * 32, h_len = h_tbl + m * kTbl * 32;
+  const size_t h_b = n * 32, h_one = h_b + n_b * 32, h_tbl = h_one + 64, h_len = h_tbl + m * tbl;
   cudaError_t e = cudaSetDevice(s0.device);
   if (e == cudaSuccess) e = grow(&s0.h_msm_sc, &s0.cap_h_msm_sc, h_len, true);
-  if (e != cudaSuccess) return cuda_fail(ctx, __func__, e);
+  if (e != cudaSuccess) return cuda_fail(ctx, where, e);
   uint8_t* stage = (uint8_t*)s0.h_msm_sc;
   if (n) copy_parts(stage, coeffs, n * 32);
+  if (n_b) copy_parts(stage + h_b, blinding, n_b * 32);
+  memset(stage + h_one, 0, 64);
+  stage[h_one] = stage[h_one + 32] = 1;
   std::vector<Fr> hm(m);
   for (size_t i = 0; i < m; i++) {
     hm[i] = fr_to_mont(fr_from_le32((const uint8_t*)shifts + i * 32));
-    fr_square_table(hm[i], (uint32_t(*)[8])(stage + h_tbl + i * kTbl * 32), kTbl);
+    if (log2_k) fr_square_table(hm[i], (uint32_t(*)[8])(stage + h_tbl + i * tbl), kTbl);
   }
   uint32_t wpow[ptau::kCosetLgKMax][8];
   fr_square_table(fr_root_mont(log2_k), wpow, log2_k);
-  // device layout of d_open, per GPU: coefficients | chunk sums | MSM result | "coefficient >= r" word | twiddles |
-  // h tables | remainders | values | proofs
-  const size_t d_sums = up256(n * 32), d_r0 = d_sums + up256(ptau::coset_quotient_sums_bytes(n, log2_k)),
-               d_bad = d_r0 + 256, d_tw = d_bad + 256, d_ht = d_tw + up256(k / 2 * 32);
+  // device layout of d_open, per GPU: coefficients | blinding | 1, 1 | chunk sums | MSM results r0, r1 | the pair
+  // (r0, r1) as consecutive records | "coefficient >= r" word | twiddles | h tables | remainders | values | random
+  // values | proofs.  For k = 1 the remainders take no space: they are the values.
+  const size_t d_b = up256(n * 32), d_one = d_b + up256(n_b * 32), d_sums = d_one + 256,
+               d_r0 = d_sums + up256(ptau::coset_quotient_sums_bytes(n_max, log2_k)), d_r1 = d_r0 + 256,
+               d_pair = d_r1 + 256, d_bad = d_pair + 256, d_tw = d_bad + 256, d_ht = d_tw + up256(k / 2 * 32);
+  struct Tail {
+    size_t rem, val, rv, pf, len;
+  };
+  auto tail = [&](size_t cnt) {
+    Tail t;
+    t.rem = d_ht + up256(cnt * tbl);
+    t.val = t.rem + (log2_k ? up256(cnt * k * 32) : 0);
+    t.rv = t.val + up256(cnt * k * 32);
+    t.pf = t.rv + up256(n_b ? cnt * 32 : 0);
+    t.len = t.pf + cnt * kMontG1;
+    return t;
+  };
   int launches = 0;
   for (int g = 0; g < G && e == cudaSuccess; g++) {
     GpuSlot& s = ctx->gpu[g];
     const ptau::Shard sh = shard(m, g, G);
     const size_t lo = sh.lo, cnt = sh.hi - sh.lo;
-    const size_t d_rem = d_ht + up256(cnt * kTbl * 32), d_val = d_rem + up256(cnt * k * 32),
-                 d_pf = d_val + up256(cnt * k * 32), d_len = d_pf + cnt * kMontG1;
+    const Tail t = tail(cnt);
     cudaStream_t st = s.stream[0];
     e = cudaSetDevice(s.device);
-    if (e == cudaSuccess) e = grow(&s.d_open, &s.cap_open, d_len);
-    if (e == cudaSuccess) e = grow(&s.d_msm_sc, &s.cap_msm_sc, nq * 32 + 16);
-    if (e == cudaSuccess) e = grow(&s.d_msm_scratch, &s.cap_msm_scratch, plan.scratch_bytes);
+    if (e == cudaSuccess) e = grow(&s.d_open, &s.cap_open, t.len);
+    if (e == cudaSuccess) e = grow(&s.d_msm_sc, &s.cap_msm_sc, n_max * 32 + 16);
+    if (e == cudaSuccess) e = grow(&s.d_msm_scratch, &s.cap_msm_scratch, scratch);
     if (e == cudaSuccess && !s.h_msm_out) e = cudaHostAlloc((void**)&s.h_msm_out, 256, cudaHostAllocPortable);
     if (e != cudaSuccess) break;
     uint8_t* d = (uint8_t*)s.d_open;
     uint32_t* bad = (uint32_t*)(d + d_bad);
     e = cudaEventRecord(s.ev_first, st);
     if (e == cudaSuccess && n) e = cudaMemcpyAsync(d, stage, n * 32, cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess)
-      e = cudaMemcpyAsync(d + d_ht, stage + h_tbl + lo * kTbl * 32, cnt * kTbl * 32, cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess && n_b) e = cudaMemcpyAsync(d + d_b, stage + h_b, n_b * 32, cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess && n_b) e = cudaMemcpyAsync(d + d_one, stage + h_one, 64, cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess && log2_k)
+      e = cudaMemcpyAsync(d + d_ht, stage + h_tbl + lo * tbl, cnt * tbl, cudaMemcpyHostToDevice, st);
     if (e == cudaSuccess) e = cudaMemsetAsync(bad, 0, 4, st);
     if (e == cudaSuccess) e = cudaEventRecord(s.ev_k0[0], st);
     if (e == cudaSuccess) e = ptau::launch_ntt_twiddles(d + d_tw, log2_k, wpow, st);
     launches += log2_k > 0;
     for (size_t j = 0; j < cnt && e == cudaSuccess; j++) {
       Fr c = hm[lo + j];  // c R = h^k R
-      for (int t = 0; t < log2_k; t++) c = fr_mont_mul(c, c);
+      for (int i = 0; i < log2_k; i++) c = fr_mont_mul(c, c);
       uint32_t cp[ptau::kKzgZPowCount][8];
       fr_square_table(c, cp, ptau::kKzgZPowCount);
       int nl = 0;
-      e = ptau::launch_coset_quotient(d, n, log2_k, cp, d + d_sums, s.d_msm_sc, d + d_rem + j * k * 32, bad, &nl, st);
+      e = ptau::launch_coset_quotient(d, n, log2_k, cp, d + d_sums, s.d_msm_sc, d + t.rem + j * k * 32, bad, &nl, st);
       launches += nl;
       if (e == cudaSuccess) e = ptau::launch_msm_g1(powers->d_pts[g], s.d_msm_sc, nq, s.d_msm_scratch, d + d_r0, &nl, st);
       launches += nl;
+      if (n_b) {
+        if (e == cudaSuccess)
+          e = ptau::launch_coset_quotient(d + d_b, n_b, 0, cp, d + d_sums, s.d_msm_sc, d + t.rv + j * 32, bad, &nl, st);
+        launches += nl;
+        if (e == cudaSuccess)
+          e = ptau::launch_msm_g1(gamma_powers->d_pts[g], s.d_msm_sc, nbq, s.d_msm_scratch, d + d_r1, &nl, st);
+        launches += nl;
+        if (e == cudaSuccess) e = cudaMemcpyAsync(d + d_pair, d + d_r0, kMontG1, cudaMemcpyDeviceToDevice, st);
+        if (e == cudaSuccess)
+          e = cudaMemcpyAsync(d + d_pair + kMontG1, d + d_r1, kMontG1, cudaMemcpyDeviceToDevice, st);
+        if (e == cudaSuccess) e = ptau::launch_msm_g1(d + d_pair, d + d_one, 2, s.d_msm_scratch, d + d_r0, &nl, st);
+        launches += nl;
+      }
       if (e == cudaSuccess)
-        e = cudaMemcpyAsync(d + d_pf + j * kMontG1, d + d_r0, kMontG1, cudaMemcpyDeviceToDevice, st);
+        e = cudaMemcpyAsync(d + t.pf + j * kMontG1, d + d_r0, kMontG1, cudaMemcpyDeviceToDevice, st);
     }
-    int nl = 0;
-    if (e == cudaSuccess) e = ptau::launch_ntt(d + d_rem, d + d_val, cnt, log2_k, d + d_ht, d + d_tw, &nl, st);
-    launches += nl;
+    if (log2_k) {
+      int nl = 0;
+      if (e == cudaSuccess) e = ptau::launch_ntt(d + t.rem, d + t.val, cnt, log2_k, d + d_ht, d + d_tw, &nl, st);
+      launches += nl;
+    }
     if (e == cudaSuccess) e = cudaEventRecord(s.ev_k1[0], st);
     if (e == cudaSuccess) e = cudaMemcpyAsync(s.h_msm_out, bad, 4, cudaMemcpyDeviceToHost, st);
-    ctx->timing.h2d_bytes[g] = n * 32 + cnt * kTbl * 32;
-    ctx->timing.d2h_bytes[g] = cnt * (kMontG1 + k * 32) + 4;
+    ctx->timing.h2d_bytes[g] = (n + n_b) * 32 + (n_b ? 64 : 0) + cnt * tbl;
+    ctx->timing.d2h_bytes[g] = cnt * (kMontG1 + k * 32 + (n_b ? 32 : 0)) + 4;
   }
   ctx->timing.kernel_launches = launches;
+  // results to the caller's (pageable) memory only once every GPU has its work queued
   bool bad_coeff = false;
   for (int g = 0; g < G && e == cudaSuccess; g++) {
     GpuSlot& s = ctx->gpu[g];
     const ptau::Shard sh = shard(m, g, G);
     const size_t lo = sh.lo, cnt = sh.hi - sh.lo;
-    const size_t d_rem = d_ht + up256(cnt * kTbl * 32), d_val = d_rem + up256(cnt * k * 32),
-                 d_pf = d_val + up256(cnt * k * 32);
+    const Tail t = tail(cnt);
     const uint8_t* d = (const uint8_t*)s.d_open;
     cudaStream_t st = s.stream[0];
     e = cudaSetDevice(s.device);
     if (e == cudaSuccess)
-      e = cudaMemcpyAsync((uint8_t*)proofs_out + lo * kMontG1, d + d_pf, cnt * kMontG1, cudaMemcpyDeviceToHost, st);
+      e = cudaMemcpyAsync((uint8_t*)proofs_out + lo * kMontG1, d + t.pf, cnt * kMontG1, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess)
-      e = cudaMemcpyAsync((uint8_t*)values_out + lo * k * 32, d + d_val, cnt * k * 32, cudaMemcpyDeviceToHost, st);
+      e = cudaMemcpyAsync((uint8_t*)values_out + lo * k * 32, d + t.val, cnt * k * 32, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess && n_b)
+      e = cudaMemcpyAsync((uint8_t*)random_v_out + lo * 32, d + t.rv, cnt * 32, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaEventRecord(s.ev_last, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
     float kms = 0, gms = 0;
@@ -1188,9 +1093,40 @@ int ptau_kzg_open_cosets(ptau_ctx* ctx, const ptau_kzg_powers* powers, const voi
     ctx->timing.gpu_ms[g] = gms;
     bad_coeff = bad_coeff || s.h_msm_out[0] != 0;
   }
-  if (e != cudaSuccess) return drain_fail(ctx, G, __func__, e);
+  if (e != cudaSuccess) return drain_fail(ctx, G, where, e);
   ctx->timing.wall_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
   return bad_coeff ? PTAU_ERR_ARG : PTAU_OK;
+}
+}  // namespace
+
+// KZG10::open of p at k points: the division by X - z of kzg_open_impl at log2_k = 0, optionally hiding.
+int ptau_kzg_open(ptau_ctx* ctx, const ptau_kzg_powers* powers, const ptau_kzg_powers* gamma_powers, const void* coeffs,
+                  size_t n, const void* blinding, size_t n_b, const void* points, size_t k, void* proofs_out,
+                  void* values_out, void* random_v_out) {
+  if (!ctx || !powers || powers->ctx != ctx || (gamma_powers && gamma_powers->ctx != ctx)) return PTAU_ERR_ARG;
+  if (n > powers->n || (n_b && (!gamma_powers || n_b > gamma_powers->n))) return PTAU_ERR_ARG;  // TooManyCoefficients
+  if ((n && !coeffs) || (n_b && !blinding)) return PTAU_ERR_ARG;
+  if (k && (!points || !proofs_out || !values_out || (n_b > 0) != (random_v_out != nullptr))) return PTAU_ERR_ARG;
+  if (!msm_fits(n) || !msm_fits(n_b)) return PTAU_ERR_ARG;
+  timing_reset(ctx);
+  if (k == 0) return PTAU_OK;
+  if (!scalars_canonical(points, k)) return PTAU_ERR_ARG;
+  return kzg_open_impl(ctx, __func__, powers, gamma_powers, coeffs, n, blinding, n_b, 0, points, k, proofs_out,
+                       values_out, random_v_out);
+}
+
+// KZG10 openings of p on m cosets h <omega_k>: kzg_open_impl over the shifts, without hiding.
+int ptau_kzg_open_cosets(ptau_ctx* ctx, const ptau_kzg_powers* powers, const void* coeffs, size_t n, int log2_k,
+                         const void* shifts, size_t m, void* proofs_out, void* values_out) {
+  if (!ctx || !powers || powers->ctx != ctx || log2_k < 0 || log2_k > ptau::kCosetLgKMax) return PTAU_ERR_ARG;
+  if (n > powers->n || (n && !coeffs) || (m && (!shifts || !proofs_out || !values_out))) return PTAU_ERR_ARG;
+  const uint64_t k = 1ull << log2_k;
+  if (!msm_fits(n > k ? n - k : 0)) return PTAU_ERR_ARG;
+  timing_reset(ctx);
+  if (m == 0) return PTAU_OK;
+  if (!shifts_valid(shifts, m)) return PTAU_ERR_ARG;
+  return kzg_open_impl(ctx, __func__, powers, nullptr, coeffs, n, nullptr, 0, log2_k, shifts, m, proofs_out, values_out,
+                       nullptr);
 }
 
 // GPU 0, one stream, no host round trip: the inverse NTT of every item's values, the randomizers and scalars, the

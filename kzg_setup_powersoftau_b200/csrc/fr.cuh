@@ -1,11 +1,11 @@
 // BLS12-381 scalar field Fr, 8 x u32 limbs: the Montgomery product (R = 2^256) of the synthetic generator
-// (kernels.cu) and what the KZG10 quotient scan (kzg_open.cu) adds to it: addition, the canonical check and 32-byte
-// little-endian load / store; the coset openings (kzg_coset.cu) add subtraction and powers from a table of squares.
+// (kernels.cu) and what the KZG10 openings (kzg_coset.cu) add to it: addition, subtraction, the canonical check,
+// 32-byte little-endian load / store and powers from a table of squares.
 //
 // Scalars in memory stay canonical (< r), not Montgomery: fr_mul(a, bR) = a b mod r, so a canonical value times a
-// constant kept in Montgomery form (z R mod r, prepared once on the host) is again canonical.
+// constant kept in Montgomery form (c R mod r, prepared once on the host) is again canonical.
 //
-// Compiled for the host too (tests/host_emul/hostemul_open.cpp), with K_FR_MOD as an ordinary array.
+// Compiled for the host too (tests/host_emul/hostemul_coset.cpp), with K_FR_MOD as an ordinary array.
 #pragma once
 #include <stdint.h>
 

@@ -52,19 +52,13 @@ cudaError_t launch_kzg_check(const void* d_vk_g1, const void* d_vk_g2, const voi
                              const void* d_values, const void* d_proofs, const void* d_random_v, const void* d_tbl,
                              uint64_t n, void* d_ok, cudaStream_t stream);
 
-// kzg_open.cu: the witness polynomial (p - p(z)) / (X - z) of n > 0 canonical 32-byte scalars d_coeffs into d_q (n - 1
-// scalars, the layout launch_msm_g1 reads) and p(z) into d_value; zpow[s] = z^(2^s) R mod r for s < kKzgZPowCount; d_sums:
-// kzg_quotient_sums_bytes(n) of scratch; *d_bad is set to 1 when a coefficient is >= r.  n == 0: p(z) = 0, no launch.
-constexpr int kKzgZPowCount = 32;
-size_t kzg_quotient_sums_bytes(uint64_t n);
-cudaError_t launch_kzg_quotient(const void* d_coeffs, uint64_t n, const uint32_t (*zpow)[8], void* d_sums, void* d_q,
-                                void* d_value, uint32_t* d_bad, int* launches, cudaStream_t stream);
-
 // kzg_coset.cu, for k = 2^lg_k, lg_k <= kCosetLgKMax.
 // launch_coset_quotient: p = (X^k - c) q + r for n > 0 canonical scalars d_coeffs; q (n - k scalars when n > k) into d_q,
 // r (k scalars) into d_rem; cpow[s] = c^(2^s) R mod r for s < kKzgZPowCount; d_sums: coset_quotient_sums_bytes(n, lg_k)
-// of scratch; *d_bad is set to 1 when a coefficient is >= r.  n == 0: r = 0, no launch but a memset.
+// of scratch; *d_bad is set to 1 when a coefficient is >= r.  n == 0: r = 0, no launch but a memset.  At lg_k = 0 it is
+// the point opening's witness polynomial: c = z, q = (p - p(z)) / (X - z) and r = p(z).
 constexpr int kCosetLgKMax = 20;
+constexpr int kKzgZPowCount = 32;
 constexpr uint32_t kCosetRhoDomain = 0x20;  // BLAKE2b domain byte of the coset check's randomizers (ratio_coeff)
 size_t coset_quotient_sums_bytes(uint64_t n, int lg_k);
 cudaError_t launch_coset_quotient(const void* d_coeffs, uint64_t n, int lg_k, const uint32_t (*cpow)[8], void* d_sums,

@@ -32,7 +32,7 @@ __global__ void __launch_bounds__(PTAU_COSET_BLOCK) coset_quotient_chunk_sums(co
 }
 
 // chunk sums -> the carry entering each chunk, in place; each chain is scanned by a segment of 2^lg_seg threads of
-// a block of min(1024, k 2^lg_seg) threads (the Hillis-Steele steps of kzg_quotient_carries, within the segment)
+// a block of min(1024, k 2^lg_seg) threads (at k = 1: one block, one segment)
 __global__ void __launch_bounds__(1 << kKzgLgCarryThreads) coset_quotient_carries(uint32_t* __restrict__ sums, uint64_t mc,
                                                                                   int lg_seg, int lg_run, KzgZPow cp) {
   constexpr int T = 1 << kKzgLgCarryThreads;

@@ -1,23 +1,74 @@
 // Per-item code of the coset openings (kzg_coset.cu): division by X^k - c for k = 2^lg_k and the radix-2 NTT over Fr.
 //
 // Division.  p = (X^k - c) q + r, deg r < k.  For each residue j < k the chain p_j, p_{j+k}, p_{j+2k}, ... is folded
-// from the top, acc <- p_{j+tk} + c acc: the acc after row t >= 1 is q_{j+(t-1)k}, the final acc is r_j.  Every chain
-// is the recurrence of kzg_open.cuh with the multiplier c, so it runs as the same exact blocked scan, chain by chain:
+// from the top, acc <- p_{j+tk} + c acc: the acc after row t >= 1 is q_{j+(t-1)k}, the final acc is r_j.  The fold is a
+// first-order linear recurrence, so each chain runs as an exact blocked scan:
 //   1. chunk b of chain j = rows [bL, bL + L) has the local sum S_{j,b} (Horner from the top, carry 0);
-//   2. the carry entering chunk b is K_{j,b+1}, K_{j,b} = S_{j,b} + c^L K_{j,b+1}: the carry items of kzg_open.cuh over
-//      chain j's mc chunk sums, 2^lg_seg threads per chain (one segment of the carry block);
-//   3. chunk b re-runs Horner from its carry and writes q straight into the MSM's scalar buffer, and r_j at b = 0.
-// Chunk sums are stored chain after chain (sums[j mc + b]) so each chain's are contiguous.  Item id = b k + j: adjacent
-// threads read adjacent coefficients.  With k = 1 this is the scan of kzg_open.cuh with z = c.
+//   2. the carry entering chunk b from above is K_{j,b+1}, where K_{j,b} = S_{j,b} + c^L K_{j,b+1} (0 above the top
+//      chunk): the same recurrence over chain j's mc chunk sums with the constant multiplier c^L.  A segment of
+//      2^lg_seg threads of the carry block scans it: each thread folds a run of 2^lg_run sums, the segment combines
+//      the runs (Hillis-Steele, multipliers c^(L 2^lg_run 2^s)), and each thread re-runs its sums from its incoming
+//      carry, leaving K_{j,b+1} in place of S_{j,b};
+//   3. chunk b re-runs Horner from K_{j,b+1} and writes q straight into the MSM's scalar buffer, and r_j at b = 0.
+// Only the top chunk (and the top run) of a chain may be short; their incoming carry is 0, so their length never enters
+// a multiplier.  Every step is exact arithmetic in Fr: the result does not depend on L, the run length or the grid.
+// Scalars stay canonical; the multipliers are c^(2^s) R (Montgomery form, fr.cuh).  Chunk sums are stored chain after
+// chain (sums[j mc + b]) so each chain's are contiguous.  Item id = b k + j: adjacent threads read adjacent
+// coefficients.  ptau_kzg_open is the case k = 1, c = z: one chain, q the witness polynomial and r_0 = p(z).
 //
 // NTT.  x natural order in and out: a bit-reversing copy (with the coset scale h^j fused in) and lg_k in-place
 // Cooley-Tukey butterfly stages whose twiddles are tw[i] = w^i R for i < k/2.
 //
 // Shared with the host build (tests/host_emul/hostemul_coset.cpp), which runs the same items serially.
 #pragma once
-#include "kzg_open.cuh"
+#include "fr.cuh"
 
 namespace ptau {
+
+constexpr int kKzgZPow = 32;          // c^(2^s) for s < 32: lg L + lg_run + 9 <= 30 for any n < 2^31
+constexpr int kKzgLgChunk = 5;        // L = 32 rows per thread
+constexpr int kKzgLgCarryThreads = 10;  // the carry block has at most 1024 threads
+
+// the multipliers of one division: w[s] = c^(2^s) R mod r
+struct KzgZPow {
+  uint32_t w[kKzgZPow][8];
+};
+
+// The carry items take their multiplier (zl = c^L R, mul) as 8 words: the kernels pass a local copy of the one entry
+// of KzgZPow they need rather than the whole table.
+
+// step 2a: thread t's fold of the sums [t 2^lg_run, (t + 1) 2^lg_run) with the multiplier c^L
+PTAU_FR_HD void kzg_run_sum_item(const uint32_t* sums, uint64_t m, int lg_run, const uint32_t* zl, uint64_t t, uint32_t* acc) {
+  const uint64_t lo = t << lg_run, hi = lo + (1ull << lg_run) < m ? lo + (1ull << lg_run) : m;
+  for (int w = 0; w < 8; w++) acc[w] = 0;
+  for (uint64_t j = hi; j-- > lo;) {
+    uint32_t s[8], u[8];
+    fr_load(s, sums + j * 8);
+    fr_mul(u, acc, zl);
+    fr_add(acc, s, u);
+  }
+}
+
+// step 2b: one Hillis-Steele step at distance 2^s: y_t + mul y_{t + 2^s}, mul = c^(L 2^lg_run 2^s) R
+PTAU_FR_HD void kzg_combine_item(const uint32_t* y_t, const uint32_t* y_up, const uint32_t* mul, uint32_t* out) {
+  uint32_t u[8];
+  fr_mul(u, y_up, mul);
+  fr_add(out, y_t, u);
+}
+
+// step 2c: thread t re-runs its sums from its incoming carry cin and leaves the carry entering each chunk in place
+PTAU_FR_HD void kzg_run_carry_item(uint32_t* sums, uint64_t m, int lg_run, const uint32_t* zl, uint64_t t, const uint32_t* cin) {
+  const uint64_t lo = t << lg_run, hi = lo + (1ull << lg_run) < m ? lo + (1ull << lg_run) : m;
+  uint32_t acc[8];
+  for (int w = 0; w < 8; w++) acc[w] = cin[w];
+  for (uint64_t j = hi; j-- > lo;) {
+    uint32_t s[8], u[8];
+    fr_load(s, sums + j * 8);
+    fr_store(sums + j * 8, acc);
+    fr_mul(u, acc, zl);
+    fr_add(acc, s, u);
+  }
+}
 
 constexpr int kCosetMaxLgK = 20;  // k <= 2^20: powers_of_h[k] stays inside a 2^21 setup
 

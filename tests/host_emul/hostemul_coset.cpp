@@ -20,12 +20,16 @@ static void square_table(const uint32_t* a, uint32_t (*t)[8], int count) {
   for (int s = 1; s < count; s++) fr_mul(t[s], t[s - 1], t[s - 1]);
 }
 
-// op 0: fr_sub(a, b); 1: fr_mont_one(); 2: a^x by fr_pow_bits (x = the low 64 bits of b, 64 table rows), canonical
+// op 0: fr_sub(a, b); 1: fr_mont_one(); 2: a^x by fr_pow_bits (x = the low 64 bits of b, 64 table rows), canonical;
+// 3: fr_mul(a, b); 4: fr_add(a, b); 5: fr_is_canonical(a) in out[0]
 extern "C" void hostemul_coset_fr_op(int op, const uint8_t* a8, const uint8_t* b8, uint8_t* out8) {
   uint32_t a[8], b[8], r[8] = {0, 0, 0, 0, 0, 0, 0, 0};
   std::memcpy(a, a8, 32);
   std::memcpy(b, b8, 32);
   if (op == 0) fr_sub(r, a, b);
+  if (op == 3) fr_mul(r, a, b);
+  if (op == 4) fr_add(r, a, b);
+  if (op == 5) r[0] = fr_is_canonical(a) ? 1 : 0;
   if (op == 1) fr_mont_one(r);
   if (op == 2) {
     uint32_t t[64][8], w[8];

@@ -79,8 +79,8 @@ def test_root_of_unity():
 
 
 def test_fr_sub_and_powers_on_edge_limbs(he):
-    """fr_sub, fr_mont_one and fr_pow_bits of csrc/fr.cuh against Python integers (the edges of
-    test_fr_ops_on_edge_limbs)."""
+    """fr_mul (a b R^-1), fr_add, fr_sub, fr_is_canonical, fr_mont_one and fr_pow_bits of csrc/fr.cuh against Python
+    integers, on edge limbs."""
     rnd = random.Random(1)
     edges = [0, 1, 2, R - 1, R - 2, 2 ** 32 - 1, 2 ** 32, 2 ** 64 - 1, 2 ** 255 % R, (R - 1) // 2, (R + 1) // 2]
     edges += [sum(0xFFFFFFFF << (32 * i) for i in range(k)) % R for k in range(1, 9)]
@@ -92,9 +92,14 @@ def test_fr_sub_and_powers_on_edge_limbs(he):
         he.hostemul_coset_fr_op(k, le(a), le(b), out)
         return int.from_bytes(out.raw, "little")
 
+    rinv = pow(2 ** 256, -1, R)
     for a in edges:
         for b in edges:
             assert op(0, a, b) == (a - b) % R, (a, b)
+            assert op(3, a, b) == a * b * rinv % R, (a, b)
+            assert op(4, a, b) == (a + b) % R, (a, b)
+    for a, canon in ((0, 1), (R - 1, 1), (R, 0), (R + 1, 0), (2 ** 256 - 1, 0), (R | (1 << 255), 0), (2 ** 254, 1)):
+        assert op(5, a, 0) == canon, a
     assert op(1, 0, 0) == 2 ** 256 % R
     for a in edges[:12] + edges[-5:]:
         for x in (0, 1, 2, 3, 2 ** 20 - 1, 2 ** 32 + 5, 2 ** 64 - 1, rnd.randrange(2 ** 64)):
@@ -112,19 +117,22 @@ def _host_quotient(lib, p, lg_k, c, lg_chunk, lg_threads):
 
 @pytest.mark.parametrize("lg_k", [0, 1, 5, 10])
 @pytest.mark.parametrize("lg_chunk,lg_threads", [(0, 2), (1, 2), (LG_CHUNK, 2), (0, LG_CARRY_THREADS),
-                                                 (LG_CHUNK, LG_CARRY_THREADS)])
+                                                 (LG_CHUNK, LG_CARRY_THREADS), (1, LG_CARRY_THREADS)])
 def test_strided_quotient_equals_division(he, lg_k, lg_chunk, lg_threads):
     """The strided blocked scan (chunks of 1, 2, 32 rows, a carry segment of at most 4 or 1024 threads) gives exactly
     the quotient and remainder of long division by X^k - c: n around k, multiples of k, the chunk and the block of
-    chunks, c = 1, r - 1 and random, and p = (X^k - c) s, whose remainder is 0 and quotient s."""
+    chunks, several runs per carry thread, c = 0, 1, r - 1 and random, p = (X^k - c) s, whose remainder is 0 and
+    quotient s, and the constant polynomials 0 and r - 1.  At k = 1 this is synthetic division by X - z, the witness
+    polynomial of ptau_kzg_open with r = [p(z)]."""
     rnd = random.Random(lg_k * 101 + lg_chunk * 7 + lg_threads)
     k, L, T = 1 << lg_k, 1 << lg_chunk, 1 << lg_threads
-    sizes = {0, 1, max(k - 1, 0), k, k + 1, 3 * k - 1, 3 * k + 1, k * L - 1, k * L + 1, k * L * T + 1}
+    sizes = {0, 1, 2, max(k - 1, 0), k, k + 1, 3 * k - 1, 3 * k + 1, k * L - 1, k * L, k * L + 1, k * L * T - 1,
+             k * L * T, k * L * T + 1}
     if k * L * T < 4096:
-        sizes |= {5 * k * L * T + 3}  # several runs per carry thread
+        sizes |= {5 * k * L * T + 3, 3 * k * L * T + 5, 17 * k * L * T - 3}  # several runs per carry thread
     for n in sorted(s for s in sizes if s <= 40000):
         p = [rnd.randrange(R) for _ in range(n)]
-        for c in (1, R - 1, rnd.randrange(R)):
+        for c in (0, 1, R - 1, rnd.randrange(R)):
             bad, q, rem = _host_quotient(he, p, lg_k, c, lg_chunk, lg_threads)
             assert bad == 0 and (q, rem) == divide(p, k, c), (n, c)
         if n > k:
@@ -133,6 +141,11 @@ def test_strided_quotient_equals_division(he, lg_k, lg_chunk, lg_threads):
             pp = [((s[i - k] if i >= k else 0) - c * (s[i] if i < n - k else 0)) % R for i in range(n)]
             bad, q, rem = _host_quotient(he, pp, lg_k, c, lg_chunk, lg_threads)
             assert bad == 0 and q == s and rem == [0] * k, n
+    for n in (k * L + 1, k * L * T + 1):
+        for v in (0, R - 1):
+            if n <= 40000:
+                c = rnd.randrange(R)
+                assert _host_quotient(he, [v] * n, lg_k, c, lg_chunk, lg_threads) == (0, *divide([v] * n, k, c)), (n, v)
 
 
 def test_strided_quotient_flags_non_canonical(he):

@@ -1,36 +1,15 @@
-"""KZG10::open on the GPU (ptau_kzg_open, KZG10.open_many): the quotient scan of csrc/kzg_open.cuh and csrc/fr.cuh
-against big-integer synthetic division on the host build, and the openings against the host quotient committed by
-the existing MSM, against a known tau, and against KZG10.check_many on the GPU."""
-import ctypes
-import os
+"""KZG10::open on the GPU (ptau_kzg_open, KZG10.open_many): the openings against the host quotient committed by the
+existing MSM, against a known tau, and against KZG10.check_many on the GPU.  The division scan they run is the k = 1
+case of the coset openings' and is tested on the host build in test_kzg_cosets.py."""
 import random
 
 import numpy as np
 import pytest
 
 import ptau_oracle as o
-from conftest import ROOT
 
 R = o.R_ORDER
 ZU, ML = 1, 4
-LG_CHUNK = 5         # kKzgLgChunk
-LG_CARRY_THREADS = 10  # kKzgLgCarryThreads
-
-
-@pytest.fixture(scope="module")
-def hostemul_open():
-    """Host build of fr.cuh and the quotient scan items (tests/host_emul/hostemul_open.cpp)."""
-    d = os.path.join(ROOT, "tests", "host_emul")
-    so = os.path.join(d, "libptau_hostemul_open.so")
-    csrc = os.path.join(ROOT, "kzg_setup_powersoftau_b200", "csrc")
-    deps = [os.path.join(d, "hostemul_open.cpp")] + [os.path.join(csrc, f) for f in os.listdir(csrc)
-                                                      if f.endswith((".cuh", ".inc", ".h"))]
-    if not os.path.exists(so) or os.path.getmtime(so) < max(os.path.getmtime(p) for p in deps):
-        import subprocess
-
-        subprocess.check_call(["g++", "-O2", "-std=c++17", "-fPIC", "-shared", "-Wno-unknown-pragmas", "-o", so,
-                               os.path.join(d, "hostemul_open.cpp")])
-    return ctypes.CDLL(so)
 
 
 def le(v: int) -> bytes:
@@ -54,79 +33,6 @@ def evaluate(coeffs, x):
     return acc
 
 
-# ---------------------------------------------------------------------------------------------- CPU
-def test_fr_ops_on_edge_limbs(hostemul_open):
-    """fr_mul (a b R^-1), fr_add and fr_is_canonical of csrc/fr.cuh against Python integers."""
-    rinv = pow(2 ** 256, -1, R)
-    rnd = random.Random(1)
-    edges = [0, 1, 2, R - 1, R - 2, 2 ** 32 - 1, 2 ** 32, 2 ** 64 - 1, 2 ** 255 % R, (R - 1) // 2, (R + 1) // 2]
-    edges += [sum(0xFFFFFFFF << (32 * i) for i in range(k)) % R for k in range(1, 9)]
-    edges += [((R >> (32 * i)) << (32 * i)) - 1 for i in range(1, 8)]
-    edges += [rnd.randrange(R) for _ in range(20)]
-    out = ctypes.create_string_buffer(32)
-
-    def op(k, a, b):
-        hostemul_open.hostemul_fr_op(k, le(a), le(b), out)
-        return int.from_bytes(out.raw, "little")
-
-    for a in edges:
-        for b in edges:
-            assert op(0, a, b) == a * b * rinv % R, (a, b)
-            assert op(1, a, b) == (a + b) % R, (a, b)
-    for a, canon in ((0, 1), (R - 1, 1), (R, 0), (R + 1, 0), (2 ** 256 - 1, 0), (R | (1 << 255), 0), (2 ** 254, 1)):
-        assert op(2, a, 0) == canon, a
-
-
-def _host_scan(lib, coeffs, z, lg_chunk, lg_threads):
-    n = len(coeffs)
-    cb = b"".join(le(c) for c in coeffs)
-    q = ctypes.create_string_buffer(max(n - 1, 1) * 32)
-    v = ctypes.create_string_buffer(32)
-    bad = lib.hostemul_kzg_quotient(cb, ctypes.c_size_t(n), le(z), lg_chunk, lg_threads, q, v)
-    return bad, int.from_bytes(v.raw, "little"), [int.from_bytes(q.raw[32 * i:32 * i + 32], "little") for i in range(max(n - 1, 0))]
-
-
-@pytest.mark.parametrize("lg_chunk", [0, 1, LG_CHUNK])
-@pytest.mark.parametrize("lg_threads", [2, LG_CARRY_THREADS])
-def test_chunked_quotient_equals_synthetic_division(hostemul_open, lg_chunk, lg_threads):
-    """The blocked scan (chunks of L = 1, 2, 32 (the shipped length), a carry block of 4 or 1024 (the shipped width)
-    threads) gives exactly the quotient and value of synthetic division: n around the chunk and around one block of
-    chunks, several runs per carry thread, z = 0, 1, r - 1, a root of p and random z, coefficients 0 and r - 1."""
-    rnd = random.Random(lg_chunk * 31 + lg_threads)
-    L, T = 1 << lg_chunk, 1 << lg_threads
-    sizes = sorted({0, 1, 2, max(L - 1, 1), L, L + 1, T * L - 1, T * L, T * L + 1})
-    if T * L < 4096:
-        sizes += [3 * T * L + 5, 17 * T * L - 3]  # several sums per carry thread
-    for n in sizes:
-        coeffs = [rnd.randrange(R) for _ in range(n)]
-        zs = [0, 1, R - 1, rnd.randrange(R)]
-        for z in zs:
-            bad, v, q = _host_scan(hostemul_open, coeffs, z, lg_chunk, lg_threads)
-            assert bad == 0 and (v, q) == synthetic_division(coeffs, z), (n, z)
-        if n >= 2:  # p = (X - a) s(X): p(a) = 0
-            a = rnd.randrange(R)
-            s = [rnd.randrange(R) for _ in range(n - 1)]
-            p = [((s[i - 1] if i else 0) - a * (s[i] if i < n - 1 else 0)) % R for i in range(n)]
-            bad, v, q = _host_scan(hostemul_open, p, a, lg_chunk, lg_threads)
-            assert bad == 0 and v == 0 and q == s, n
-    for n in (L + 1, T * L + 1):
-        for c in (0, R - 1):
-            z = rnd.randrange(R)
-            assert _host_scan(hostemul_open, [c] * n, z, lg_chunk, lg_threads)[1:] == synthetic_division([c] * n, z)
-
-
-def test_chunked_quotient_flags_non_canonical(hostemul_open):
-    """A coefficient >= r anywhere (first, middle, last) sets the flag; the flag stays clear otherwise."""
-    n = 100
-    for at in (0, 50, n - 1):
-        for bad_value in (R, 2 ** 256 - 1):
-            coeffs = [7] * n
-            coeffs[at] = bad_value
-            assert _host_scan(hostemul_open, coeffs, 3, LG_CHUNK, LG_CARRY_THREADS)[0] == 1, (at, bad_value)
-    assert _host_scan(hostemul_open, [R - 1] * n, 3, LG_CHUNK, LG_CARRY_THREADS)[0] == 0
-
-
-# ---------------------------------------------------------------------------------------------- GPU
 def _kz():
     import kzg_setup_powersoftau_b200 as kz
     return kz

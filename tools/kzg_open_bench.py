@@ -4,7 +4,7 @@
 for n in {2^16, 2^18, 2^20, 2^21} coefficients and k in {1, 16} points: wall time host to host and the library's
 CUDA-event kernel time (median of 5 runs after one warm-up), every output compared with the old path's.  Then
 KZG10.open with Python ints before (host quotient + resident MSM) and after (open_many), and, in a separate
-torch.profiler pass, the per-kernel split of one open into the quotient kernels (kzg_quotient_*) and the MSM.
+torch.profiler pass, the per-kernel split of one open into the quotient kernels (coset_quotient_*) and the MSM.
 Writes profiles/kzg_open_bench.json (or the path given as the first argument) with the card's name and power
 limit read in the same run."""
 import json
@@ -149,7 +149,7 @@ def main():
                 if ev.device_type != torch.autograd.DeviceType.CUDA:
                     continue
                 us = ev.device_time if hasattr(ev, "device_time") else ev.cuda_time
-                if "kzg_quotient" in ev.name:
+                if "coset_quotient" in ev.name:
                     quot += us
                     names[ev.name] = names.get(ev.name, 0.0) + us
                 elif "msm" in ev.name:
